@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl product|reference]
                     [--workload edos|large|phonon|sweep] [--scaling weak|strong] [--batch B_PER_GPU] [--graph auto|on|off]
+                    [--dump-outputs DIR]
 
 Headline (default flags; BASELINE.json configs[1]/[2]): DOSTransformer(3 GNN, 2 transformer layers, hidden 256), eDOS
 random-split shape (SURVEY.md 8d config 2: ~20 atoms/crystal log-normal, 12 neighbours, 200-d node features, 41-d edge
@@ -24,6 +25,10 @@ the other BASELINE configurations as extra keys, each with its own `config.workl
   optimizer_in_loop (N = 1) fwd + bwd + fused AdamW every step (weight operand planes refreshed every step)
   cpu_baseline(s)  (N = 1) the reference's own modules (oracle/_ref) on the host cores: all cores and the reference's
                    torch.set_num_threads(2) (main_eDOS.py:12), eDOS B = 64 / B = 8 and phonon fp64 B = 1
+
+`--dump-outputs DIR` writes what the last timed step of the line's train step returned to its caller - the loss and the
+gradient of every parameter - as DIR/<name>.npy, so that two builds run with the same arguments (hence the same seeded
+model and batches) can be compared output for output.
 
 `--workload/--scaling/--batch` make one of those the line's own metric instead (same JSON contract).  `--impl reference`
 times the reference's CPU implementation (kind "reference" when oracle/_ref or /root/reference is present, else the oracle
@@ -150,6 +155,34 @@ def flops_per_crystal_fwd(n_nodes: float, n_edges: float, nmax: float) -> float:
     f += 3 * t * 4 * T * nmax * H + 2 * t * 4 * T * T * H + 5 * t * 2 * T * (8 * H * H)
     f += 2 * T * (2 * H * H) + 2 * T * (2.5 * H * H) + 4 * T * H + 2 * (2 * H * H)
     return f
+
+
+# ======================================================================================================== output dump
+DUMP_BYTES = 60 << 20        # array data of --dump-outputs; with the .npy headers the directory stays under 64 MB
+
+
+def step_outputs(model, loss) -> dict:
+    """What a caller of the train step receives: the loss and the gradient of every parameter that has one."""
+    out = {"loss": loss}
+    out.update({f"grad.{k}": p.grad for k, p in model.named_parameters() if p.grad is not None})
+    return out
+
+
+def dump_outputs(out_dir: str, arrays: dict, budget: int = DUMP_BYTES) -> None:
+    """Writes every tensor as out_dir/<name>.npy, float64 ones as float64 and all others as float32.  When the set holds
+    more than `budget` bytes, every array is cut to the same fraction of its elements (flattened), chosen by a generator
+    seeded from nothing but the array's length: two runs with the same arguments write the same elements."""
+    import numpy as np
+    host = {k: v.detach().to("cpu", torch.float64 if v.dtype == torch.float64 else torch.float32) for k, v in arrays.items()}
+    total = sum(v.numel() * v.element_size() for v in host.values())
+    keep = min(1.0, budget / max(total, 1))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in host.items():
+        if keep < 1.0:
+            n = v.numel()
+            idx = torch.randperm(n, generator=torch.Generator().manual_seed(n))[:max(1, int(n * keep))].sort().values
+            v = v.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), v.numpy())
 
 
 # ======================================================================================================== CPU legs
@@ -430,6 +463,7 @@ class Runner:
         self.graph = GraphedStep(model, mode, loss_weight=weight, world=world) if use_graph else None
         self.tkey = "y_ft" if mode == "edos" else "phdos"
         self.fallback = None
+        self.last = None          # the loss of the last step (a graph replay overwrites it with the next one)
 
     def describe(self):
         if self.graph is not None:
@@ -438,6 +472,10 @@ class Runner:
         return base + (f" (graph capture failed: {self.fallback})" if self.fallback else "")
 
     def __call__(self, g):
+        self.last = self._step(g)
+        return self.last
+
+    def _step(self, g):
         if self.graph is not None:
             try:
                 return self.graph(g)
@@ -817,6 +855,8 @@ def run_product(args, rank: int, world: int, local_rank: int):
     sec, dev_each = timed_steps(step, resident, args.steps, 0, barrier, st, args.ncu_window)
     launches = (L.launch_count() - l0) + ((step.graph.launches - g0) if step.graph is not None else 0)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:       # before any further step overwrites them
+        dump_outputs(args.dump_outputs, step_outputs(model, step.last))
     sec = max_over_ranks(sec, world, dev)
     value = world * B * args.steps / sec
 
@@ -1091,7 +1131,14 @@ def main():
                     "ncu --profile-from-start off; a number printed under a profiler is not a bench value)")
     ap.add_argument("--energies", type=int, default=T, help="energy-grid length (201 = the reference's eDOS grid; 1001 = the "
                     "long-grid variant of the large-cell stress configuration); not the headline line when changed")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps write the loss and the parameter gradients "
+                    "of the last timed step as DIR/<name>.npy (float32, float64 for a float64 model; at most 64 MB in all, "
+                    "a fixed seeded sample of every array beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "product" or args.scaling != "weak" or args.workload not in ("edos", "large")):
+        ap.error("--dump-outputs covers the weak-scaling train-step line of the product (--workload edos or large)")
     if args.energies != T:
         globals()["T"] = args.energies
     rank = int(os.environ.get("RANK", "0"))

@@ -12,14 +12,16 @@ oracle/shims.py -- on seeded synthetic batches
 main_phDOS.py:109-114.
 
 Fixtures
-  edos_small.pt / phonon_small.pt   hidden=32: full state_dict, the batch, outputs, loss and
-                                    every live gradient, in the model dtype and (arbiter) fp64.
+  edos_small.pt / phonon_small.pt   hidden=32: outputs, loss and every live gradient in (arbiter) fp64,
+                                    outputs and loss in the model dtype, and per gradient the model
+                                    dtype's distance from fp64 (see compact()).
   edos_h256.pt / phonon_h256.pt     hidden=256, torch.manual_seed(0) init (weights NOT stored: the
                                     product model must reproduce them from the seed), outputs, loss,
                                     per-parameter gradient summaries, fp32 and fp64.
 """
 from __future__ import annotations
 
+import hashlib
 import os
 import sys
 
@@ -66,6 +68,77 @@ def _run(model, g, loss_fn):
                 loss=loss.detach().clone(), grads=grads, dead=dead)
 
 
+def _relerr(a, b):
+    """max |a - b| / max |b|, as tests/conftest.py:relerr."""
+    a, b = a.detach().double(), b.detach().double()
+    return (a - b).abs().max().item() / max(b.abs().max().item(), 1e-30)
+
+
+def _rel_l2(a, b):
+    a, b = a.detach().double(), b.detach().double()
+    return ((a - b).norm() / b.norm().clamp_min(1e-30)).item()
+
+
+def digest(d: dict) -> str:
+    """SHA-256 over the names, dtypes, shapes and bytes of a dict's tensors (other values by repr)."""
+    h = hashlib.sha256()
+    for k, v in d.items():
+        h.update(k.encode())
+        if torch.is_tensor(v):
+            h.update(f"{v.dtype}{tuple(v.shape)}".encode())
+            h.update(v.detach().contiguous().cpu().numpy().tobytes())
+        else:
+            h.update(repr(v).encode())
+    return h.hexdigest()
+
+
+def compact(fx, kind, batch_args):
+    """The stored form of a small fixture.  The initial weights and the batch are kept as what draws them - the init seed
+    with the model's own constructor, the synthetic generator's arguments - plus a digest of their bytes: expand() redraws
+    them and checks the digest, so a fixture still holds the reference's weights bit for bit.  Of the model-dtype gradients
+    only what the tests read is kept: per tensor, their max-norm and L2 distance from the fp64 arbiter.  An fp64 model is
+    its own arbiter: its *64 outputs are the same tensors."""
+    sd, batch, grads = fx.pop("state_dict"), fx.pop("batch"), fx.pop("grads")
+    fx.pop("state_keys")
+    fx.update(model=kind, state_dict_sha256=digest(sd), batch_args=batch_args, batch_keys=list(batch),
+              batch_sha256=digest(batch),
+              grads_noise={k: (_relerr(v, fx["grads64"][k]), _rel_l2(v, fx["grads64"][k])) for k, v in grads.items()})
+    for k in ("loss", "dos_global", "dos_system", "x"):
+        if fx[k].dtype == fx[k + "64"].dtype and torch.equal(fx[k], fx[k + "64"]):
+            fx[k + "64"] = fx[k]
+    flat = torch.cat([v.reshape(-1) for v in fx["grads64"].values()])     # one storage in the file, not one per tensor
+    ends = torch.tensor([v.numel() for v in fx["grads64"].values()]).cumsum(0).tolist()
+    fx["grads64"] = {k: flat[e - v.numel():e].view(v.shape) for (k, v), e in zip(fx["grads64"].items(), ends)}
+    return fx
+
+
+def expand(fx):
+    """Inverse of compact() (fixtures without a weight digest are returned as they are)."""
+    if "state_dict_sha256" not in fx:
+        return fx
+    from dostransformer_b200.embedder_eDOS.DOSTransformer import DOSTransformer
+    from dostransformer_b200.embedder_phDOS.DOSTransformer_phonon import DOSTransformer_phonon
+    cls = {"edos": DOSTransformer, "phonon": DOSTransformer_phonon}[fx["model"]]
+    prev = torch.get_default_dtype()
+    with torch.random.fork_rng(devices=[]):
+        torch.set_default_dtype(getattr(torch, fx["dtype"].split(".")[-1]))
+        try:
+            torch.manual_seed(fx["init_seed"])
+            sd = {k: v.detach().clone() for k, v in cls(*fx["ctor_args"]).state_dict().items()}
+        finally:
+            torch.set_default_dtype(prev)
+    g = {"edos": make_edos_batch, "phonon": make_phonon_batch}[fx["model"]](**fx["batch_args"])
+    batch = {k: getattr(g, k) for k in fx["batch_keys"]}
+    if digest(sd) != fx["state_dict_sha256"]:
+        raise AssertionError(f"{fx['model']} fixture: the initial weights drawn from seed {fx['init_seed']} are not the "
+                             "reference's (the model's parameter order or initialisation changed)")
+    if digest(batch) != fx["batch_sha256"]:
+        raise AssertionError(f"{fx['model']} fixture: synthetic batch {fx['batch_args']} is not the stored one (the "
+                             "generator changed)")
+    fx.update(state_dict=sd, batch=batch)
+    return fx
+
+
 def _summ(gr):
     return {k: dict(norm=v.double().norm().item(), sum=v.double().sum().item(),
                     head=v.flatten()[:8].clone(), shape=tuple(v.shape)) for k, v in gr.items()}
@@ -104,9 +177,9 @@ def main():
     EDOS, PHONON, _ = reference_loader.load()
     cpu = torch.device("cpu")
 
-    g = make_edos_batch(4, seed=2001, mean_atoms=6.0, max_atoms=14)
-    fx = _fixture(EDOS, (3, 2, 200, 41, 2, 32, cpu, 0.0), g, _edos_loss, torch.float32, True)
-    torch.save(fx, os.path.join(OUT, "edos_small.pt"))
+    args = dict(B=4, seed=2001, mean_atoms=6.0, max_atoms=14)
+    fx = _fixture(EDOS, (3, 2, 200, 41, 2, 32, cpu, 0.0), make_edos_batch(**args), _edos_loss, torch.float32, True)
+    torch.save(compact(fx, "edos", args), os.path.join(OUT, "edos_small.pt"))
 
     g = make_edos_batch(8, seed=2002)
     fx = _fixture(EDOS, (3, 2, 200, 41, 2, 256, cpu, 0.0), g, _edos_loss, torch.float32, False)
@@ -114,9 +187,9 @@ def main():
     fx["batch_B"] = 8
     torch.save(fx, os.path.join(OUT, "edos_h256.pt"))
 
-    g = make_phonon_batch(3, seed=1001, K=8, max_atoms=6)
-    fx = _fixture(PHONON, (3, 2, 118, 4, 32, cpu, 0.0), g, _phonon_loss, torch.float64, True)
-    torch.save(fx, os.path.join(OUT, "phonon_small.pt"))
+    args = dict(B=3, seed=1001, K=8, max_atoms=6)
+    fx = _fixture(PHONON, (3, 2, 118, 4, 32, cpu, 0.0), make_phonon_batch(**args), _phonon_loss, torch.float64, True)
+    torch.save(compact(fx, "phonon", args), os.path.join(OUT, "phonon_small.pt"))
 
     g = make_phonon_batch(1, seed=1002)
     fx = _fixture(PHONON, (3, 2, 118, 4, 256, cpu, 0.0), g, _phonon_loss, torch.float64, False)

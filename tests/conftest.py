@@ -39,4 +39,5 @@ def relerr(a: torch.Tensor, b: torch.Tensor) -> float:
 
 
 def load_golden(name):
-    return torch.load(os.path.join(GOLDEN, name), weights_only=False)
+    from oracle.make_golden import expand
+    return expand(torch.load(os.path.join(GOLDEN, name), weights_only=False))

@@ -173,3 +173,35 @@ def test_graph_replay_follows_the_models_padding_length():
         losses[nm] = want.item()
     m.max_num_nodes = None
     assert step.captures == 2 and losses[None] != losses[g.max_num_nodes + 9]
+
+
+def test_bench_dumps_the_last_timed_step(tmp_path):
+    """bench.py --steps K --dump-outputs DIR: the dumped loss and gradients are those of the K-th timed step (batch
+    (K - 1) mod 3 of the rotation, not the warm-up's last), recomputed here eagerly from the same seeded model and batch."""
+    import json
+    import os
+    import subprocess
+    import sys
+    import numpy as np
+    from conftest import ROOT
+    K, B = 5, 8
+    out = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(K), "--warmup", "0", "--batch", str(B),
+                        "--no-extras", "--no-cpu-baseline", "--no-alt", "--dump-outputs", str(out)],
+                       capture_output=True, text=True, timeout=600, cwd=ROOT, env=dict(os.environ, DOST_BENCH_NO_SAMPLER="1"))
+    assert r.returncode == 0, r.stderr[-3000:]
+    line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+    assert line["steps"] == K and len(line["ms_each_step_device"]) == K
+    batches = [make_edos_batch(B, seed=2000 + i, T=201) for i in range(3)]
+    torch.manual_seed(0)
+    m = DOSTransformer(3, 2, 200, 41, 2, 256, torch.device(DEV), 0.0, n_energies=201, precision="bf16x3").to(DEV).train()
+    m.max_num_nodes = max(int(torch.bincount(b.batch).max()) for b in batches)
+    loss, grads = _eager(m, batches[(K - 1) % 3].to(DEV))
+    want = {"loss": loss, **{f"grad.{k}": v for k, v in grads.items()}}
+    assert sorted(p.name[:-4] for p in out.iterdir()) == sorted(want)
+    assert sum(p.stat().st_size for p in out.iterdir()) <= 64 << 20
+    for k, v in want.items():
+        got = np.load(out / f"{k}.npy")
+        assert got.dtype == np.float32 and got.shape == tuple(v.shape), k
+        got, v = torch.from_numpy(got).double(), v.cpu().double()
+        assert ((got - v).norm() / v.norm().clamp_min(1e-30)).item() < 1e-5, k

@@ -247,6 +247,29 @@ def test_bench_reference_arm_contract_and_product_arm_needs_gpu():
         assert r.returncode != 0 and "no CPU fallback" in (r.stderr + r.stdout)
 
 
+def test_bench_dump_outputs_dtypes_and_budget(tmp_path):
+    """bench.py --dump-outputs: float64 arrays are written as float64, all others as float32; past the byte budget every
+    array keeps the same seeded sample of its elements, run after run, and a scalar is never cut away."""
+    import numpy as np
+    import bench
+    arrays = {"loss": torch.tensor(1.5), "grad.w": torch.arange(1000.0).view(10, 100),
+              "grad.h": torch.arange(50, dtype=torch.float16), "grad.d": torch.arange(300, dtype=torch.float64)}
+    bench.dump_outputs(str(tmp_path / "full"), arrays)
+    for k, v in arrays.items():
+        got = np.load(tmp_path / "full" / f"{k}.npy")
+        assert got.dtype == (np.float64 if v.dtype == torch.float64 else np.float32) and got.shape == tuple(v.shape), k
+        assert np.array_equal(got, v.double().numpy()), k
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), arrays, budget=2000)
+    total = 0
+    for k, v in arrays.items():
+        a, b = np.load(tmp_path / "a" / f"{k}.npy"), np.load(tmp_path / "b" / f"{k}.npy")
+        assert np.array_equal(a, b) and a.ndim == 1 and 1 <= a.size < max(2, v.numel()), k
+        assert np.isin(a, v.double().numpy()).all() and np.unique(a).size == a.size, k      # distinct elements of v
+        total += a.nbytes
+    assert total <= 2000 + 8
+
+
 def test_bucket_padding_is_a_semantic_no_op_for_the_real_crystals():
     """synthetic.pad_edos_batch (the shape bucketing behind graphed.GraphedStep): on the CPU oracle, the padded batch's
     outputs, loss over the first n_valid crystals and gradients equal those of the unpadded batch (the padding length
@@ -282,18 +305,27 @@ def test_bucket_padding_is_a_semantic_no_op_for_the_real_crystals():
     assert len(sigs) <= 6
 
 
-def test_staged_reference_copy_is_byte_identical():
-    """oracle/build_ref.py stages the reference's model files for the GPU box: same bytes as /root/reference."""
+def test_staged_reference_copy_is_byte_identical(tmp_path, monkeypatch):
+    """oracle/build_ref.py stages the reference's model files for machines without the reference: the same bytes as the
+    source, their SHA-256 in the manifest, and the staged copy still found once the source is gone.  A stand-in source
+    tree takes the reference's place."""
     import hashlib
     import json
     from oracle import build_ref
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("reference not present")
-    dst = build_ref.build()
-    man = json.load(open(os.path.join(dst, "MANIFEST.json")))
+    src, dst = tmp_path / "reference", tmp_path / "staged"
+    for i, rel in enumerate(build_ref.FILES):
+        (src / rel).parent.mkdir(parents=True, exist_ok=True)
+        (src / rel).write_bytes(f"# {rel}\n".encode() + bytes(range(256)) * i)
+    monkeypatch.setattr(build_ref, "SRC", str(src))
+    monkeypatch.setattr(build_ref, "DST", str(dst))
+    assert build_ref.build() == str(dst)
+    man = json.load(open(dst / "MANIFEST.json"))
+    assert set(man["sha256"]) == set(build_ref.FILES)
     for rel, sha in man["sha256"].items():
-        with open(os.path.join("/root/reference", rel), "rb") as f:
-            assert hashlib.sha256(f.read()).hexdigest() == sha, rel
+        data = (src / rel).read_bytes()
+        assert (dst / rel).read_bytes() == data and hashlib.sha256(data).hexdigest() == sha, rel
+    monkeypatch.setattr(build_ref, "SRC", str(tmp_path / "absent"))
+    assert build_ref.build() == str(dst)
 
 
 def test_kernel_path_gates_are_host_decisions(monkeypatch):

@@ -24,10 +24,9 @@ def test_oracle_matches_golden_edos_small():
     assert relerr(outs[2], fx["dos_system"]) < 2e-6
     assert relerr(outs[1], fx["x"]) < 2e-6
     assert abs(loss.item() - fx["loss"].item()) < 1e-6
-    assert set(grads) == set(fx["grads"])
-    for k, ref in fx["grads"].items():
-        ref64 = fx["grads64"][k]
-        tol = max(1e-4, 3 * relerr(ref, ref64))
+    assert set(grads) == set(fx["grads64"])
+    for k, ref64 in fx["grads64"].items():
+        tol = max(1e-4, 3 * fx["grads_noise"][k][0])        # relerr(the reference's fp32 gradient, ref64)
         assert relerr(grads[k], ref64) < tol, k
 
 
@@ -54,7 +53,7 @@ def test_oracle_matches_golden_phonon_small():
     assert relerr(outs[0], fx["dos_global"]) < 1e-10
     assert relerr(outs[2], fx["dos_system"]) < 1e-10
     assert abs(loss.item() - fx["loss"].item()) < 1e-10
-    for k, ref in fx["grads"].items():
+    for k, ref in fx["grads64"].items():
         assert relerr(grads[k], ref) < 1e-7, k
 
 
@@ -67,7 +66,8 @@ def test_dead_parameters_listed():
     assert len(fxp["dead"]) == 46 and "alpha" in fxp["dead"]
 
 
-@pytest.mark.skipif(not reference_loader.available(), reason="/root/reference not present")
+@pytest.mark.skipif(not reference_loader.available(),
+                    reason="the original project's model code is not available (DOST_REFERENCE_ROOT or oracle/_ref/)")
 def test_oracle_matches_live_reference():
     EDOS, PHONON, _ = reference_loader.load()
     torch.manual_seed(5)

@@ -187,6 +187,18 @@ _SIGNATURES = {
                                        C.c_void_p]),
 }
 
+
+def _with_seed_offset(args):
+    """The argument list of a dost_<name>_dseed sibling: `const unsigned long long* seed_offset` after the seed."""
+    i = args.index(C.c_ulonglong) + 1
+    return args[:i] + [C.c_void_p] + args[i:]
+
+
+for _name in ("dost_xattn_fwd", "dost_xattn_bwd", "dost_xattn_softmax_fwd", "dost_xattn_softmax_bwd", "dost_softmax_fwd",
+              "dost_softmax_bwd", "dost_softmax_fwd_planes", "dost_softmax_bwd_planes", "dost_attn_fused_fwd"):
+    _res, _args = _SIGNATURES[_name]
+    _SIGNATURES[_name + "_dseed"] = (_res, _with_seed_offset(_args))
+
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 
 

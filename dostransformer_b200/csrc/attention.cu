@@ -15,11 +15,12 @@ namespace dost {
 bool xattn_v2_supported(int H);
 int xattn_v2_fwd(const float* q, long long q_ss, const float* kv, const float* phantom, const int* ptr, const int* nmax,
                  const float* resid, long long r_ss, float* out, float* lse, int S, int B, int Tn, int H, float scale,
-                 unsigned int thresh, float inv_keep, unsigned long long seed, cudaStream_t st);
+                 unsigned int thresh, float inv_keep, unsigned long long seed, const unsigned long long* seed_offset,
+                 cudaStream_t st);
 int xattn_v2_bwd(const float* dO, const float* q, long long q_ss, const float* kv, const float* phantom, const int* ptr,
                  const int* nmax, const float* out, const float* resid, long long r_ss, const float* lse, float* dq, float* dkv,
                  float* Dbuf, float* part, int S, int B, int Tn, int H, float scale, unsigned int thresh, float inv_keep,
-                 unsigned long long seed, bool do_kv, cudaStream_t st);
+                 unsigned long long seed, const unsigned long long* seed_offset, bool do_kv, cudaStream_t st);
 
 constexpr int kQPW = 4;               // queries per warp
 constexpr int kAttWarps = 8;
@@ -46,8 +47,9 @@ __global__ void __launch_bounds__(kAttWarps * 32) xattn_fwd_kernel(
     const T* __restrict__ q, long long q_ss, const T* __restrict__ kv, const T* __restrict__ phantom,
     const int* __restrict__ ptr, const int* __restrict__ nmax_p, const T* __restrict__ resid, long long r_ss,
     T* __restrict__ out, float* __restrict__ lse, int S, int B, int Tn, T scale, unsigned int thresh, float inv_keep,
-    unsigned long long seed) {
+    unsigned long long seed, const unsigned long long* __restrict__ seed_offset) {
   constexpr int H = 32 * HV;
+  seed = mask_seed(seed, seed_offset);
   extern __shared__ __align__(16) unsigned char smem_raw[];
   T* ks = reinterpret_cast<T*>(smem_raw);  // [kKT][H]
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -160,8 +162,9 @@ __global__ void __launch_bounds__(kAttWarps * 32) xattn_bwd_q_kernel(
     const T* __restrict__ phantom, const int* __restrict__ ptr, const int* __restrict__ nmax_p,
     const T* __restrict__ out, const T* __restrict__ resid, long long r_ss, const float* __restrict__ lse,
     T* __restrict__ dq, T* __restrict__ Dbuf, T* __restrict__ dph_part, int S, int B, int Tn, T scale,
-    unsigned int thresh, float inv_keep, unsigned long long seed) {
+    unsigned int thresh, float inv_keep, unsigned long long seed, const unsigned long long* __restrict__ seed_offset) {
   constexpr int H = 32 * HV;
+  seed = mask_seed(seed, seed_offset);
   extern __shared__ __align__(16) unsigned char smem_raw[];
   T* ks = reinterpret_cast<T*>(smem_raw);  // [kKT][H], reused as [kAttWarps][H] for the phantom reduction
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -302,8 +305,9 @@ __global__ void __launch_bounds__(kAttWarps * 32) xattn_bwd_kv_kernel(
     const T* __restrict__ dO, const T* __restrict__ q, long long q_ss, const T* __restrict__ kv,
     const int* __restrict__ ptr, const int* __restrict__ node_crystal, const int* __restrict__ nmax_p,
     const float* __restrict__ lse, const T* __restrict__ Dbuf, T* __restrict__ dkv, int S, int B, int Tn, long long N,
-    T scale, unsigned int thresh, float inv_keep, unsigned long long seed) {
+    T scale, unsigned int thresh, float inv_keep, unsigned long long seed, const unsigned long long* __restrict__ seed_offset) {
   constexpr int H = 32 * HV;
+  seed = mask_seed(seed, seed_offset);
   extern __shared__ __align__(16) unsigned char smem_raw[];
   T* ks = reinterpret_cast<T*>(smem_raw);  // [kNT][H] keys, then [kAttWarps][H] reduction scratch
   T* red = ks + kNT * H;
@@ -386,9 +390,11 @@ template <typename T, int NPL>
 __global__ void __launch_bounds__(256) softmax_fwd_kernel(const T* __restrict__ sc, T* __restrict__ p,
                                                           T* __restrict__ pd, long long rows, int cols, long long ld, T scale,
                                                           unsigned int thresh, float inv_keep,
-                                                          unsigned long long seed, __nv_bfloat16* __restrict__ hi,
-                                                          __nv_bfloat16* __restrict__ lo, long long ldp) {
+                                                          unsigned long long seed, const unsigned long long* __restrict__ seed_offset,
+                                                          __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo,
+                                                          long long ldp) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  seed = mask_seed(seed, seed_offset);
   for (long long r = blockIdx.x * 8LL + warp; r < rows; r += (long long)gridDim.x * 8) {
     const T* sr = sc + r * ld;
     float v[NPL];
@@ -434,9 +440,11 @@ template <typename T, int NPL>
 __global__ void __launch_bounds__(256) softmax_bwd_kernel(const T* __restrict__ p, const T* __restrict__ dpd,
                                                           T* __restrict__ ds, long long rows, int cols, long long ld, T scale,
                                                           unsigned int thresh, float inv_keep,
-                                                          unsigned long long seed, __nv_bfloat16* __restrict__ hi,
-                                                          __nv_bfloat16* __restrict__ lo, long long ldp) {
+                                                          unsigned long long seed, const unsigned long long* __restrict__ seed_offset,
+                                                          __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo,
+                                                          long long ldp) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  seed = mask_seed(seed, seed_offset);
   for (long long r = blockIdx.x * 8LL + warp; r < rows; r += (long long)gridDim.x * 8) {
     T pv[NPL], dp[NPL];
     T dot = T(0);
@@ -475,12 +483,13 @@ __global__ void __launch_bounds__(256) softmax_bwd_kernel(const T* __restrict__ 
 template <typename T>
 static int run_xattn_fwd(const void* q, long long q_ss, const void* kv, const void* phantom, const int* ptr,
                          const int* nmax, const void* resid, long long r_ss, void* out, float* lse, int S, int B,
-                         int Tn, int H, double scale, double drop_p, unsigned long long seed, cudaStream_t st) {
+                         int Tn, int H, double scale, double drop_p, unsigned long long seed,
+                         const unsigned long long* seed_offset, cudaStream_t st) {
   const unsigned int thresh = drop_p > 0 ? drop_threshold(drop_p) : 0u;
   const float inv_keep = drop_p > 0 ? (float)(1.0 / (1.0 - drop_p)) : 1.f;
   if (sizeof(T) == 4 && xattn_v2_supported(H))
     return xattn_v2_fwd((const float*)q, q_ss, (const float*)kv, (const float*)phantom, ptr, nmax, (const float*)resid, r_ss,
-                        (float*)out, lse, S, B, Tn, H, (float)scale, thresh, inv_keep, seed, st);
+                        (float*)out, lse, S, B, Tn, H, (float)scale, thresh, inv_keep, seed, seed_offset, st);
   dim3 grid(ceil_div(Tn, kQPB), S);
   const size_t smem = sizeof(T) * (size_t)kKT * H;
 #define DOST_XF(HV)                                                                                                  \
@@ -489,7 +498,7 @@ static int run_xattn_fwd(const void* q, long long q_ss, const void* kv, const vo
       cudaFuncSetAttribute(xattn_fwd_kernel<T, HV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);         \
     xattn_fwd_kernel<T, HV><<<grid, kAttWarps * 32, smem, st>>>((const T*)q, q_ss, (const T*)kv, (const T*)phantom, ptr, \
                                                                 nmax, (const T*)resid, r_ss, (T*)out, lse, S, B, Tn,  \
-                                                                (T)scale, thresh, inv_keep, seed);                   \
+                                                                (T)scale, thresh, inv_keep, seed, seed_offset);      \
     break;
   switch (H / 32) {
     DOST_XF(1) DOST_XF(2) DOST_XF(4) DOST_XF(8) DOST_XF(16)
@@ -507,8 +516,8 @@ template <typename T>
 static int run_xattn_bwd(const void* dO, const void* q, long long q_ss, const void* kv, const void* phantom,
                          const int* ptr, const int* node_crystal, const int* nmax, const void* out, const void* resid,
                          long long r_ss, const float* lse, void* dq, void* dkv, void* dphantom, int S, int B, int Tn,
-                         int H, long long N, double scale, double drop_p, unsigned long long seed, void* workspace,
-                         size_t workspace_bytes, cudaStream_t st) {
+                         int H, long long N, double scale, double drop_p, unsigned long long seed,
+                         const unsigned long long* seed_offset, void* workspace, size_t workspace_bytes, cudaStream_t st) {
   const unsigned int thresh = drop_p > 0 ? drop_threshold(drop_p) : 0u;
   const float inv_keep = drop_p > 0 ? (float)(1.0 / (1.0 - drop_p)) : 1.f;
   dim3 grid(ceil_div(Tn, kQPB), S);
@@ -529,7 +538,7 @@ static int run_xattn_bwd(const void* dO, const void* q, long long q_ss, const vo
   if (v2) {   // dq, D and the phantom partials from the FMA-bound kernel; dkv keeps the node-block kernel below
     int rc2 = xattn_v2_bwd((const float*)dO, (const float*)q, q_ss, (const float*)kv, (const float*)phantom, ptr, nmax,
                            (const float*)out, (const float*)resid, r_ss, lse, (float*)dq, (float*)dkv, (float*)Dbuf, (float*)part, S,
-                           B, Tn, H, (float)scale, thresh, inv_keep, seed, false, st);
+                           B, Tn, H, (float)scale, thresh, inv_keep, seed, seed_offset, false, st);
     if (rc2 != DOST_OK) return rc2;
   }
   const size_t smem_q = sizeof(T) * (size_t)kKT * H;
@@ -544,12 +553,12 @@ static int run_xattn_bwd(const void* dO, const void* q, long long q_ss, const vo
     if (!v2) {                                                                                                        \
       xattn_bwd_q_kernel<T, HV><<<grid, kAttWarps * 32, smem_q, st>>>(                                                \
           (const T*)dO, (const T*)q, q_ss, (const T*)kv, (const T*)phantom, ptr, nmax, (const T*)out, (const T*)resid, \
-          r_ss, lse, (T*)dq, Dbuf, part, S, B, Tn, (T)scale, thresh, inv_keep, seed);                                 \
+          r_ss, lse, (T*)dq, Dbuf, part, S, B, Tn, (T)scale, thresh, inv_keep, seed, seed_offset);                    \
       count_launch();                                                                                                 \
     }                                                                                                                 \
     xattn_bwd_kv_kernel<T, HV><<<kvblocks, kAttWarps * 32, smem_kv, st>>>(                                            \
         (const T*)dO, (const T*)q, q_ss, (const T*)kv, ptr, node_crystal, nmax, lse, Dbuf, (T*)dkv, S, B, Tn, N,      \
-        (T)scale, thresh, inv_keep, seed);                                                                            \
+        (T)scale, thresh, inv_keep, seed, seed_offset);                                                               \
     break;
   switch (H / 32) {
     DOST_XB(1) DOST_XB(2) DOST_XB(4) DOST_XB(8) DOST_XB(16)
@@ -565,8 +574,8 @@ static int run_xattn_bwd(const void* dO, const void* q, long long q_ss, const vo
 
 template <typename T>
 static int run_softmax(bool fwd, const void* a, void* b, void* c, long long rows, int cols, long long ld, double scale,
-                       double drop_p, unsigned long long seed, cudaStream_t st, void* hi = nullptr, void* lo = nullptr,
-                       long long ldp = 0) {
+                       double drop_p, unsigned long long seed, const unsigned long long* seed_offset, cudaStream_t st,
+                       void* hi = nullptr, void* lo = nullptr, long long ldp = 0) {
   const unsigned int thresh = drop_p > 0 ? drop_threshold(drop_p) : 0u;
   const float inv_keep = drop_p > 0 ? (float)(1.0 / (1.0 - drop_p)) : 1.f;
   int npl = (cols + 31) / 32, pw = 1;
@@ -576,10 +585,11 @@ static int run_softmax(bool fwd, const void* a, void* b, void* c, long long rows
   case NPL:                                                                                                       \
     if (fwd)                                                                                                      \
       softmax_fwd_kernel<T, NPL><<<blocks, 256, 0, st>>>((const T*)a, (T*)b, (T*)c, rows, cols, ld, (T)scale, thresh, \
-                                                         inv_keep, seed, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo, ldp); \
+                                                         inv_keep, seed, seed_offset, (__nv_bfloat16*)hi,         \
+                                                         (__nv_bfloat16*)lo, ldp);                                \
     else                                                                                                          \
       softmax_bwd_kernel<T, NPL><<<blocks, 256, 0, st>>>((const T*)a, (const T*)b, (T*)c, rows, cols, ld, (T)scale,   \
-                                                         thresh, inv_keep, seed, (__nv_bfloat16*)hi,              \
+                                                         thresh, inv_keep, seed, seed_offset, (__nv_bfloat16*)hi, \
                                                          (__nv_bfloat16*)lo, ldp);                                \
     break;
   switch (pw) {
@@ -596,20 +606,30 @@ static int run_softmax(bool fwd, const void* a, void* b, void* c, long long rows
 
 using namespace dost;
 
-extern "C" int dost_xattn_fwd(int dtype, const void* q, long long q_sstride, const void* kv, const void* phantom,
-                              const int32_t* ptr, const int32_t* nmax, const void* resid, long long resid_sstride,
-                              void* out, float* lse, int S, int B, int T, int H, double scale, double drop_p,
-                              unsigned long long seed, dost_stream_t stream) {
+extern "C" int dost_xattn_fwd_dseed(int dtype, const void* q, long long q_sstride, const void* kv, const void* phantom,
+                                    const int32_t* ptr, const int32_t* nmax, const void* resid, long long resid_sstride,
+                                    void* out, float* lse, int S, int B, int T, int H, double scale, double drop_p,
+                                    unsigned long long seed, const unsigned long long* seed_offset, dost_stream_t stream) {
   DOST_REQUIRE(q && kv && phantom && ptr && nmax && resid && out && lse, "xattn_fwd: null pointer");
   DOST_REQUIRE(S > 0 && B > 0 && S % B == 0 && T > 0 && H % 32 == 0, "xattn_fwd: bad shape S=%d B=%d T=%d H=%d", S, B, T, H);
   DOST_REQUIRE(drop_p >= 0.0 && drop_p < 1.0, "xattn_fwd: dropout must be in [0,1)");
   cudaStream_t st = (cudaStream_t)stream;
   if (dtype == DOST_F32)
-    return run_xattn_fwd<float>(q, q_sstride, kv, phantom, ptr, nmax, resid, resid_sstride, out, lse, S, B, T, H, scale, drop_p, seed, st);
+    return run_xattn_fwd<float>(q, q_sstride, kv, phantom, ptr, nmax, resid, resid_sstride, out, lse, S, B, T, H, scale, drop_p, seed,
+                                seed_offset, st);
   if (dtype == DOST_F64)
-    return run_xattn_fwd<double>(q, q_sstride, kv, phantom, ptr, nmax, resid, resid_sstride, out, lse, S, B, T, H, scale, drop_p, seed, st);
+    return run_xattn_fwd<double>(q, q_sstride, kv, phantom, ptr, nmax, resid, resid_sstride, out, lse, S, B, T, H, scale, drop_p, seed,
+                                 seed_offset, st);
   set_error("xattn_fwd: unsupported dtype %d", dtype);
   return DOST_ERR_UNSUPPORTED;
+}
+
+extern "C" int dost_xattn_fwd(int dtype, const void* q, long long q_sstride, const void* kv, const void* phantom,
+                              const int32_t* ptr, const int32_t* nmax, const void* resid, long long resid_sstride,
+                              void* out, float* lse, int S, int B, int T, int H, double scale, double drop_p,
+                              unsigned long long seed, dost_stream_t stream) {
+  return dost_xattn_fwd_dseed(dtype, q, q_sstride, kv, phantom, ptr, nmax, resid, resid_sstride, out, lse, S, B, T, H, scale, drop_p,
+                              seed, nullptr, stream);
 }
 
 extern "C" size_t dost_xattn_bwd_workspace_bytes(int dtype, int S, int T, int H) {
@@ -620,62 +640,100 @@ extern "C" size_t dost_xattn_bwd_workspace_bytes(int dtype, int S, int T, int H)
   return o_cs + dost_colsum_workspace_bytes(dtype, nblk, H);
 }
 
-extern "C" int dost_xattn_bwd(int dtype, const void* d_out, const void* q, long long q_sstride, const void* kv,
-                              const void* phantom, const int32_t* ptr, const int32_t* node_crystal,
-                              const int32_t* nmax, const void* out, const void* resid, long long resid_sstride,
-                              const float* lse, void* dq, void* dkv, void* dphantom, int S, int B, int T, int H,
-                              long long N, double scale, double drop_p, unsigned long long seed, void* workspace,
-                              size_t workspace_bytes, dost_stream_t stream) {
+extern "C" int dost_xattn_bwd_dseed(int dtype, const void* d_out, const void* q, long long q_sstride, const void* kv,
+                                    const void* phantom, const int32_t* ptr, const int32_t* node_crystal,
+                                    const int32_t* nmax, const void* out, const void* resid, long long resid_sstride,
+                                    const float* lse, void* dq, void* dkv, void* dphantom, int S, int B, int T, int H,
+                                    long long N, double scale, double drop_p, unsigned long long seed,
+                                    const unsigned long long* seed_offset, void* workspace, size_t workspace_bytes,
+                                    dost_stream_t stream) {
   DOST_REQUIRE(d_out && q && kv && phantom && ptr && node_crystal && nmax && out && resid && lse && dq && dkv && dphantom,
                "xattn_bwd: null pointer");
   DOST_REQUIRE(S > 0 && B > 0 && S % B == 0 && T > 0 && H % 32 == 0 && N > 0, "xattn_bwd: bad shape");
   cudaStream_t st = (cudaStream_t)stream;
   if (dtype == DOST_F32)
     return run_xattn_bwd<float>(d_out, q, q_sstride, kv, phantom, ptr, node_crystal, nmax, out, resid, resid_sstride, lse,
-                                dq, dkv, dphantom, S, B, T, H, N, scale, drop_p, seed, workspace, workspace_bytes, st);
+                                dq, dkv, dphantom, S, B, T, H, N, scale, drop_p, seed, seed_offset, workspace, workspace_bytes, st);
   if (dtype == DOST_F64)
     return run_xattn_bwd<double>(d_out, q, q_sstride, kv, phantom, ptr, node_crystal, nmax, out, resid, resid_sstride, lse,
-                                 dq, dkv, dphantom, S, B, T, H, N, scale, drop_p, seed, workspace, workspace_bytes, st);
+                                 dq, dkv, dphantom, S, B, T, H, N, scale, drop_p, seed, seed_offset, workspace, workspace_bytes, st);
   set_error("xattn_bwd: unsupported dtype %d", dtype);
+  return DOST_ERR_UNSUPPORTED;
+}
+
+extern "C" int dost_xattn_bwd(int dtype, const void* d_out, const void* q, long long q_sstride, const void* kv,
+                              const void* phantom, const int32_t* ptr, const int32_t* node_crystal,
+                              const int32_t* nmax, const void* out, const void* resid, long long resid_sstride,
+                              const float* lse, void* dq, void* dkv, void* dphantom, int S, int B, int T, int H,
+                              long long N, double scale, double drop_p, unsigned long long seed, void* workspace,
+                              size_t workspace_bytes, dost_stream_t stream) {
+  return dost_xattn_bwd_dseed(dtype, d_out, q, q_sstride, kv, phantom, ptr, node_crystal, nmax, out, resid, resid_sstride, lse, dq,
+                              dkv, dphantom, S, B, T, H, N, scale, drop_p, seed, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int dost_softmax_fwd_dseed(int dtype, const void* s, void* p, void* pd, long long rows, int cols, long long ld,
+                                      double scale, double drop_p, unsigned long long seed, const unsigned long long* seed_offset,
+                                      dost_stream_t stream) {
+  DOST_REQUIRE(s && p && rows > 0 && cols > 0 && ld >= cols, "softmax_fwd: bad args");
+  if (!pd) pd = p;
+  DOST_REQUIRE(!(drop_p > 0 && pd == p), "softmax_fwd: dropout needs a separate pd buffer");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == DOST_F32) return run_softmax<float>(true, s, p, pd, rows, cols, ld, scale, drop_p, seed, seed_offset, st);
+  if (dtype == DOST_F64) return run_softmax<double>(true, s, p, pd, rows, cols, ld, scale, drop_p, seed, seed_offset, st);
+  set_error("softmax_fwd: unsupported dtype %d", dtype);
   return DOST_ERR_UNSUPPORTED;
 }
 
 extern "C" int dost_softmax_fwd(int dtype, const void* s, void* p, void* pd, long long rows, int cols, long long ld, double scale,
                                 double drop_p, unsigned long long seed, dost_stream_t stream) {
-  DOST_REQUIRE(s && p && rows > 0 && cols > 0 && ld >= cols, "softmax_fwd: bad args");
-  if (!pd) pd = p;
-  DOST_REQUIRE(!(drop_p > 0 && pd == p), "softmax_fwd: dropout needs a separate pd buffer");
+  return dost_softmax_fwd_dseed(dtype, s, p, pd, rows, cols, ld, scale, drop_p, seed, nullptr, stream);
+}
+
+extern "C" int dost_softmax_bwd_dseed(int dtype, const void* p, const void* dpd, void* ds, long long rows, int cols, long long ld,
+                                      double scale, double drop_p, unsigned long long seed, const unsigned long long* seed_offset,
+                                      dost_stream_t stream) {
+  DOST_REQUIRE(p && dpd && ds && rows > 0 && cols > 0 && ld >= cols, "softmax_bwd: bad args");
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == DOST_F32) return run_softmax<float>(true, s, p, pd, rows, cols, ld, scale, drop_p, seed, st);
-  if (dtype == DOST_F64) return run_softmax<double>(true, s, p, pd, rows, cols, ld, scale, drop_p, seed, st);
-  set_error("softmax_fwd: unsupported dtype %d", dtype);
+  if (dtype == DOST_F32) return run_softmax<float>(false, p, (void*)dpd, ds, rows, cols, ld, scale, drop_p, seed, seed_offset, st);
+  if (dtype == DOST_F64) return run_softmax<double>(false, p, (void*)dpd, ds, rows, cols, ld, scale, drop_p, seed, seed_offset, st);
+  set_error("softmax_bwd: unsupported dtype %d", dtype);
   return DOST_ERR_UNSUPPORTED;
 }
 
 extern "C" int dost_softmax_bwd(int dtype, const void* p, const void* dpd, void* ds, long long rows, int cols, long long ld,
                                 double scale, double drop_p, unsigned long long seed, dost_stream_t stream) {
-  DOST_REQUIRE(p && dpd && ds && rows > 0 && cols > 0 && ld >= cols, "softmax_bwd: bad args");
-  cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == DOST_F32) return run_softmax<float>(false, p, (void*)dpd, ds, rows, cols, ld, scale, drop_p, seed, st);
-  if (dtype == DOST_F64) return run_softmax<double>(false, p, (void*)dpd, ds, rows, cols, ld, scale, drop_p, seed, st);
-  set_error("softmax_bwd: unsupported dtype %d", dtype);
-  return DOST_ERR_UNSUPPORTED;
+  return dost_softmax_bwd_dseed(dtype, p, dpd, ds, rows, cols, ld, scale, drop_p, seed, nullptr, stream);
 }
 
 /* fp32 softmax whose (dropped-out) probabilities / score gradients are also written as bf16 hi/lo operand planes
  * (rows ldp elements apart) for the batched tensor-core GEMMs that consume them. */
-extern "C" int dost_softmax_fwd_planes(const float* s, float* p, float* pd, long long rows, int cols, long long ld, double scale,
-                                       double drop_p, unsigned long long seed, void* hi, void* lo, long long ldp,
-                                       dost_stream_t stream) {
+extern "C" int dost_softmax_fwd_planes_dseed(const float* s, float* p, float* pd, long long rows, int cols, long long ld,
+                                             double scale, double drop_p, unsigned long long seed,
+                                             const unsigned long long* seed_offset, void* hi, void* lo, long long ldp,
+                                             dost_stream_t stream) {
   DOST_REQUIRE(s && p && hi && rows > 0 && cols > 0 && ld >= cols && ldp >= cols, "softmax_fwd_planes: bad args");
   if (!pd) pd = p;
   DOST_REQUIRE(!(drop_p > 0 && pd == p), "softmax_fwd_planes: dropout needs a separate pd buffer");
-  return run_softmax<float>(true, s, p, pd, rows, cols, ld, scale, drop_p, seed, (cudaStream_t)stream, hi, lo, ldp);
+  return run_softmax<float>(true, s, p, pd, rows, cols, ld, scale, drop_p, seed, seed_offset, (cudaStream_t)stream, hi, lo, ldp);
+}
+
+extern "C" int dost_softmax_fwd_planes(const float* s, float* p, float* pd, long long rows, int cols, long long ld, double scale,
+                                       double drop_p, unsigned long long seed, void* hi, void* lo, long long ldp,
+                                       dost_stream_t stream) {
+  return dost_softmax_fwd_planes_dseed(s, p, pd, rows, cols, ld, scale, drop_p, seed, nullptr, hi, lo, ldp, stream);
+}
+
+extern "C" int dost_softmax_bwd_planes_dseed(const float* p, const float* dpd, float* ds, long long rows, int cols, long long ld,
+                                             double scale, double drop_p, unsigned long long seed,
+                                             const unsigned long long* seed_offset, void* hi, void* lo, long long ldp,
+                                             dost_stream_t stream) {
+  DOST_REQUIRE(p && dpd && hi && rows > 0 && cols > 0 && ld >= cols && ldp >= cols, "softmax_bwd_planes: bad args");
+  return run_softmax<float>(false, p, (void*)dpd, ds, rows, cols, ld, scale, drop_p, seed, seed_offset, (cudaStream_t)stream, hi, lo,
+                            ldp);
 }
 
 extern "C" int dost_softmax_bwd_planes(const float* p, const float* dpd, float* ds, long long rows, int cols, long long ld,
                                        double scale, double drop_p, unsigned long long seed, void* hi, void* lo, long long ldp,
                                        dost_stream_t stream) {
-  DOST_REQUIRE(p && dpd && hi && rows > 0 && cols > 0 && ld >= cols && ldp >= cols, "softmax_bwd_planes: bad args");
-  return run_softmax<float>(false, p, (void*)dpd, ds, rows, cols, ld, scale, drop_p, seed, (cudaStream_t)stream, hi, lo, ldp);
+  return dost_softmax_bwd_planes_dseed(p, dpd, ds, rows, cols, ld, scale, drop_p, seed, nullptr, hi, lo, ldp, stream);
 }

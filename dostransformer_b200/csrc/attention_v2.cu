@@ -52,8 +52,10 @@ __global__ void __launch_bounds__(kWarps * 32) fwd_kernel(const float* __restric
                                                           const int* __restrict__ nmax_p, const float* __restrict__ resid,
                                                           long long r_ss, float* __restrict__ out, float* __restrict__ lse, int S,
                                                           int B, int Tn, float scale, unsigned int thresh, float inv_keep,
-                                                          unsigned long long seed) {
+                                                          unsigned long long seed,
+                                                          const unsigned long long* __restrict__ seed_offset) {
   constexpr int H = 128 * NF, KP = H + 4;
+  seed = mask_seed(seed, seed_offset);
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* Qs = reinterpret_cast<float*>(smem_raw);   // [32][H]
   float* Ks = Qs + 32 * H;                           // [32][KP]
@@ -194,8 +196,10 @@ __global__ void __launch_bounds__(kWarps * 32) bwd_q_kernel(const float* __restr
                                                             long long r_ss, const float* __restrict__ lse, float* __restrict__ dq,
                                                             float* __restrict__ Dbuf, float* __restrict__ dph_part, int S, int B, int Tn,
                                                             float scale, unsigned int thresh, float inv_keep,
-                                                            unsigned long long seed) {
+                                                            unsigned long long seed,
+                                                            const unsigned long long* __restrict__ seed_offset) {
   constexpr int H = 128 * NF, KP = H + 4;
+  seed = mask_seed(seed, seed_offset);
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* Qs = reinterpret_cast<float*>(smem_raw);   // [32][H]
   float* Gs = Qs + 32 * H;                           // [32][H]   dO
@@ -356,8 +360,10 @@ __global__ void __launch_bounds__(kWarps * 32) bwd_kv_kernel(const float* __rest
                                                              const int* __restrict__ nmax_p, const float* __restrict__ lse,
                                                              const float* __restrict__ Dbuf, float* __restrict__ dkv, int S, int B, int Tn,
                                                              float scale, unsigned int thresh, float inv_keep,
-                                                             unsigned long long seed) {
+                                                             unsigned long long seed,
+                                                             const unsigned long long* __restrict__ seed_offset) {
   constexpr int H = 128 * NF, KP = H + 4;
+  seed = mask_seed(seed, seed_offset);
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* Qs = reinterpret_cast<float*>(smem_raw);   // [32][H]
   float* Gs = Qs + 32 * H;                           // [32][H]
@@ -452,7 +458,8 @@ __global__ void __launch_bounds__(kWarps * 32) bwd_kv_kernel(const float* __rest
 template <int NF>
 static int launch_fwd(const float* q, long long q_ss, const float* kv, const float* phantom, const int* ptr, const int* nmax,
                       const float* resid, long long r_ss, float* out, float* lse, int S, int B, int Tn, float scale,
-                      unsigned int thresh, float inv_keep, unsigned long long seed, cudaStream_t st) {
+                      unsigned int thresh, float inv_keep, unsigned long long seed, const unsigned long long* seed_offset,
+                      cudaStream_t st) {
   constexpr int H = 128 * NF;
   const size_t smem = sizeof(float) * (32 * H + 32 * (H + 4) + kWarps * 32 * 4);
   static PerDevice cfg_once;
@@ -462,7 +469,7 @@ static int launch_fwd(const float* q, long long q_ss, const float* kv, const flo
   }
   dim3 grid(ceil_div(Tn, kQB), S);
   fwd_kernel<NF><<<grid, kWarps * 32, smem, st>>>(q, q_ss, kv, phantom, ptr, nmax, resid, r_ss, out, lse, S, B, Tn, scale, thresh,
-                                                  inv_keep, seed);
+                                                  inv_keep, seed, seed_offset);
   return check_launch("xattn_fwd");
 }
 
@@ -470,7 +477,8 @@ template <int NF>
 static int launch_bwd(const float* dO, const float* q, long long q_ss, const float* kv, const float* phantom, const int* ptr,
                       const int* nmax, const float* out, const float* resid, long long r_ss, const float* lse, float* dq,
                       float* dkv, float* Dbuf, float* part, int S, int B, int Tn, float scale, unsigned int thresh,
-                      float inv_keep, unsigned long long seed, bool do_kv, cudaStream_t st) {
+                      float inv_keep, unsigned long long seed, const unsigned long long* seed_offset, bool do_kv,
+                      cudaStream_t st) {
   constexpr int H = 128 * NF;
   const size_t smem_q = sizeof(float) * (2 * 32 * H + 32 * (H + 4) + kWarps * 32 * 4);
   const size_t smem_kv = sizeof(float) * (2 * 32 * H + 32 * (H + 4) + 2 * 32 * 32);
@@ -482,12 +490,12 @@ static int launch_bwd(const float* dO, const float* q, long long q_ss, const flo
   }
   dim3 grid(ceil_div(Tn, kQB), S);
   bwd_q_kernel<NF><<<grid, kWarps * 32, smem_q, st>>>(dO, q, q_ss, kv, phantom, ptr, nmax, out, resid, r_ss, lse, dq, Dbuf, part, S, B,
-                                                      Tn, scale, thresh, inv_keep, seed);
+                                                      Tn, scale, thresh, inv_keep, seed, seed_offset);
   int rc = check_launch("xattn_bwd_q");
   if (rc != DOST_OK || !do_kv) return rc;
   dim3 gkv(B, 4);
   bwd_kv_kernel<NF><<<gkv, kWarps * 32, smem_kv, st>>>(dO, q, q_ss, kv, ptr, nmax, lse, Dbuf, dkv, S, B, Tn, scale, thresh, inv_keep,
-                                                       seed);
+                                                       seed, seed_offset);
   return check_launch("xattn_bwd_kv");
 }
 
@@ -497,22 +505,23 @@ bool xattn_v2_supported(int H) { return H == 128 || H == 256 || H == 512; }
 
 int xattn_v2_fwd(const float* q, long long q_ss, const float* kv, const float* phantom, const int* ptr, const int* nmax,
                  const float* resid, long long r_ss, float* out, float* lse, int S, int B, int Tn, int H, float scale,
-                 unsigned int thresh, float inv_keep, unsigned long long seed, cudaStream_t st) {
+                 unsigned int thresh, float inv_keep, unsigned long long seed, const unsigned long long* seed_offset,
+                 cudaStream_t st) {
   switch (H) {
-    case 128: return xa2::launch_fwd<1>(q, q_ss, kv, phantom, ptr, nmax, resid, r_ss, out, lse, S, B, Tn, scale, thresh, inv_keep, seed, st);
-    case 256: return xa2::launch_fwd<2>(q, q_ss, kv, phantom, ptr, nmax, resid, r_ss, out, lse, S, B, Tn, scale, thresh, inv_keep, seed, st);
-    default: return xa2::launch_fwd<4>(q, q_ss, kv, phantom, ptr, nmax, resid, r_ss, out, lse, S, B, Tn, scale, thresh, inv_keep, seed, st);
+    case 128: return xa2::launch_fwd<1>(q, q_ss, kv, phantom, ptr, nmax, resid, r_ss, out, lse, S, B, Tn, scale, thresh, inv_keep, seed, seed_offset, st);
+    case 256: return xa2::launch_fwd<2>(q, q_ss, kv, phantom, ptr, nmax, resid, r_ss, out, lse, S, B, Tn, scale, thresh, inv_keep, seed, seed_offset, st);
+    default: return xa2::launch_fwd<4>(q, q_ss, kv, phantom, ptr, nmax, resid, r_ss, out, lse, S, B, Tn, scale, thresh, inv_keep, seed, seed_offset, st);
   }
 }
 
 int xattn_v2_bwd(const float* dO, const float* q, long long q_ss, const float* kv, const float* phantom, const int* ptr,
                  const int* nmax, const float* out, const float* resid, long long r_ss, const float* lse, float* dq, float* dkv,
                  float* Dbuf, float* part, int S, int B, int Tn, int H, float scale, unsigned int thresh, float inv_keep,
-                 unsigned long long seed, bool do_kv, cudaStream_t st) {
+                 unsigned long long seed, const unsigned long long* seed_offset, bool do_kv, cudaStream_t st) {
   switch (H) {
-    case 128: return xa2::launch_bwd<1>(dO, q, q_ss, kv, phantom, ptr, nmax, out, resid, r_ss, lse, dq, dkv, Dbuf, part, S, B, Tn, scale, thresh, inv_keep, seed, do_kv, st);
-    case 256: return xa2::launch_bwd<2>(dO, q, q_ss, kv, phantom, ptr, nmax, out, resid, r_ss, lse, dq, dkv, Dbuf, part, S, B, Tn, scale, thresh, inv_keep, seed, do_kv, st);
-    default: return xa2::launch_bwd<4>(dO, q, q_ss, kv, phantom, ptr, nmax, out, resid, r_ss, lse, dq, dkv, Dbuf, part, S, B, Tn, scale, thresh, inv_keep, seed, do_kv, st);
+    case 128: return xa2::launch_bwd<1>(dO, q, q_ss, kv, phantom, ptr, nmax, out, resid, r_ss, lse, dq, dkv, Dbuf, part, S, B, Tn, scale, thresh, inv_keep, seed, seed_offset, do_kv, st);
+    case 256: return xa2::launch_bwd<2>(dO, q, q_ss, kv, phantom, ptr, nmax, out, resid, r_ss, lse, dq, dkv, Dbuf, part, S, B, Tn, scale, thresh, inv_keep, seed, seed_offset, do_kv, st);
+    default: return xa2::launch_bwd<4>(dO, q, q_ss, kv, phantom, ptr, nmax, out, resid, r_ss, lse, dq, dkv, Dbuf, part, S, B, Tn, scale, thresh, inv_keep, seed, seed_offset, do_kv, st);
   }
 }
 

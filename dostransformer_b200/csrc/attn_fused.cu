@@ -73,6 +73,7 @@ struct Params {
   unsigned int thresh;
   float inv_keep;
   unsigned long long seed;
+  const unsigned long long* seed_offset;   // optional device word added to seed (dost.h), read before the work-item loop
   float* lse;                    // optional [S * Lq]: log-sum-exp of the scaled scores (the dropout backward recomputes P)
 };
 
@@ -321,6 +322,7 @@ __global__ void __launch_bounds__(kThreads, 1) attn_fwd_kernel(const __grid_cons
     float* xmax = xch;                 // [2][128]
     float* xsum = xch + 2 * BM;        // [2][128]
     const float sl2 = p.scale_log2e;
+    const unsigned long long seed = mask_seed(p.seed, p.seed_offset);
     int local = 0;
     for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x, ++local) {
       const Item it = item_of(p, tile);
@@ -377,7 +379,7 @@ __global__ void __launch_bounds__(kThreads, 1) attn_fwd_kernel(const __grid_cons
       float ph_scale = 1.f;
       if (thresh && it.nph > 0 && it.nb >= cbeg * KC && it.nb < cend * KC) {
         int kept = 0;
-        for (int jj = it.nb; jj < it.nb + it.nph; ++jj) kept += keep_mask(p.seed, mbase + jj, thresh) ? 1 : 0;
+        for (int jj = it.nb; jj < it.nb + it.nph; ++jj) kept += keep_mask(seed, mbase + jj, thresh) ? 1 : 0;
         ph_scale = (float)kept * p.inv_keep / (float)it.nph;
       }
       if (p.lse && half == 0 && it.m0 + row < p.Lq) p.lse[rglob] = mx * 0.6931471805599453f + logf(xsum[row] + xsum[BM + row]);
@@ -391,7 +393,7 @@ __global__ void __launch_bounds__(kThreads, 1) attn_fwd_kernel(const __grid_cons
             const int col = c * KC + j;
             float e = __uint_as_float(r[j]);
             if (col == it.nb) e *= ph_scale;
-            else e = keep_mask(p.seed, mbase + col, thresh) ? e * p.inv_keep : 0.f;
+            else e = keep_mask(seed, mbase + col, thresh) ? e * p.inv_keep : 0.f;
             r[j] = __float_as_uint(e);
           }
         }
@@ -597,11 +599,13 @@ extern "C" int dost_attn_fused_supported(int Lq, int H, int max_keys) {
   return (Lq >= 1 && H >= 64 && H <= 256 && H % 64 == 0 && max_keys >= 1 && max_keys <= fa::kMaxKeys) ? 1 : 0;
 }
 
-extern "C" int dost_attn_fused_fwd(const void* q_hi, const void* q_lo, long long ld_q, const void* k_hi, const void* k_lo, long long ld_k,
-                                   long long k_rows, int S, int Lq, int Lk, int H, const int32_t* k_rowoff, const int32_t* k_count,
-                                   const int32_t* nmax, int max_keys, double scale, const float* residual, long long res_seq_stride,
-                                   float* out, void* p_hi, void* p_lo, long long ld_p, int precision, double drop_p,
-                                   unsigned long long seed, float* lse, dost_stream_t stream) {
+extern "C" int dost_attn_fused_fwd_dseed(const void* q_hi, const void* q_lo, long long ld_q, const void* k_hi, const void* k_lo,
+                                         long long ld_k, long long k_rows, int S, int Lq, int Lk, int H, const int32_t* k_rowoff,
+                                         const int32_t* k_count, const int32_t* nmax, int max_keys, double scale,
+                                         const float* residual, long long res_seq_stride, float* out, void* p_hi, void* p_lo,
+                                         long long ld_p, int precision, double drop_p,
+                                         unsigned long long seed, const unsigned long long* seed_offset, float* lse,
+                                         dost_stream_t stream) {
   DOST_REQUIRE(q_hi && k_hi && out && S > 0 && Lq > 0, "attn_fused_fwd: null pointer / empty problem");
   DOST_REQUIRE(precision == DOST_PREC_BF16X3 || precision == DOST_PREC_BF16, "attn_fused_fwd: precision must be bf16x3 or bf16");
   const bool split3 = precision == DOST_PREC_BF16X3;
@@ -635,6 +639,7 @@ extern "C" int dost_attn_fused_fwd(const void* q_hi, const void* q_lo, long long
   p.thresh = drop_p > 0.0 ? drop_threshold(drop_p) : 0u;
   p.inv_keep = (float)(1.0 / (1.0 - drop_p));
   p.seed = seed;
+  p.seed_offset = seed_offset;
   p.lse = lse;
   int rc = fa::make_map(&maps.q_hi, q_hi, H, Lq, ld_q, fa::BM, S, (long long)Lq * ld_q);
   if (rc == DOST_OK && split3) rc = fa::make_map(&maps.q_lo, q_lo, H, Lq, ld_q, fa::BM, S, (long long)Lq * ld_q);
@@ -674,6 +679,15 @@ extern "C" int dost_attn_fused_fwd(const void* q_hi, const void* q_lo, long long
   }
   cudaStream_t st = (cudaStream_t)stream;
   return split3 ? fa::launch<3>(maps, p, st) : fa::launch<1>(maps, p, st);
+}
+
+extern "C" int dost_attn_fused_fwd(const void* q_hi, const void* q_lo, long long ld_q, const void* k_hi, const void* k_lo, long long ld_k,
+                                   long long k_rows, int S, int Lq, int Lk, int H, const int32_t* k_rowoff, const int32_t* k_count,
+                                   const int32_t* nmax, int max_keys, double scale, const float* residual, long long res_seq_stride,
+                                   float* out, void* p_hi, void* p_lo, long long ld_p, int precision, double drop_p,
+                                   unsigned long long seed, float* lse, dost_stream_t stream) {
+  return dost_attn_fused_fwd_dseed(q_hi, q_lo, ld_q, k_hi, k_lo, ld_k, k_rows, S, Lq, Lk, H, k_rowoff, k_count, nmax, max_keys, scale,
+                                   residual, res_seq_stride, out, p_hi, p_lo, ld_p, precision, drop_p, seed, nullptr, lse, stream);
 }
 
 extern "C" int dost_softmax_bwd_from_planes(const void* p_hi, const void* p_lo, long long ld_pp, const float* dP, long long ld_dp,

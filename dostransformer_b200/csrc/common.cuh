@@ -92,6 +92,11 @@ __device__ __forceinline__ bool keep_mask(unsigned long long seed, unsigned long
   z = z ^ (z >> 31);
   return static_cast<unsigned int>(z >> 32) >= thresh;  // P(keep) = 1 - thresh / 2^32
 }
+// The seed a kernel hands to keep_mask: the launch's seed plus the optional device word seed_offset (dost.h), read once
+// per thread before any loop.  A replayed CUDA graph keeps its launch arguments, so the host rewrites that word instead.
+__device__ __forceinline__ unsigned long long mask_seed(unsigned long long seed, const unsigned long long* seed_offset) {
+  return seed_offset ? seed + *seed_offset : seed;
+}
 inline unsigned int drop_threshold(double p) {
   double t = p * 4294967296.0;
   if (t < 0) t = 0;

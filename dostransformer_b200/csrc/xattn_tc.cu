@@ -123,9 +123,11 @@ __global__ void __launch_bounds__(256) softmax_fwd_kernel(const float* __restric
                                                           const int* __restrict__ nmax_p, long long rows, int B, int Tn, int npad,
                                                           float scale, __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo,
                                                           long long ldp, float* __restrict__ lse, unsigned int* __restrict__ errw,
-                                                          unsigned int thresh, float inv_keep, unsigned long long seed) {
+                                                          unsigned int thresh, float inv_keep, unsigned long long seed,
+                                                          const unsigned long long* __restrict__ seed_offset) {
   const int lane = threadIdx.x & 31;
   const int nmax = *nmax_p;
+  seed = mask_seed(seed, seed_offset);
   for (long long r = blockIdx.x * 8LL + (threadIdx.x >> 5); r < rows; r += (long long)gridDim.x * 8) {
     const int b = (int)((r / Tn) % B);
     int nb = __ldg(ptr + b + 1) - __ldg(ptr + b);
@@ -177,9 +179,11 @@ __global__ void __launch_bounds__(256) softmax_bwd_kernel(const float* __restric
                                                           const float* __restrict__ dP, const int* __restrict__ ptr,
                                                           const int* __restrict__ nmax_p, long long rows, int B, int Tn, int npad,
                                                           float scale, __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo,
-                                                          long long ldp, unsigned int thresh, float inv_keep, unsigned long long seed) {
+                                                          long long ldp, unsigned int thresh, float inv_keep, unsigned long long seed,
+                                                          const unsigned long long* __restrict__ seed_offset) {
   const int lane = threadIdx.x & 31;
   const int nmax = *nmax_p;
+  seed = mask_seed(seed, seed_offset);
   for (long long r = blockIdx.x * 8LL + (threadIdx.x >> 5); r < rows; r += (long long)gridDim.x * 8) {
     const int b = (int)((r / Tn) % B);
     const int nb = min(__ldg(ptr + b + 1) - __ldg(ptr + b), npad - 1);
@@ -267,9 +271,10 @@ static inline int npl_for(long long ldp) {
   return p;
 }
 
-extern "C" int dost_xattn_softmax_fwd(const float* scores, const int32_t* ptr, const int32_t* nmax, long long rows, int B, int T,
-                                      int npad, double scale, void* hi, void* lo, long long ldp, float* lse, double drop_p,
-                                      unsigned long long seed, dost_stream_t stream) {
+extern "C" int dost_xattn_softmax_fwd_dseed(const float* scores, const int32_t* ptr, const int32_t* nmax, long long rows, int B,
+                                            int T, int npad, double scale, void* hi, void* lo, long long ldp, float* lse,
+                                            double drop_p, unsigned long long seed, const unsigned long long* seed_offset,
+                                            dost_stream_t stream) {
   DOST_REQUIRE(scores && ptr && nmax && hi && lse && rows > 0 && npad > 0 && ldp >= npad && ldp <= 1024, "xattn_softmax_fwd: bad args");
   cudaStream_t st = (cudaStream_t)stream;
   const int npl = npl_for(ldp);
@@ -278,13 +283,20 @@ extern "C" int dost_xattn_softmax_fwd(const float* scores, const int32_t* ptr, c
   const unsigned int thresh = drop_p > 0.0 ? drop_threshold(drop_p) : 0u;
   const float inv_keep = (float)(1.0 / (1.0 - drop_p));
   DOST_XTC_DISPATCH(softmax_fwd_kernel, scores, ptr, nmax, rows, B, T, npad, (float)scale, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo, ldp, lse,
-                    device_error_words(), thresh, inv_keep, seed)
+                    device_error_words(), thresh, inv_keep, seed, seed_offset)
   return check_launch("xattn_softmax_fwd");
 }
 
-extern "C" int dost_xattn_softmax_bwd(const float* scores, const float* lse, const float* dP, const int32_t* ptr, const int32_t* nmax,
-                                      long long rows, int B, int T, int npad, double scale, void* hi, void* lo, long long ldp,
-                                      double drop_p, unsigned long long seed, dost_stream_t stream) {
+extern "C" int dost_xattn_softmax_fwd(const float* scores, const int32_t* ptr, const int32_t* nmax, long long rows, int B, int T,
+                                      int npad, double scale, void* hi, void* lo, long long ldp, float* lse, double drop_p,
+                                      unsigned long long seed, dost_stream_t stream) {
+  return dost_xattn_softmax_fwd_dseed(scores, ptr, nmax, rows, B, T, npad, scale, hi, lo, ldp, lse, drop_p, seed, nullptr, stream);
+}
+
+extern "C" int dost_xattn_softmax_bwd_dseed(const float* scores, const float* lse, const float* dP, const int32_t* ptr,
+                                            const int32_t* nmax, long long rows, int B, int T, int npad, double scale, void* hi,
+                                            void* lo, long long ldp, double drop_p, unsigned long long seed,
+                                            const unsigned long long* seed_offset, dost_stream_t stream) {
   DOST_REQUIRE(scores && lse && dP && ptr && nmax && hi && rows > 0 && npad > 0 && ldp >= npad && ldp <= 1024, "xattn_softmax_bwd: bad args");
   cudaStream_t st = (cudaStream_t)stream;
   const int npl = npl_for(ldp);
@@ -293,6 +305,12 @@ extern "C" int dost_xattn_softmax_bwd(const float* scores, const float* lse, con
   const unsigned int thresh = drop_p > 0.0 ? drop_threshold(drop_p) : 0u;
   const float inv_keep = (float)(1.0 / (1.0 - drop_p));
   DOST_XTC_DISPATCH(softmax_bwd_kernel, scores, lse, dP, ptr, nmax, rows, B, T, npad, (float)scale, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo,
-                    ldp, thresh, inv_keep, seed)
+                    ldp, thresh, inv_keep, seed, seed_offset)
   return check_launch("xattn_softmax_bwd");
+}
+
+extern "C" int dost_xattn_softmax_bwd(const float* scores, const float* lse, const float* dP, const int32_t* ptr, const int32_t* nmax,
+                                      long long rows, int B, int T, int npad, double scale, void* hi, void* lo, long long ldp,
+                                      double drop_p, unsigned long long seed, dost_stream_t stream) {
+  return dost_xattn_softmax_bwd_dseed(scores, lse, dP, ptr, nmax, rows, B, T, npad, scale, hi, lo, ldp, drop_p, seed, nullptr, stream);
 }

@@ -20,8 +20,11 @@ step, the tensor maps, workspaces and every intermediate live in the graph's pri
   (the dummies never enter the loss; their padding-length contribution is excluded, see there).
 * Data parallel: the gradient all-reduce runs right after the replay on the same stream (one flat NCCL call; a step this
   short has nothing left to overlap it with).
-
-Dropout > 0 draws a fresh host seed per step and therefore stays eager.
+* Attention dropout: the captured kernels read their seed offset from one int64 word on the device (``nn_core.device_seed``,
+  warm-up and capture run in that mode and draw no host random number).  Every call of a training model with
+  ``attn_drop > 0`` draws the one host base an eager step draws and writes ``base << 20`` into the word on the current
+  stream before the replay: a fresh mask per step, the same masks, loss and gradients as the eager step after the same
+  ``torch.manual_seed``, and the same CPU random-number stream.
 """
 from __future__ import annotations
 
@@ -32,6 +35,7 @@ import torch
 
 from . import _lib as L
 from . import ops
+from .nn_core import device_seed, draw_dropout_base
 from .synthetic import CrystalBatch
 
 
@@ -87,6 +91,7 @@ class GraphedStep:
         self.launches = 0          # kernels of this library executed by replays (captured count x replays)
         self._params = [p for p in model.parameters()]
         self._stream = None
+        self._seed_word = None     # int64 [1] on the model's device: the dropout seed offset the captured kernels read
         from .nn_core import gemm_weights
         wid = {id(w) for w in gemm_weights(model)}
         self._weight_names = [n for n, p in model.named_parameters() if id(p) in wid]
@@ -125,9 +130,6 @@ class GraphedStep:
         loss.backward()
         return loss.detach()       # (a loss with its grad_fn would keep the whole autograd graph of a capture alive)
 
-    def _capturable(self) -> bool:
-        return not (self.train and getattr(self.model, "attn_drop", 0.0) > 0.0)
-
     def _capture(self, g) -> _Entry:
         dev = g.x.device
         e = _Entry()
@@ -147,7 +149,7 @@ class GraphedStep:
         s = self._stream
         s.wait_stream(torch.cuda.current_stream(dev))
         e.leaves = None
-        with torch.cuda.stream(s):
+        with torch.cuda.stream(s), device_seed(self._seed_word):
             if self.train:
                 e.leaves = {n: p.detach().requires_grad_(p.requires_grad) for n, p in self.model.named_parameters()}
             self._eager(e.static, leaves=e.leaves)
@@ -162,7 +164,7 @@ class GraphedStep:
         # capture-unsafe calls
         import os
         pool = None if os.environ.get("DOST_GRAPH_PRIVATE_POOLS") else self._pool
-        with torch.cuda.graph(e.graph, pool=pool, stream=s, capture_error_mode="thread_local"):
+        with torch.cuda.graph(e.graph, pool=pool, stream=s, capture_error_mode="thread_local"), device_seed(self._seed_word):
             e.out = self._eager(e.static, refresh=True, leaves=e.leaves)
         e.launches = L.launch_count() - l0
         # the gradient buffers this graph writes (graph-pool memory, fixed addresses): re-attached on every replay, since
@@ -175,13 +177,16 @@ class GraphedStep:
         return e
 
     def __call__(self, g):
-        if not self._capturable():
-            out = self._eager(g)
-            if self.train and self.world > 1:
-                allreduce_gradients(self._params, self.group)
-            return out
-        # (the model's data-parallel padding length is a host integer baked into the captured launches: part of the key)
-        sig = batch_signature(g) + (("model_max_num_nodes", getattr(self.model, "max_num_nodes", None)),)
+        # (the model's data-parallel padding length and its dropout probability are host values baked into the captured
+        # launches, and training decides whether dropout runs at all: part of the key)
+        attn_drop = float(getattr(self.model, "attn_drop", 0.0))
+        sig = batch_signature(g) + (("model_max_num_nodes", getattr(self.model, "max_num_nodes", None)),
+                                    ("attn_drop", attn_drop), ("training", self.model.training))
+        if self.model.training and attn_drop > 0.0:
+            # exactly the host draw of the eager step (nn_core._Seeds); a capture draws nothing.  No sync, no device read.
+            if self._seed_word is None:
+                self._seed_word = torch.zeros(1, dtype=torch.int64, device=self._params[0].device)
+            self._seed_word.fill_(draw_dropout_base() << 20)
         e = self._entries.get(sig)
         if e is None:
             if len(self._entries) >= self.max_graphs:

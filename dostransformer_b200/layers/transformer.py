@@ -37,7 +37,7 @@ class TransformerEncoder(K.EnergyEncoderParams):
             ln0 = layer.layer_norms[0]
             k = ops.layer_norm(kv0, ln0.weight, ln0.bias)
             q = ops.layer_norm(x, ln0.weight, ln0.bias)
-            y = ops.self_attention(q, k, x, seeds.p, seeds.next())
+            y = ops.self_attention(q, k, x, seeds.p, *seeds.next())
             x = K._ffn(layer, y)
         x = ops.layer_norm(x, self.layer_norm.weight, self.layer_norm.bias)
         return x.transpose(0, 1)

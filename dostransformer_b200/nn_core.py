@@ -9,7 +9,9 @@ in/out projections, phonon ``alpha``) are created too, never used, and never rec
 from __future__ import annotations
 
 import os
-from typing import Optional
+import threading
+from contextlib import contextmanager
+from typing import Optional, Tuple
 
 import torch
 from torch import nn
@@ -137,15 +139,40 @@ def _ffn(layer, y):
     return ops.linear([(h, None)], layer.fc2.weight, layer.fc2.bias, residual=y2d).view(y.shape)
 
 
+def draw_dropout_base() -> int:
+    """The one host random number a forward with attention dropout consumes (torch's CPU generator): attention call n of
+    that forward masks with seed (base << 20) + n."""
+    return int(torch.randint(0, 2 ** 31 - 1, (1,)).item())
+
+
+_device_seed = threading.local()
+
+
+@contextmanager
+def device_seed(word: torch.Tensor):
+    """Forwards inside this block draw no host base: attention call n passes seed n and ``word`` (a 1-element int64 tensor
+    on the model's device) as its seed offset, so the kernels mask with n + word.  Writing ``base << 20`` into the word
+    before the kernels run reproduces the masks of an eager forward that drew ``base`` (graphed.GraphedStep does this
+    before every replay).  Per thread."""
+    prev = getattr(_device_seed, "word", None)
+    _device_seed.word = word
+    try:
+        yield word
+    finally:
+        _device_seed.word = prev
+
+
 class _Seeds:
     def __init__(self, drop_p: float, training: bool):
         self.p = drop_p if training else 0.0
-        self.base = int(torch.randint(0, 2 ** 31 - 1, (1,)).item()) if self.p > 0 else 0
+        self.word = getattr(_device_seed, "word", None) if self.p > 0 else None
+        self.base = draw_dropout_base() if self.p > 0 and self.word is None else 0
         self.n = 0
 
-    def next(self) -> int:
+    def next(self) -> Tuple[int, Optional[torch.Tensor]]:
+        """(seed, seed_offset) of the next attention call."""
         self.n += 1
-        return (self.base << 20) + self.n
+        return (self.base << 20) + self.n, self.word
 
 
 def cross_stack(enc: EnergyEncoderParams, q, x_nodes, graph: ops.CrystalGraph, S: int, T: int, seeds: _Seeds):
@@ -155,7 +182,7 @@ def cross_stack(enc: EnergyEncoderParams, q, x_nodes, graph: ops.CrystalGraph, S
         ln0 = layer.layer_norms[0]
         kv = ops.layer_norm(x_nodes, ln0.weight, ln0.bias)
         q_ln, q_res = ops.layer_norm(q, ln0.weight, ln0.bias, want_planes=q.dim() == 3, with_residual=True)
-        y = ops.cross_attention(q_ln, kv, ln0.bias, q_res, graph, S, seeds.p, seeds.next())
+        y = ops.cross_attention(q_ln, kv, ln0.bias, q_res, graph, S, seeds.p, *seeds.next())
         q = _ffn(layer, y)
     return ops.layer_norm(q, enc.layer_norm.weight, enc.layer_norm.bias)
 
@@ -172,7 +199,7 @@ def self_stack(enc: EnergyEncoderParams, x0, seeds: _Seeds):
         else:
             k = ops.layer_norm(x0, ln0.weight, ln0.bias, want_planes=True)
             q, x_res = ops.layer_norm(x, ln0.weight, ln0.bias, want_planes=True, with_residual=True)
-        y = ops.self_attention(q, k, x_res, seeds.p, seeds.next())
+        y = ops.self_attention(q, k, x_res, seeds.p, *seeds.next())
         x = _ffn(layer, y)
     return ops.layer_norm(x, enc.layer_norm.weight, enc.layer_norm.bias)
 

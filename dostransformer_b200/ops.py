@@ -1363,10 +1363,11 @@ def segment_reduce(src, csr: CSR, mean: bool = False):
 # =====================================================================================================
 class _CrossAttention(torch.autograd.Function):
     """out = resid + softmax(q kv^T / sqrt(H)) kv over the atoms of each sequence's crystal plus
-    (nmax - n_b) phantom keys equal to ``phantom``.  q/resid: [S,T,H] or [T,H] (broadcast over S)."""
+    (nmax - n_b) phantom keys equal to ``phantom``.  q/resid: [S,T,H] or [T,H] (broadcast over S).
+    seed_offset: optional 1-element int64 device tensor added to ``seed`` by the kernels (dost.h, ``_dseed`` entry points)."""
 
     @staticmethod
-    def forward(ctx, q, kv, phantom, resid, graph: CrystalGraph, S: int, drop_p: float, seed: int):
+    def forward(ctx, q, kv, phantom, resid, graph: CrystalGraph, S: int, drop_p: float, seed: int, seed_offset=None):
         H = kv.shape[1]
         T = q.shape[-2]
         q, resid = q.contiguous(), resid.contiguous()
@@ -1375,11 +1376,11 @@ class _CrossAttention(torch.autograd.Function):
         out = torch.empty(S, T, H, dtype=kv.dtype, device=kv.device)
         lse = torch.empty(S, T, dtype=torch.float32, device=kv.device)
         scale = float(H) ** -0.5
-        L.check(L.lib().dost_xattn_fwd(L.dt(kv), L.p(q), q_ss, L.p(kv), L.p(phantom), L.p(graph.ptr), L.p(graph.nmax),
-                                       L.p(resid), r_ss, L.p(out), L.p(lse), S, graph.B, T, H, scale, drop_p, seed,
-                                       L.stream()), "xattn_fwd")
+        L.check(L.lib().dost_xattn_fwd_dseed(L.dt(kv), L.p(q), q_ss, L.p(kv), L.p(phantom), L.p(graph.ptr), L.p(graph.nmax),
+                                             L.p(resid), r_ss, L.p(out), L.p(lse), S, graph.B, T, H, scale, drop_p, seed,
+                                             L.p(seed_offset), L.stream()), "xattn_fwd")
         ctx.save_for_backward(q, kv, phantom, resid, out, lse)
-        ctx.graph, ctx.S, ctx.drop_p, ctx.seed = graph, S, drop_p, seed
+        ctx.graph, ctx.S, ctx.drop_p, ctx.seed, ctx.seed_offset = graph, S, drop_p, seed, seed_offset
         ctx.q_ss, ctx.r_ss = q_ss, r_ss
         return out
 
@@ -1397,13 +1398,13 @@ class _CrossAttention(torch.autograd.Function):
         lib = L.lib()
         nb = lib.dost_xattn_bwd_workspace_bytes(L.dt(kv), S, T, H)
         ws = _ws(nb, dev)
-        L.check(lib.dost_xattn_bwd(L.dt(kv), L.p(d_out), L.p(q), ctx.q_ss, L.p(kv), L.p(phantom), L.p(g.ptr), L.p(g.batch),
-                                   L.p(g.nmax), L.p(out), L.p(resid), ctx.r_ss, L.p(lse), L.p(dq), L.p(dkv), L.p(dph),
-                                   S, g.B, T, H, g.N, float(H) ** -0.5, ctx.drop_p, ctx.seed, L.p(ws), nb, L.stream()),
-                "xattn_bwd")
+        L.check(lib.dost_xattn_bwd_dseed(L.dt(kv), L.p(d_out), L.p(q), ctx.q_ss, L.p(kv), L.p(phantom), L.p(g.ptr),
+                                         L.p(g.batch), L.p(g.nmax), L.p(out), L.p(resid), ctx.r_ss, L.p(lse), L.p(dq), L.p(dkv),
+                                         L.p(dph), S, g.B, T, H, g.N, float(H) ** -0.5, ctx.drop_p, ctx.seed,
+                                         L.p(ctx.seed_offset), L.p(ws), nb, L.stream()), "xattn_bwd")
         d_q = dq if ctx.q_ss else colsum(dq.view(S, T * H)).view(T, H)
         d_resid = d_out if ctx.r_ss else colsum(d_out.view(S, T * H)).view(T, H)
-        return d_q, dkv, dph, d_resid, None, None, None, None
+        return d_q, dkv, dph, d_resid, None, None, None, None, None
 
 
 def _grad_planes(d_out: torch.Tensor, rows: int, cols: int) -> Planes:
@@ -1425,12 +1426,13 @@ def fused_attention_ok(H: int, max_keys: int, drop_p: float = 0.0) -> bool:
 
 
 def _fused_attention_fwd(qp: Planes, kp: Planes, k_rows: int, S: int, Lq: int, Lk: int, H: int, rowoff, count, nmax, max_keys: int,
-                         resid2d, res_seq_stride: int, out2d, pp: Optional[Planes], drop_p: float = 0.0, seed: int = 0, lse=None):
-    L.check(L.lib().dost_attn_fused_fwd(L.p(qp.hi), L.p(qp.lo), qp.ld, L.p(kp.hi), L.p(kp.lo), kp.ld, k_rows, S, Lq, Lk, H,
-                                        L.p(rowoff), L.p(count), L.p(nmax), max_keys, float(H) ** -0.5, L.p(resid2d),
-                                        res_seq_stride, L.p(out2d), L.p(pp.hi) if pp is not None else None,
-                                        L.p(pp.lo) if pp is not None else None, pp.ld if pp is not None else 0, _PRECISION,
-                                        float(drop_p), int(seed), L.p(lse), L.stream()), "attn_fused_fwd")
+                         resid2d, res_seq_stride: int, out2d, pp: Optional[Planes], drop_p: float = 0.0, seed: int = 0, lse=None,
+                         seed_offset=None):
+    L.check(L.lib().dost_attn_fused_fwd_dseed(L.p(qp.hi), L.p(qp.lo), qp.ld, L.p(kp.hi), L.p(kp.lo), kp.ld, k_rows, S, Lq, Lk, H,
+                                              L.p(rowoff), L.p(count), L.p(nmax), max_keys, float(H) ** -0.5, L.p(resid2d),
+                                              res_seq_stride, L.p(out2d), L.p(pp.hi) if pp is not None else None,
+                                              L.p(pp.lo) if pp is not None else None, pp.ld if pp is not None else 0, _PRECISION,
+                                              float(drop_p), int(seed), L.p(seed_offset), L.p(lse), L.stream()), "attn_fused_fwd")
 
 
 def _ds_from_planes(pp: Planes, dP2d: torch.Tensor, rows: int, cols: int, scale: float, dsp: Planes):
@@ -1446,7 +1448,8 @@ class _CrossAttentionTC(torch.autograd.Function):
     kernel when it writes the probability planes.  Needs the padding length on the host."""
 
     @staticmethod
-    def forward(ctx, q, kv, phantom, resid, graph: CrystalGraph, qpl: Optional[Planes], S: int, drop_p: float = 0.0, seed: int = 0):
+    def forward(ctx, q, kv, phantom, resid, graph: CrystalGraph, qpl: Optional[Planes], S: int, drop_p: float = 0.0, seed: int = 0,
+                seed_offset=None):
         N, H = kv.shape
         B = graph.B
         T = q.shape[-2]
@@ -1469,7 +1472,7 @@ class _CrossAttentionTC(torch.autograd.Function):
         r2 = resid.view(-1, H)
         ctx.graph, ctx.prec, ctx.npad = graph, _PRECISION, npad
         ctx.bcast_q, ctx.bcast_r, ctx.T, ctx.S = bcast_q, resid.dim() == 2, T, S
-        ctx.drop_p, ctx.seed = drop_p, seed
+        ctx.drop_p, ctx.seed, ctx.seed_offset = drop_p, seed, seed_offset
         ctx.fused = fused_attention_ok(H, graph.nkeys_host, drop_p)
         if ctx.fused:
             # one kernel: scores stay in TMEM, the probabilities leave only as the operand planes the backward needs
@@ -1478,7 +1481,7 @@ class _CrossAttentionTC(torch.autograd.Function):
             # with dropout the planes hold the dropped-out probabilities; the backward recomputes P from the log-sum-exp
             lse = torch.empty(S * T, dtype=torch.float32, device=dev) if (need and drop_p > 0) else None
             _fused_attention_fwd(qp, kvp, N + B, S, T, 0, H, ptr_ext, n_ext, graph.nmax, graph.nkeys_host, r2,
-                                 0 if resid.dim() == 2 else T * H, out.view(S * T, H), pp, drop_p, seed, lse)
+                                 0 if resid.dim() == 2 else T * H, out.view(S * T, H), pp, drop_p, seed, lse, seed_offset)
             if need:
                 ctx.save_for_backward(kv, phantom, None, lse, *_planes_save(qp), *_planes_save(kvp), *_planes_save(pp))
             return out
@@ -1488,8 +1491,9 @@ class _CrossAttentionTC(torch.autograd.Function):
         pp = empty_planes(S * T, npad, dev, _with_lo())
         lse = torch.empty(S * T, dtype=torch.float32, device=dev)
         scale = float(H) ** -0.5
-        L.check(lib.dost_xattn_softmax_fwd(L.p(scores), L.p(graph.ptr), L.p(graph.nmax), S * T, B, T, npad, scale, L.p(pp.hi),
-                                           L.p(pp.lo), pp.ld, L.p(lse), drop_p, seed, L.stream()), "xattn_softmax_fwd")
+        L.check(lib.dost_xattn_softmax_fwd_dseed(L.p(scores), L.p(graph.ptr), L.p(graph.nmax), S * T, B, T, npad, scale, L.p(pp.hi),
+                                                 L.p(pp.lo), pp.ld, L.p(lse), drop_p, seed, L.p(seed_offset), L.stream()),
+                "xattn_softmax_fwd")
         gemm_planes(M=T, N=H, K=npad, a=[pp], a_mode=L.KC, b=kvp, b_mode=L.MC, b_rows=N + B, out=out.view(S * T, H), residual=r2,
                     batch=S, a_bstride=T * pp.ld, c_bstride=T * H, res_bstride=(0 if resid.dim() == 2 else T * H),
                     b_rowoff=ptr_ext)
@@ -1523,9 +1527,9 @@ class _CrossAttentionTC(torch.autograd.Function):
             if ctx.fused and ctx.drop_p == 0:      # probabilities from their saved planes (the phantom column behaves like one key of its total mass)
                 _ds_from_planes(pp, dP, S * T, npad, float(H) ** -0.5, dsp)
             else:
-                L.check(lib.dost_xattn_softmax_bwd(L.p(scores), L.p(lse), L.p(dP), L.p(g.ptr), L.p(g.nmax), S * T, B, T, npad,
-                                                   float(H) ** -0.5, L.p(dsp.hi), L.p(dsp.lo), dsp.ld, ctx.drop_p, ctx.seed,
-                                                   L.stream()), "xattn_softmax_bwd")
+                L.check(lib.dost_xattn_softmax_bwd_dseed(L.p(scores), L.p(lse), L.p(dP), L.p(g.ptr), L.p(g.nmax), S * T, B, T, npad,
+                                                         float(H) ** -0.5, L.p(dsp.hi), L.p(dsp.lo), dsp.ld, ctx.drop_p, ctx.seed,
+                                                         L.p(ctx.seed_offset), L.stream()), "xattn_softmax_bwd")
             # dQ = dS k
             dq = torch.empty(S, T, H, dtype=torch.float32, device=dev)
             gemm_planes(M=T, N=H, K=npad, a=[dsp], a_mode=L.KC, b=kvp, b_mode=L.MC, b_rows=N + B, out=dq.view(S * T, H), batch=S,
@@ -1547,7 +1551,7 @@ class _CrossAttentionTC(torch.autograd.Function):
                 dph = colsum(dbrows)
                 d_q = colsum(dq.view(S, T * H)).view(T, H) if ctx.bcast_q else dq
                 d_resid = colsum(d_out.view(S, T * H)).view(T, H) if ctx.bcast_r else d_out
-                return d_q, dkv, dph, d_resid, None, None, None, None, None
+                return d_q, dkv, dph, d_resid, None, None, None, None, None, None
             dext = torch.empty(N + B, H, dtype=torch.float32, device=dev)
             p1, n1 = g.ragged(1)
             for rep in range(reps):
@@ -1561,7 +1565,7 @@ class _CrossAttentionTC(torch.autograd.Function):
             dph = colsum(dbrows)
             d_q = colsum(dq.view(S, T * H)).view(T, H) if ctx.bcast_q else dq
             d_resid = colsum(d_out.view(S, T * H)).view(T, H) if ctx.bcast_r else d_out
-        return d_q, dkv, dph, d_resid, None, None, None, None, None
+        return d_q, dkv, dph, d_resid, None, None, None, None, None, None
 
 
 def _rows(pl: Planes, r0: int, r1: int) -> Planes:
@@ -1569,15 +1573,23 @@ def _rows(pl: Planes, r0: int, r1: int) -> Planes:
     return Planes(pl.hi[r0:r1], pl.lo[r0:r1] if pl.lo is not None else None, r1 - r0, pl.cols)
 
 
-def cross_attention(q, kv, phantom, resid, graph: CrystalGraph, S: int, drop_p: float = 0.0, seed: int = 0):
+def _check_seed_offset(seed_offset) -> None:
+    if seed_offset is not None and (seed_offset.dtype != torch.int64 or seed_offset.numel() != 1):
+        raise ValueError("seed_offset must be a 1-element int64 CUDA tensor")
+
+
+def cross_attention(q, kv, phantom, resid, graph: CrystalGraph, S: int, drop_p: float = 0.0, seed: int = 0, seed_offset=None):
+    """Energy -> atom cross attention (see _CrossAttention).  Dropout masks with ``seed``, plus the value of ``seed_offset``
+    (optional 1-element int64 CUDA tensor) read on the device when the kernels run: a captured step rewrites it per replay."""
+    _check_seed_offset(seed_offset)
     H = kv.shape[1]
     if (tc_active(kv) and H % 128 == 0 and S % graph.B == 0 and graph.nmax_host is not None
             and graph.nkeys_host <= 1016 and q.shape[-2] >= 64 and not L.switch("DOST_NO_XATTN_TC")
             and (q.dim() == 3 or S == graph.B)):
-        out = _CrossAttentionTC.apply(q, kv, phantom, resid, graph, _planes3(q), S, drop_p, seed)
+        out = _CrossAttentionTC.apply(q, kv, phantom, resid, graph, _planes3(q), S, drop_p, seed, seed_offset)
         out._dost_attn_out = True        # (its backward takes the incoming gradient as operand planes, see _grad_planes)
         return out
-    return _CrossAttention.apply(q, kv, phantom, resid, graph, S, drop_p, seed)
+    return _CrossAttention.apply(q, kv, phantom, resid, graph, S, drop_p, seed, seed_offset)
 
 
 # =====================================================================================================
@@ -1587,7 +1599,7 @@ class _SelfAttention(torch.autograd.Function):
     """out = resid + softmax_fp32(q k^T / sqrt(H)) k, per sequence; q, resid: [S,Lq,H], k (= v): [S,Lk,H]."""
 
     @staticmethod
-    def forward(ctx, q, k, resid, drop_p: float, seed: int):
+    def forward(ctx, q, k, resid, drop_p: float, seed: int, seed_offset=None):
         S, Lq, H = q.shape
         Lk = k.shape[1]
         qpl, kpl = _planes3(q), _planes3(k)
@@ -1599,14 +1611,14 @@ class _SelfAttention(torch.autograd.Function):
             # the four batched contractions on the TMA-fed tensor-core kernel (3-D tensor maps, one batch per sequence)
             qp = qpl if qpl is not None else split_planes(q.view(S * Lq, H))
             kp = kpl if kpl is not None else split_planes(k.view(S * Lk, H))
-            ctx.drop_p, ctx.seed, ctx.prec = drop_p, seed, _PRECISION
+            ctx.drop_p, ctx.seed, ctx.seed_offset, ctx.prec = drop_p, seed, seed_offset, _PRECISION
             ctx.dims = (S, Lq, Lk, H, Lp)
             ctx.fused = fused_attention_ok(H, Lk, drop_p)
             if ctx.fused:
                 out = torch.empty(S, Lq, H, dtype=dtype, device=dev)
                 pdp = empty_planes(S * Lq, Lk, dev, _with_lo()) if any(ctx.needs_input_grad[:3]) else None
                 _fused_attention_fwd(qp, kp, S * Lk, S, Lq, Lk, H, None, None, None, Lk, resid.view(S * Lq, H), Lq * H,
-                                     out.view(S * Lq, H), pdp, drop_p, seed)
+                                     out.view(S * Lq, H), pdp, drop_p, seed, seed_offset=seed_offset)
                 if pdp is not None:
                     ctx.save_for_backward(None, None, *_planes_save(qp), *_planes_save(kp), *_planes_save(pdp))
                 return out
@@ -1615,8 +1627,9 @@ class _SelfAttention(torch.autograd.Function):
                         batch=S, a_bstride=Lq * qp.ld, b_bstride=Lk * kp.ld, c_bstride=Lq * Lp)
             pd = torch.empty_like(scores) if drop_p > 0 else scores
             pdp = empty_planes(S * Lq, Lk, dev, _with_lo())      # probabilities straight into operand planes
-            L.check(L.lib().dost_softmax_fwd_planes(L.p(scores), L.p(scores), L.p(pd), S * Lq, Lk, Lp, float(H) ** -0.5, drop_p,
-                                                    seed, L.p(pdp.hi), L.p(pdp.lo), pdp.ld, L.stream()), "softmax_fwd_planes")
+            L.check(L.lib().dost_softmax_fwd_planes_dseed(L.p(scores), L.p(scores), L.p(pd), S * Lq, Lk, Lp, float(H) ** -0.5,
+                                                          drop_p, seed, L.p(seed_offset), L.p(pdp.hi), L.p(pdp.lo), pdp.ld,
+                                                          L.stream()), "softmax_fwd_planes")
             out = torch.empty(S, Lq, H, dtype=dtype, device=dev)
             gemm_planes(M=Lq, N=H, K=Lk, a=[pdp], a_mode=L.KC, b=kp, b_mode=L.MC, out=out.view(S * Lq, H),
                         residual=resid.view(S * Lq, H), batch=S, a_bstride=Lq * pdp.ld, b_bstride=Lk * kp.ld, c_bstride=Lq * H,
@@ -1627,13 +1640,13 @@ class _SelfAttention(torch.autograd.Function):
         gemm_raw(M=Lq, N=Lk, K=H, a=[(q.view(S * Lq, H), None)], a_mode=L.KC, b=k.view(S * Lk, H), b_mode=L.KC,
                  out=scores, batch=S, a_bstride=Lq * H, b_bstride=Lk * H, c_bstride=Lq * Lp, ldc=Lp)
         pd = torch.empty_like(scores) if drop_p > 0 else scores
-        L.check(L.lib().dost_softmax_fwd(L.dt(q), L.p(scores), L.p(scores), L.p(pd), S * Lq, Lk, Lp, float(H) ** -0.5,
-                                         drop_p, seed, L.stream()), "softmax_fwd")
+        L.check(L.lib().dost_softmax_fwd_dseed(L.dt(q), L.p(scores), L.p(scores), L.p(pd), S * Lq, Lk, Lp, float(H) ** -0.5,
+                                               drop_p, seed, L.p(seed_offset), L.stream()), "softmax_fwd")
         out = torch.empty(S, Lq, H, dtype=dtype, device=dev)
         gemm_raw(M=Lq, N=H, K=Lk, a=[(pd.view(S * Lq, Lp), None)], a_mode=L.KC, b=k.view(S * Lk, H), b_mode=L.MC,
                  out=out, residual=resid, batch=S, a_bstride=Lq * Lp, b_bstride=Lk * H, c_bstride=Lq * H, ldc=H, lda=Lp)
         ctx.save_for_backward(q, k, scores, pd if drop_p > 0 else None)
-        ctx.drop_p, ctx.seed, ctx.prec = drop_p, seed, _PRECISION
+        ctx.drop_p, ctx.seed, ctx.seed_offset, ctx.prec = drop_p, seed, seed_offset, _PRECISION
         return out
 
     @staticmethod
@@ -1654,8 +1667,8 @@ class _SelfAttention(torch.autograd.Function):
         gemm_raw(M=Lq, N=Lk, K=H, a=[(d_out.view(S * Lq, H), None)], a_mode=L.KC, b=k.view(S * Lk, H), b_mode=L.KC,
                  out=dpd, batch=S, a_bstride=Lq * H, b_bstride=Lk * H, c_bstride=Lq * Lp, ldc=Lp, prec=ctx.prec)
         ds = dpd  # in place
-        L.check(L.lib().dost_softmax_bwd(L.dt(q), L.p(prob), L.p(dpd), L.p(ds), S * Lq, Lk, Lp, scale, ctx.drop_p,
-                                         ctx.seed, L.stream()), "softmax_bwd")
+        L.check(L.lib().dost_softmax_bwd_dseed(L.dt(q), L.p(prob), L.p(dpd), L.p(ds), S * Lq, Lk, Lp, scale, ctx.drop_p,
+                                               ctx.seed, L.p(ctx.seed_offset), L.stream()), "softmax_bwd")
         # dQ = dS k
         dq = torch.empty(S, Lq, H, dtype=dtype, device=dev)
         gemm_raw(M=Lq, N=H, K=Lk, a=[(ds.view(S * Lq, Lp), None)], a_mode=L.KC, b=k.view(S * Lk, H), b_mode=L.MC,
@@ -1667,7 +1680,7 @@ class _SelfAttention(torch.autograd.Function):
         gemm_raw(M=Lk, N=H, K=Lq, a=[(pd.view(S * Lq, Lp), None)], a_mode=L.MC, b=d_out.view(S * Lq, H), b_mode=L.MC,
                  out=dk, accumulate=True, batch=S, a_bstride=Lq * Lp, b_bstride=Lq * H, c_bstride=Lk * H, ldc=H, lda=Lp,
                  prec=ctx.prec)
-        return dq, dk, d_out, None, None
+        return dq, dk, d_out, None, None, None
 
 
 def _self_attention_backward_planes(ctx, d_out):
@@ -1693,8 +1706,9 @@ def _self_attention_backward_planes(ctx, d_out):
     if ctx.fused and ctx.drop_p == 0:
         _ds_from_planes(pdp, dpd.view(S * Lq, Lp), S * Lq, Lk, scale, dsp)
     else:
-        L.check(L.lib().dost_softmax_bwd_planes(L.p(prob), L.p(dpd), None, S * Lq, Lk, Lp, scale, ctx.drop_p, ctx.seed, L.p(dsp.hi),
-                                                L.p(dsp.lo), dsp.ld, L.stream()), "softmax_bwd_planes")
+        L.check(L.lib().dost_softmax_bwd_planes_dseed(L.p(prob), L.p(dpd), None, S * Lq, Lk, Lp, scale, ctx.drop_p, ctx.seed,
+                                                      L.p(ctx.seed_offset), L.p(dsp.hi), L.p(dsp.lo), dsp.ld, L.stream()),
+                "softmax_bwd_planes")
     # dQ = dS k
     dq = torch.empty(S, Lq, H, dtype=torch.float32, device=dev)
     gemm_planes(M=Lq, N=H, K=Lk, a=[dsp], a_mode=L.KC, b=kp, b_mode=L.MC, out=dq.view(S * Lq, H), batch=S,
@@ -1705,7 +1719,7 @@ def _self_attention_backward_planes(ctx, d_out):
                 a_bstride=Lq * dsp.ld, b_bstride=Lq * qp.ld, c_bstride=Lk * H)
     gemm_planes(M=Lk, N=H, K=Lq, a=[pdp], a_mode=L.MC, b=dop, b_mode=L.MC, out=dk.view(S * Lk, H), accumulate=True, batch=S,
                 a_bstride=Lq * pdp.ld, b_bstride=Lq * dop.ld, c_bstride=Lk * H)
-    return dq, dk, d_out, None, None
+    return dq, dk, d_out, None, None, None
 
 
 _SelfAttention._backward_planes = staticmethod(_self_attention_backward_planes)
@@ -1725,8 +1739,10 @@ def _planes3(t: torch.Tensor) -> Optional[Planes]:
     return None
 
 
-def self_attention(q, k, resid, drop_p: float = 0.0, seed: int = 0):
-    out = _SelfAttention.apply(q, k, resid, drop_p, seed)
+def self_attention(q, k, resid, drop_p: float = 0.0, seed: int = 0, seed_offset=None):
+    """Dense self attention (see _SelfAttention); ``seed_offset`` as in cross_attention."""
+    _check_seed_offset(seed_offset)
+    out = _SelfAttention.apply(q, k, resid, drop_p, seed, seed_offset)
     if tc_active(q) and q.shape[-1] % 8 == 0:
         out._dost_attn_out = True
     return out

@@ -16,6 +16,12 @@
  *   - dtype: DOST_F32 (eDOS, reference default) or DOST_F64 (phonon: main_phDOS.py:15-16 sets float64).
  *   - index arrays are int32 (dost_cast_i64_i32 converts the int64 PyG tensors once per batch).
  *   - stateless and re-entrant; one host thread per GPU in data-parallel runs.
+ *   - attention dropout seeds: every entry point that takes `unsigned long long seed` has a sibling
+ *     dost_<name>_dseed whose argument list inserts `const unsigned long long* seed_offset` right after
+ *     `seed`.  seed_offset is NULL or a device pointer to one word; the kernels then mask with
+ *     seed + *seed_offset, reading the word when they run, not when they are enqueued.  A captured CUDA
+ *     graph replays its launch arguments unchanged, so a host that rewrites the word on the stream before
+ *     each replay draws a new dropout mask per replay.  NULL (and the plain entry point) is seed alone.
  */
 #ifndef DOST_H_
 #define DOST_H_
@@ -285,6 +291,16 @@ int dost_xattn_bwd(int dtype, const void* d_out, const void* q, long long q_sstr
                    const void* out, const void* resid, long long resid_sstride, const float* lse, void* dq,
                    void* dkv, void* dphantom, int S, int B, int T, int H, long long N, double scale, double drop_p,
                    unsigned long long seed, void* workspace, size_t workspace_bytes, dost_stream_t stream);
+int dost_xattn_fwd_dseed(int dtype, const void* q, long long q_sstride, const void* kv, const void* phantom,
+                         const int32_t* ptr, const int32_t* nmax, const void* resid, long long resid_sstride, void* out,
+                         float* lse, int S, int B, int T, int H, double scale, double drop_p, unsigned long long seed,
+                         const unsigned long long* seed_offset, dost_stream_t stream);
+int dost_xattn_bwd_dseed(int dtype, const void* d_out, const void* q, long long q_sstride, const void* kv,
+                         const void* phantom, const int32_t* ptr, const int32_t* node_crystal, const int32_t* nmax,
+                         const void* out, const void* resid, long long resid_sstride, const float* lse, void* dq,
+                         void* dkv, void* dphantom, int S, int B, int T, int H, long long N, double scale, double drop_p,
+                         unsigned long long seed, const unsigned long long* seed_offset, void* workspace,
+                         size_t workspace_bytes, dost_stream_t stream);
 
 /* Tensor-core formulation of the same attention (fp32, no dropout, one sequence per crystal): the contractions are ragged
  * batched dost_gemm_bf16 problems over an extended key plane [N + B, H] that holds one phantom-key row per crystal after its
@@ -308,6 +324,13 @@ int dost_xattn_softmax_fwd(const float* scores, const int32_t* ptr, const int32_
 int dost_xattn_softmax_bwd(const float* scores, const float* lse, const float* dP, const int32_t* ptr, const int32_t* nmax,
                            long long rows, int B, int T, int npad, double scale, void* hi, void* lo, long long ldp,
                            double drop_p, unsigned long long seed, dost_stream_t stream);
+int dost_xattn_softmax_fwd_dseed(const float* scores, const int32_t* ptr, const int32_t* nmax, long long rows, int B, int T,
+                                 int npad, double scale, void* hi, void* lo, long long ldp, float* lse, double drop_p,
+                                 unsigned long long seed, const unsigned long long* seed_offset, dost_stream_t stream);
+int dost_xattn_softmax_bwd_dseed(const float* scores, const float* lse, const float* dP, const int32_t* ptr, const int32_t* nmax,
+                                 long long rows, int B, int T, int npad, double scale, void* hi, void* lo, long long ldp,
+                                 double drop_p, unsigned long long seed, const unsigned long long* seed_offset,
+                                 dost_stream_t stream);
 
 /* Row softmax for the dense T x T self attention (layers/multihead_attention.py:68-70): p = softmax_fp32(s*scale);
  * pd = dropout(p); rows are ld elements apart (ld >= cols).  Backward: ds = scale * p * (dp - sum(dp*p)) with dp = mask/(1-p) * dpd. */
@@ -315,6 +338,11 @@ int dost_softmax_fwd(int dtype, const void* s, void* p, void* pd, long long rows
                      double drop_p, unsigned long long seed, dost_stream_t stream);
 int dost_softmax_bwd(int dtype, const void* p, const void* dpd, void* ds, long long rows, int cols, long long ld, double scale,
                      double drop_p, unsigned long long seed, dost_stream_t stream);
+int dost_softmax_fwd_dseed(int dtype, const void* s, void* p, void* pd, long long rows, int cols, long long ld, double scale,
+                           double drop_p, unsigned long long seed, const unsigned long long* seed_offset, dost_stream_t stream);
+int dost_softmax_bwd_dseed(int dtype, const void* p, const void* dpd, void* ds, long long rows, int cols, long long ld,
+                           double scale, double drop_p, unsigned long long seed, const unsigned long long* seed_offset,
+                           dost_stream_t stream);
 
 /* Same, with the (dropped-out) probabilities / the score gradients also written as bf16 hi/lo operand planes (ds may be
  * NULL when only the planes are wanted). */
@@ -322,6 +350,12 @@ int dost_softmax_fwd_planes(const float* s, float* p, float* pd, long long rows,
                             double drop_p, unsigned long long seed, void* hi, void* lo, long long ldp, dost_stream_t stream);
 int dost_softmax_bwd_planes(const float* p, const float* dpd, float* ds, long long rows, int cols, long long ld, double scale,
                             double drop_p, unsigned long long seed, void* hi, void* lo, long long ldp, dost_stream_t stream);
+int dost_softmax_fwd_planes_dseed(const float* s, float* p, float* pd, long long rows, int cols, long long ld, double scale,
+                                  double drop_p, unsigned long long seed, const unsigned long long* seed_offset, void* hi,
+                                  void* lo, long long ldp, dost_stream_t stream);
+int dost_softmax_bwd_planes_dseed(const float* p, const float* dpd, float* ds, long long rows, int cols, long long ld,
+                                  double scale, double drop_p, unsigned long long seed, const unsigned long long* seed_offset,
+                                  void* hi, void* lo, long long ldp, dost_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Fused single-head attention forward on the tensor cores (layers/multihead_attention.py:68-72 with
@@ -349,6 +383,12 @@ int dost_attn_fused_fwd(const void* q_hi, const void* q_lo, long long ld_q, cons
                         const int32_t* nmax, int max_keys, double scale, const float* residual, long long res_seq_stride,
                         float* out, void* p_hi, void* p_lo, long long ld_p, int precision, double drop_p,
                         unsigned long long seed, float* lse, dost_stream_t stream);
+int dost_attn_fused_fwd_dseed(const void* q_hi, const void* q_lo, long long ld_q, const void* k_hi, const void* k_lo,
+                              long long ld_k, long long k_rows, int S, int Lq, int Lk, int H, const int32_t* k_rowoff,
+                              const int32_t* k_count, const int32_t* nmax, int max_keys, double scale, const float* residual,
+                              long long res_seq_stride, float* out, void* p_hi, void* p_lo, long long ld_p, int precision,
+                              double drop_p, unsigned long long seed, const unsigned long long* seed_offset, float* lse,
+                              dost_stream_t stream);
 int dost_softmax_bwd_from_planes(const void* p_hi, const void* p_lo, long long ld_pp, const float* dP, long long ld_dp,
                                  long long rows, int cols, double scale, void* hi, void* lo, long long ldp, dost_stream_t stream);
 

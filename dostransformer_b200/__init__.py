@@ -6,6 +6,7 @@ Public surface (mirrors the reference's model API, SURVEY.md section 8b):
     from dostransformer_b200.embedder_phDOS.DOSTransformer_phonon import DOSTransformer_phonon
     from dostransformer_b200.layers import TransformerEncoder
     from dostransformer_b200.ops import dos_loss
+    from dostransformer_b200 import attention_maps      # records every encoder layer's attention probabilities
 
 ``install_dropin()`` registers these under the reference's import paths (``embedder_eDOS.DOSTransformer``,
 ``embedder_phDOS.DOSTransformer_phonon``, ``layers``) so main_eDOS.py / main_phDOS.py pick them up unchanged.
@@ -14,6 +15,8 @@ The compute path is libdost_b200.so (hand-written CUDA, C ABI in include/dost.h)
 from __future__ import annotations
 
 import sys
+
+from .nn_core import attention_maps
 
 __version__ = "0.1.0"
 

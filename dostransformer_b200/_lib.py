@@ -163,6 +163,12 @@ _SIGNATURES = {
                                       C.c_double, C.c_ulonglong, C.c_void_p, C.c_void_p]),
     "dost_softmax_bwd_from_planes": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p, C.c_longlong, C.c_longlong, C.c_int,
                                                C.c_double, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p]),
+    "dost_xattn_probs": (C.c_int, [C.c_int, C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                   C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_double, C.c_ulonglong,
+                                   C.c_void_p, C.c_void_p]),
+    "dost_attn_maps_from_planes": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_longlong, C.c_int, C.c_int, C.c_int,
+                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_ulonglong, C.c_void_p,
+                                             C.c_void_p]),
     "dost_eval_metrics": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "dost_adamw_step": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_double,
                                   C.c_double, C.c_double, C.c_double, C.c_longlong, C.c_void_p]),

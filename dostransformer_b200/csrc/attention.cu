@@ -154,6 +154,93 @@ __global__ void __launch_bounds__(kAttWarps * 32) xattn_fwd_kernel(
   }
 }
 
+// ------------------------------------------------------------------------------------------------ attention maps
+// The probabilities of a forward recomputed from its log-sum-exp, in the reference's padded layout (attn_weights of
+// multihead_attention.py:68-71 after to_dense_batch): map[s, t, j] = exp(q_t . k_j scale - lse[s, t]) for the n_b atoms,
+// the same value for each of the phantom key slots n_b .. nmax - 1, 0 past nmax; with dropout mask / (1 - p) times that,
+// the mask regenerated per slot (index (s T + t) nmax + j, as in the forward).  Scoring loop of xattn_fwd_kernel.
+template <typename T, int HV>
+__global__ void __launch_bounds__(kAttWarps * 32) xattn_probs_kernel(
+    const T* __restrict__ q, long long q_ss, const T* __restrict__ kv, const T* __restrict__ phantom,
+    const int* __restrict__ ptr, const int* __restrict__ nmax_p, const float* __restrict__ lse, T* __restrict__ out, int cols,
+    int S, int B, int Tn, T scale, unsigned int thresh, float inv_keep, unsigned long long seed,
+    const unsigned long long* __restrict__ seed_offset) {
+  constexpr int H = 32 * HV;
+  seed = mask_seed(seed, seed_offset);
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  T* ks = reinterpret_cast<T*>(smem_raw);  // [kKT][H]
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int s = blockIdx.y;
+  const int b = s % B;
+  const int kbeg = ptr[b], kend = ptr[b + 1];
+  const int nb = kend - kbeg;
+  const int nmax = *nmax_p;
+  const int t0 = blockIdx.x * kQPB + warp * kQPW;
+
+  T qv[kQPW][HV];
+  float ls[kQPW];
+#pragma unroll
+  for (int qi = 0; qi < kQPW; ++qi) {
+    const int t = min(t0 + qi, Tn - 1);
+    load_row<T, HV>(q + (long long)s * q_ss + (long long)t * H, lane, qv[qi]);
+    ls[qi] = lse[(long long)s * Tn + t];
+  }
+
+  for (int j0 = 0; j0 < nb; j0 += kKT) {
+    const int kt = min(kKT, nb - j0);
+    __syncthreads();
+    for (int i = threadIdx.x; i < kt * H; i += blockDim.x) ks[i] = kv[(long long)(kbeg + j0) * H + i];
+    __syncthreads();
+    float mine[kQPW] = {0.f, 0.f, 0.f, 0.f};     // lane j keeps key j0 + j of the tile
+    for (int j = 0; j < kt; ++j) {
+      T kk[HV];
+#pragma unroll
+      for (int i = 0; i < HV; ++i) kk[i] = ks[j * H + lane + 32 * i];
+      T d[kQPW];
+#pragma unroll
+      for (int qi = 0; qi < kQPW; ++qi) d[qi] = dot_partial<T, HV>(qv[qi], kk);
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+        for (int qi = 0; qi < kQPW; ++qi) d[qi] += __shfl_xor_sync(0xffffffffu, d[qi], o);
+      }
+#pragma unroll
+      for (int qi = 0; qi < kQPW; ++qi) {
+        float p = expf(static_cast<float>(d[qi] * scale) - ls[qi]);
+        if (thresh) {
+          const unsigned long long idx = ((unsigned long long)s * Tn + t0 + qi) * (unsigned long long)nmax + (j0 + j);
+          p = keep_mask(seed, idx, thresh) ? p * inv_keep : 0.f;
+        }
+        mine[qi] = (lane == j) ? p : mine[qi];
+      }
+    }
+#pragma unroll
+    for (int qi = 0; qi < kQPW; ++qi) {
+      const int t = t0 + qi;
+      if (t < Tn && lane < kt && j0 + lane < cols) out[((long long)s * Tn + t) * cols + j0 + lane] = static_cast<T>(mine[qi]);
+    }
+  }
+  // phantom slots (each the probability of ONE zero-padded key), then zeros
+  T pk[HV];
+  if (nmax > nb) load_row<T, HV>(phantom, lane, pk);
+#pragma unroll
+  for (int qi = 0; qi < kQPW; ++qi) {
+    float pph = 0.f;
+    if (nmax > nb) pph = expf(static_cast<float>(warp_sum(dot_partial<T, HV>(qv[qi], pk)) * scale) - ls[qi]);
+    const int t = t0 + qi;
+    if (t >= Tn) continue;
+    T* orow = out + ((long long)s * Tn + t) * cols;
+    for (int c = nb + lane; c < cols; c += 32) {
+      float v = 0.f;
+      if (c < nmax) {
+        v = pph;
+        if (thresh) v = keep_mask(seed, ((unsigned long long)s * Tn + t) * (unsigned long long)nmax + c, thresh) ? v * inv_keep : 0.f;
+      }
+      orow[c] = static_cast<T>(v);
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------------------------ backward: dq
 // Also writes D[s,t] = dO . (out - resid) and per-block partial sums of the phantom-key gradient.
 template <typename T, int HV>
@@ -510,6 +597,32 @@ static int run_xattn_fwd(const void* q, long long q_ss, const void* kv, const vo
   return check_launch("xattn_fwd");
 }
 
+template <typename T>
+static int run_xattn_probs(const void* q, long long q_ss, const void* kv, const void* phantom, const int* ptr, const int* nmax,
+                           const float* lse, void* out, int cols, int S, int B, int Tn, int H, double scale, double drop_p,
+                           unsigned long long seed, const unsigned long long* seed_offset, cudaStream_t st) {
+  const unsigned int thresh = drop_p > 0 ? drop_threshold(drop_p) : 0u;
+  const float inv_keep = drop_p > 0 ? (float)(1.0 / (1.0 - drop_p)) : 1.f;
+  dim3 grid(ceil_div(Tn, kQPB), S);
+  const size_t smem = sizeof(T) * (size_t)kKT * H;
+#define DOST_XP(HV)                                                                                                    \
+  case HV:                                                                                                             \
+    if (smem > 48 * 1024)                                                                                              \
+      cudaFuncSetAttribute(xattn_probs_kernel<T, HV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);         \
+    xattn_probs_kernel<T, HV><<<grid, kAttWarps * 32, smem, st>>>((const T*)q, q_ss, (const T*)kv, (const T*)phantom, ptr, \
+                                                                  nmax, lse, (T*)out, cols, S, B, Tn, (T)scale, thresh, \
+                                                                  inv_keep, seed, seed_offset);                        \
+    break;
+  switch (H / 32) {
+    DOST_XP(1) DOST_XP(2) DOST_XP(4) DOST_XP(8) DOST_XP(16)
+    default:
+      set_error("xattn_probs: hidden %d unsupported (32,64,128,256,512)", H);
+      return DOST_ERR_UNSUPPORTED;
+  }
+#undef DOST_XP
+  return check_launch("xattn_probs");
+}
+
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 template <typename T>
@@ -630,6 +743,25 @@ extern "C" int dost_xattn_fwd(int dtype, const void* q, long long q_sstride, con
                               unsigned long long seed, dost_stream_t stream) {
   return dost_xattn_fwd_dseed(dtype, q, q_sstride, kv, phantom, ptr, nmax, resid, resid_sstride, out, lse, S, B, T, H, scale, drop_p,
                               seed, nullptr, stream);
+}
+
+extern "C" int dost_xattn_probs(int dtype, const void* q, long long q_sstride, const void* kv, const void* phantom,
+                                const int32_t* ptr, const int32_t* nmax, const float* lse, void* out, int cols, int S, int B, int T,
+                                int H, double scale, double drop_p, unsigned long long mask_seed,
+                                const unsigned long long* seed_offset, dost_stream_t stream) {
+  DOST_REQUIRE(q && kv && phantom && ptr && nmax && lse && out, "xattn_probs: null pointer");
+  DOST_REQUIRE(S > 0 && B > 0 && S % B == 0 && T > 0 && H % 32 == 0 && cols > 0, "xattn_probs: bad shape S=%d B=%d T=%d H=%d cols=%d",
+               S, B, T, H, cols);
+  DOST_REQUIRE(drop_p >= 0.0 && drop_p < 1.0, "xattn_probs: dropout must be in [0,1)");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == DOST_F32)
+    return run_xattn_probs<float>(q, q_sstride, kv, phantom, ptr, nmax, lse, out, cols, S, B, T, H, scale, drop_p, mask_seed, seed_offset,
+                                  st);
+  if (dtype == DOST_F64)
+    return run_xattn_probs<double>(q, q_sstride, kv, phantom, ptr, nmax, lse, out, cols, S, B, T, H, scale, drop_p, mask_seed, seed_offset,
+                                   st);
+  set_error("xattn_probs: unsupported dtype %d", dtype);
+  return DOST_ERR_UNSUPPORTED;
 }
 
 extern "C" size_t dost_xattn_bwd_workspace_bytes(int dtype, int S, int T, int H) {

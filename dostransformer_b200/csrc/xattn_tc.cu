@@ -11,6 +11,7 @@
 //                  as operand planes (phantom column = total phantom probability), log-sum-exp saved
 //   softmax_bwd  : dS = p (dP - sum p dP) scale, phantom column = the sum over its copies, written as planes
 //   kv_ext_split : gradient of the extended key plane -> gradient of the atoms and of the phantom key
+//   maps_from_planes : probability planes -> fp32 attention maps in the reference's padded layout (attention_maps recording)
 #include <math.h>
 #include <cuda_bf16.h>
 #include "common.cuh"
@@ -225,10 +226,96 @@ __global__ void __launch_bounds__(256) softmax_bwd_kernel(const float* __restric
   }
 }
 
+// Attention maps (the reference's attn_weights, multihead_attention.py:68-71) from the probability planes a forward wrote:
+// map[r, c] = hi + lo (hi alone without lo), i.e. exactly the P that the P K product consumed.  One warp per row, lane l owns
+// columns 8 l .. 8 l + 7 of every 256-column pass (16-byte plane loads).
+//   dense  (ptr == NULL): plane column c -> map column c < cols
+//   ragged (ptr != NULL): row r belongs to crystal b = (r / Tn) % B; its n_b atom columns are copied, the phantom column n_b
+//                         (total probability of the nmax - n_b zero-padded keys) is expanded into the key slots
+//                         n_b .. nmax - 1 of the map - total / (nmax - n_b) each, or with dropout total / kept for the
+//                         slots whose mask bit (index r * nmax + slot, as in the forward) survived and 0 for the others;
+//                         columns past nmax are 0.
+__global__ void __launch_bounds__(256) maps_from_planes_kernel(const __nv_bfloat16* __restrict__ hi, const __nv_bfloat16* __restrict__ lo,
+                                                               long long ldp, long long rows, int cols, int Tn, int B,
+                                                               const int* __restrict__ ptr, const int* __restrict__ nmax_p,
+                                                               float* __restrict__ out, unsigned int thresh, unsigned long long seed,
+                                                               const unsigned long long* __restrict__ seed_offset) {
+  const int lane = threadIdx.x & 31;
+  seed = mask_seed(seed, seed_offset);
+  const int nmax = ptr ? *nmax_p : 0;
+  const bool vec = (cols & 3) == 0;
+  for (long long r = blockIdx.x * 8LL + (threadIdx.x >> 5); r < rows; r += (long long)gridDim.x * 8) {
+    int nb = cols, nph = 0;
+    float slot = 0.f;                              // value of one surviving phantom slot
+    if (ptr) {
+      const int b = (int)((r / Tn) % B);
+      nb = min(__ldg(ptr + b + 1) - __ldg(ptr + b), (int)ldp - 1);
+      nph = max(nmax - nb, 0);
+      if (nph > 0) {
+        float total = __bfloat162float(hi[r * ldp + nb]);
+        if (lo) total += __bfloat162float(lo[r * ldp + nb]);
+        const int kept = thresh ? phantom_kept(seed, r, nb, nmax, thresh, lane) : nph;
+        slot = kept > 0 ? total / (float)kept : 0.f;
+      }
+    }
+    const int pend = min(nb + nph, cols);          // last map column that carries probability (exclusive)
+    float* orow = out + r * cols;
+    for (int c0 = lane * 8; c0 < cols; c0 += 256) {
+      float v[8];
+      if (c0 < nb && c0 < ldp) {
+        const uint4 h = __ldg(reinterpret_cast<const uint4*>(hi + r * ldp + c0));
+        uint4 l = make_uint4(0u, 0u, 0u, 0u);
+        if (lo) l = __ldg(reinterpret_cast<const uint4*>(lo + r * ldp + c0));
+        const uint32_t hw[4] = {h.x, h.y, h.z, h.w}, lw[4] = {l.x, l.y, l.z, l.w};
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+          v[2 * k] = __uint_as_float(hw[k] << 16) + __uint_as_float(lw[k] << 16);
+          v[2 * k + 1] = __uint_as_float(hw[k] & 0xFFFF0000u) + __uint_as_float(lw[k] & 0xFFFF0000u);
+        }
+      }
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const int c = c0 + j;
+        if (c >= nb) {
+          float s = 0.f;
+          if (c < pend) s = (!thresh || keep_mask(seed, (unsigned long long)r * (unsigned long long)nmax + c, thresh)) ? slot : 0.f;
+          v[j] = s;
+        }
+      }
+      if (vec && c0 + 8 <= cols) {
+        *reinterpret_cast<float4*>(orow + c0) = make_float4(v[0], v[1], v[2], v[3]);
+        *reinterpret_cast<float4*>(orow + c0 + 4) = make_float4(v[4], v[5], v[6], v[7]);
+      } else {
+#pragma unroll
+        for (int j = 0; j < 8; ++j)
+          if (c0 + j < cols) orow[c0 + j] = v[j];
+      }
+    }
+  }
+}
+
 }  // namespace xtc
 }  // namespace dost
 
 using namespace dost;
+
+extern "C" int dost_attn_maps_from_planes(const void* p_hi, const void* p_lo, long long ld_p, long long rows, int cols, int T, int B,
+                                          const int32_t* ptr, const int32_t* nmax, float* out, double drop_p,
+                                          unsigned long long mask_seed, const unsigned long long* seed_offset,
+                                          dost_stream_t stream) {
+  DOST_REQUIRE(p_hi && out && rows > 0 && cols > 0 && ld_p > 0 && ld_p % 8 == 0 && ((uintptr_t)p_hi & 15) == 0 &&
+                   ((uintptr_t)p_lo & 15) == 0 && ((uintptr_t)out & 15) == 0,
+               "attn_maps_from_planes: bad args (ld_p %% 8 == 0, 16-byte aligned planes and map)");
+  DOST_REQUIRE(ptr ? (nmax && T > 0 && B > 0) : cols <= ld_p, "attn_maps_from_planes: ragged maps need ptr, nmax, T and B; dense "
+               "maps at most ld_p columns");
+  DOST_REQUIRE(drop_p >= 0.0 && drop_p < 1.0, "attn_maps_from_planes: drop_p must be in [0, 1)");
+  const unsigned int thresh = drop_p > 0.0 ? drop_threshold(drop_p) : 0u;
+  const int blocks = (int)min64((rows + 7) / 8, 32LL * kNumSMs);
+  xtc::maps_from_planes_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>((const __nv_bfloat16*)p_hi, (const __nv_bfloat16*)p_lo, ld_p,
+                                                                         rows, cols, T, B, ptr, nmax, out, thresh, mask_seed,
+                                                                         seed_offset);
+  return check_launch("attn_maps_from_planes");
+}
 
 extern "C" int dost_xattn_kv_ext_build(const float* y, const float* beta, const int32_t* batch, const int32_t* ptr, long long N, int B,
                                        int H, void* hi, void* lo, long long ldp, dost_stream_t stream) {

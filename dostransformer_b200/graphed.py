@@ -35,7 +35,7 @@ import torch
 
 from . import _lib as L
 from . import ops
-from .nn_core import device_seed, draw_dropout_base
+from .nn_core import active_recorder, device_seed, draw_dropout_base
 from .synthetic import CrystalBatch
 
 
@@ -177,6 +177,9 @@ class GraphedStep:
         return e
 
     def __call__(self, g):
+        if active_recorder() is not None:
+            raise RuntimeError("GraphedStep cannot run inside attention_maps(): a replayed graph has no attention maps to "
+                               "record; run the model eagerly to record them")
         # (the model's data-parallel padding length and its dropout probability are host values baked into the captured
         # launches, and training decides whether dropout runs at all: part of the key)
         attn_drop = float(getattr(self.model, "attn_drop", 0.0))

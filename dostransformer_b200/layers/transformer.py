@@ -33,11 +33,15 @@ class TransformerEncoder(K.EnergyEncoderParams):
         x = _to_batch_first(x_in)
         kv0 = x if x_in_k is x_in else _to_batch_first(x_in_k)
         S, Lq, H = x.shape
-        for layer in self.layers:
+        rec = K.active_recorder()
+        for li, layer in enumerate(self.layers):
             ln0 = layer.layer_norms[0]
             k = ops.layer_norm(kv0, ln0.weight, ln0.bias)
             q = ops.layer_norm(x, ln0.weight, ln0.bias)
-            y = ops.self_attention(q, k, x, seeds.p, *seeds.next())
+            key, maps = rec._buffer(self, li, S, Lq, k.shape[1], q) if rec is not None else (None, None)
+            y = ops.self_attention(q, k, x, seeds.p, *seeds.next(), maps_out=maps)
+            if rec is not None:
+                rec._add(key, maps, S)
             x = K._ffn(layer, y)
         x = ops.layer_norm(x, self.layer_norm.weight, self.layer_norm.bias)
         return x.transpose(0, 1)

@@ -11,7 +11,7 @@ from __future__ import annotations
 import os
 import threading
 from contextlib import contextmanager
-from typing import Optional, Tuple
+from typing import Dict, List, Optional, Tuple
 
 import torch
 from torch import nn
@@ -162,6 +162,68 @@ def device_seed(word: torch.Tensor):
         _device_seed.word = prev
 
 
+class AttentionMaps:
+    """What ``attention_maps(model)`` records (per thread).
+
+    ``maps[key]``: the attention probabilities of the layer whose reference ``MultiheadAttention`` module path is ``key``
+    (``<stack>.layers.<i>.self_attn``), one tensor per call in the order a forward hook on that module would see them: the
+    reference's ``attn_weights`` (multihead_attention.py:68-71) batch-first - [B, T, T] for the energy self-attention,
+    [B, T, Nmax] for the energy -> atom cross-attention with atom j of the crystal in column j and the probability of ONE
+    zero-padded key in each of the columns n_b .. Nmax - 1 (none with ``per_crystal_eval`` in eval mode: those columns are
+    0).  With attention dropout the dropped-out probabilities mask / (1 - p) * P.  fp32, or the model's dtype for fp64.
+    ``n_atoms``: atoms per crystal [B] of the last recorded forward of a DOS model."""
+
+    def __init__(self, model: nn.Module):
+        self.maps: Dict[str, List[torch.Tensor]] = {}
+        self.n_atoms: Optional[torch.Tensor] = None
+        self._names = {id(m): n for n, m in model.named_modules() if isinstance(m, EnergyEncoderParams)}
+        self._width = None
+
+    def _begin(self, graph: ops.CrystalGraph, per_crystal: bool) -> None:
+        """Per forward of a DOS model: the padding length of its cross-attention maps (read back only when the host does not
+        know it)."""
+        self.n_atoms = (graph.ptr[1:] - graph.ptr[:-1]).long()
+        if graph.nmax_host is not None:
+            self._width = graph.nmax_host
+        else:
+            self._width = int(self.n_atoms.max()) if per_crystal else int(graph.nmax.item())
+
+    def _buffer(self, enc: nn.Module, layer: int, S: int, T: int, width: int, like: torch.Tensor):
+        """(key, [S, T, width] output buffer) for one attention call of ``enc``, or (None, None) when it is not recorded."""
+        name = self._names.get(id(enc))
+        if name is None:
+            return None, None
+        key = f"{name}.layers.{layer}.self_attn" if name else f"layers.{layer}.self_attn"
+        return key, torch.empty(S, T, width, dtype=like.dtype, device=like.device)
+
+    def _add(self, key: Optional[str], buf: Optional[torch.Tensor], B: int) -> None:
+        """S = reps * B sequences (the global and the system branch batched): one B-row tensor per branch, in branch order."""
+        if key is not None:
+            self.maps.setdefault(key, []).extend(buf.split(B))
+
+
+_recording = threading.local()
+
+
+@contextmanager
+def attention_maps(model: nn.Module):
+    """``with attention_maps(model) as rec: model(batch)`` records every encoder layer's attention probabilities of the
+    forwards run inside the block on this thread into ``rec.maps`` (see AttentionMaps).  The forward's results, its
+    gradients and the random-number stream are unchanged; recording costs the map buffers and one extra kernel per
+    attention call.  CUDA-graph replays (graphed.GraphedStep) refuse to run inside the block."""
+    rec = AttentionMaps(model)
+    prev = getattr(_recording, "rec", None)
+    _recording.rec = rec
+    try:
+        yield rec
+    finally:
+        _recording.rec = prev
+
+
+def active_recorder() -> Optional[AttentionMaps]:
+    return getattr(_recording, "rec", None)
+
+
 class _Seeds:
     def __init__(self, drop_p: float, training: bool):
         self.p = drop_p if training else 0.0
@@ -177,20 +239,25 @@ class _Seeds:
 
 def cross_stack(enc: EnergyEncoderParams, q, x_nodes, graph: ops.CrystalGraph, S: int, T: int, seeds: _Seeds):
     """Energy tokens attend to the atoms of their crystal (keys = values = LN0(x), fixed across layers)."""
-    H = x_nodes.shape[1]
-    for layer in enc.layers:
+    rec = active_recorder()
+    for li, layer in enumerate(enc.layers):
         ln0 = layer.layer_norms[0]
         kv = ops.layer_norm(x_nodes, ln0.weight, ln0.bias)
         q_ln, q_res = ops.layer_norm(q, ln0.weight, ln0.bias, want_planes=q.dim() == 3, with_residual=True)
-        y = ops.cross_attention(q_ln, kv, ln0.bias, q_res, graph, S, seeds.p, *seeds.next())
+        key, maps = rec._buffer(enc, li, S, T, rec._width, kv) if rec is not None else (None, None)
+        y = ops.cross_attention(q_ln, kv, ln0.bias, q_res, graph, S, seeds.p, *seeds.next(), maps_out=maps)
+        if rec is not None:
+            rec._add(key, maps, graph.B)
         q = _ffn(layer, y)
     return ops.layer_norm(q, enc.layer_norm.weight, enc.layer_norm.bias)
 
 
-def self_stack(enc: EnergyEncoderParams, x0, seeds: _Seeds):
-    """Self attention over the T energy tokens; keys are LN0_l of the ORIGINAL input in every layer."""
+def self_stack(enc: EnergyEncoderParams, x0, seeds: _Seeds, B: int):
+    """Self attention over the T energy tokens; keys are LN0_l of the ORIGINAL input in every layer.  B: crystals of the
+    batch (sequence s belongs to crystal s % B)."""
     S, T, H = x0.shape
     x = x0
+    rec = active_recorder()
     for li, layer in enumerate(enc.layers):
         ln0 = layer.layer_norms[0]
         if li == 0:
@@ -199,7 +266,10 @@ def self_stack(enc: EnergyEncoderParams, x0, seeds: _Seeds):
         else:
             k = ops.layer_norm(x0, ln0.weight, ln0.bias, want_planes=True)
             q, x_res = ops.layer_norm(x, ln0.weight, ln0.bias, want_planes=True, with_residual=True)
-        y = ops.self_attention(q, k, x_res, seeds.p, *seeds.next())
+        key, maps = rec._buffer(enc, li, S, T, T, q) if rec is not None else (None, None)
+        y = ops.self_attention(q, k, x_res, seeds.p, *seeds.next(), maps_out=maps)
+        if rec is not None:
+            rec._add(key, maps, B)
         x = _ffn(layer, y)
     return ops.layer_norm(x, enc.layer_norm.weight, enc.layer_norm.bias)
 
@@ -208,6 +278,9 @@ def dos_heads(model, x_nodes, graph: ops.CrystalGraph, graph_vec, prompt_table, 
     """DOSTransformer.py:61-91: cross-attention -> (fc | fc_prompt) -> self-attention -> cross-attention -> out_layer,
     for the global and the system branch (shared transformer_self / transformer_source / out_layer)."""
     B, H = graph.B, x_nodes.shape[1]
+    rec = active_recorder()
+    if rec is not None:
+        rec._begin(graph, model.per_crystal_eval and not model.training)
     energies = cross_stack(model.transformer, model.embeddings.weight, x_nodes, graph, B, T, seeds)   # [B,T,H]
     e2d = energies.view(B * T, H)
     per_crystal = RowMap(div=T, div_rowptr=graph.token_rowptr(T))
@@ -215,7 +288,7 @@ def dos_heads(model, x_nodes, graph: ops.CrystalGraph, graph_vec, prompt_table, 
 
     def branches(both, S):
         """transformer_self -> transformer_source -> out_layer on S sequences (sequence s belongs to crystal s % B)."""
-        h = self_stack(model.transformer_self, both.view(S, T, H), seeds)
+        h = self_stack(model.transformer_self, both.view(S, T, H), seeds, B)
         h = cross_stack(model.transformer_source, h, x_nodes, graph, S, T, seeds)
         return ops.linear([(h.view(S * T, H), None)], model.out_layer.weight, model.out_layer.bias).view(S, T)
 

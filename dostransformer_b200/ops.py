@@ -1367,7 +1367,7 @@ class _CrossAttention(torch.autograd.Function):
     seed_offset: optional 1-element int64 device tensor added to ``seed`` by the kernels (dost.h, ``_dseed`` entry points)."""
 
     @staticmethod
-    def forward(ctx, q, kv, phantom, resid, graph: CrystalGraph, S: int, drop_p: float, seed: int, seed_offset=None):
+    def forward(ctx, q, kv, phantom, resid, graph: CrystalGraph, S: int, drop_p: float, seed: int, seed_offset=None, maps_out=None):
         H = kv.shape[1]
         T = q.shape[-2]
         q, resid = q.contiguous(), resid.contiguous()
@@ -1379,6 +1379,10 @@ class _CrossAttention(torch.autograd.Function):
         L.check(L.lib().dost_xattn_fwd_dseed(L.dt(kv), L.p(q), q_ss, L.p(kv), L.p(phantom), L.p(graph.ptr), L.p(graph.nmax),
                                              L.p(resid), r_ss, L.p(out), L.p(lse), S, graph.B, T, H, scale, drop_p, seed,
                                              L.p(seed_offset), L.stream()), "xattn_fwd")
+        if maps_out is not None:      # the probabilities once more, from the log-sum-exp
+            L.check(L.lib().dost_xattn_probs(L.dt(kv), L.p(q), q_ss, L.p(kv), L.p(phantom), L.p(graph.ptr), L.p(graph.nmax), L.p(lse),
+                                             L.p(maps_out), maps_out.shape[-1], S, graph.B, T, H, scale, drop_p, seed,
+                                             L.p(seed_offset), L.stream()), "xattn_probs")
         ctx.save_for_backward(q, kv, phantom, resid, out, lse)
         ctx.graph, ctx.S, ctx.drop_p, ctx.seed, ctx.seed_offset = graph, S, drop_p, seed, seed_offset
         ctx.q_ss, ctx.r_ss = q_ss, r_ss
@@ -1404,7 +1408,7 @@ class _CrossAttention(torch.autograd.Function):
                                          L.p(ctx.seed_offset), L.p(ws), nb, L.stream()), "xattn_bwd")
         d_q = dq if ctx.q_ss else colsum(dq.view(S, T * H)).view(T, H)
         d_resid = d_out if ctx.r_ss else colsum(d_out.view(S, T * H)).view(T, H)
-        return d_q, dkv, dph, d_resid, None, None, None, None, None
+        return d_q, dkv, dph, d_resid, None, None, None, None, None, None
 
 
 def _grad_planes(d_out: torch.Tensor, rows: int, cols: int) -> Planes:
@@ -1449,7 +1453,7 @@ class _CrossAttentionTC(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, q, kv, phantom, resid, graph: CrystalGraph, qpl: Optional[Planes], S: int, drop_p: float = 0.0, seed: int = 0,
-                seed_offset=None):
+                seed_offset=None, maps_out=None):
         N, H = kv.shape
         B = graph.B
         T = q.shape[-2]
@@ -1477,11 +1481,13 @@ class _CrossAttentionTC(torch.autograd.Function):
         if ctx.fused:
             # one kernel: scores stay in TMEM, the probabilities leave only as the operand planes the backward needs
             need = any(ctx.needs_input_grad[:4])
-            pp = empty_planes(S * T, npad, dev, _with_lo()) if need else None
+            pp = empty_planes(S * T, npad, dev, _with_lo()) if (need or maps_out is not None) else None
             # with dropout the planes hold the dropped-out probabilities; the backward recomputes P from the log-sum-exp
             lse = torch.empty(S * T, dtype=torch.float32, device=dev) if (need and drop_p > 0) else None
             _fused_attention_fwd(qp, kvp, N + B, S, T, 0, H, ptr_ext, n_ext, graph.nmax, graph.nkeys_host, r2,
                                  0 if resid.dim() == 2 else T * H, out.view(S * T, H), pp, drop_p, seed, lse, seed_offset)
+            if maps_out is not None:
+                _maps_from_planes(pp, maps_out, S * T, graph, T, drop_p, seed, seed_offset)
             if need:
                 ctx.save_for_backward(kv, phantom, None, lse, *_planes_save(qp), *_planes_save(kvp), *_planes_save(pp))
             return out
@@ -1494,6 +1500,8 @@ class _CrossAttentionTC(torch.autograd.Function):
         L.check(lib.dost_xattn_softmax_fwd_dseed(L.p(scores), L.p(graph.ptr), L.p(graph.nmax), S * T, B, T, npad, scale, L.p(pp.hi),
                                                  L.p(pp.lo), pp.ld, L.p(lse), drop_p, seed, L.p(seed_offset), L.stream()),
                 "xattn_softmax_fwd")
+        if maps_out is not None:
+            _maps_from_planes(pp, maps_out, S * T, graph, T, drop_p, seed, seed_offset)
         gemm_planes(M=T, N=H, K=npad, a=[pp], a_mode=L.KC, b=kvp, b_mode=L.MC, b_rows=N + B, out=out.view(S * T, H), residual=r2,
                     batch=S, a_bstride=T * pp.ld, c_bstride=T * H, res_bstride=(0 if resid.dim() == 2 else T * H),
                     b_rowoff=ptr_ext)
@@ -1551,7 +1559,7 @@ class _CrossAttentionTC(torch.autograd.Function):
                 dph = colsum(dbrows)
                 d_q = colsum(dq.view(S, T * H)).view(T, H) if ctx.bcast_q else dq
                 d_resid = colsum(d_out.view(S, T * H)).view(T, H) if ctx.bcast_r else d_out
-                return d_q, dkv, dph, d_resid, None, None, None, None, None, None
+                return d_q, dkv, dph, d_resid, None, None, None, None, None, None, None
             dext = torch.empty(N + B, H, dtype=torch.float32, device=dev)
             p1, n1 = g.ragged(1)
             for rep in range(reps):
@@ -1565,7 +1573,18 @@ class _CrossAttentionTC(torch.autograd.Function):
             dph = colsum(dbrows)
             d_q = colsum(dq.view(S, T * H)).view(T, H) if ctx.bcast_q else dq
             d_resid = colsum(d_out.view(S, T * H)).view(T, H) if ctx.bcast_r else d_out
-        return d_q, dkv, dph, d_resid, None, None, None, None, None, None
+        return d_q, dkv, dph, d_resid, None, None, None, None, None, None, None
+
+
+def _maps_from_planes(pp: Planes, maps_out: torch.Tensor, rows: int, graph: Optional[CrystalGraph], T: int = 0, drop_p: float = 0.0,
+                      seed: int = 0, seed_offset=None) -> None:
+    """Attention maps from probability planes (dost_attn_maps_from_planes): ragged with the graph (phantom column expanded into
+    the padded key slots, the dropout mask of the forward regenerated there), dense without."""
+    B = graph.B if graph is not None else 0
+    L.check(L.lib().dost_attn_maps_from_planes(L.p(pp.hi), L.p(pp.lo), pp.ld, rows, maps_out.shape[-1], T, B,
+                                               L.p(graph.ptr) if graph is not None else None,
+                                               L.p(graph.nmax) if graph is not None else None, L.p(maps_out), float(drop_p), int(seed),
+                                               L.p(seed_offset), L.stream()), "attn_maps_from_planes")
 
 
 def _rows(pl: Planes, r0: int, r1: int) -> Planes:
@@ -1578,18 +1597,29 @@ def _check_seed_offset(seed_offset) -> None:
         raise ValueError("seed_offset must be a 1-element int64 CUDA tensor")
 
 
-def cross_attention(q, kv, phantom, resid, graph: CrystalGraph, S: int, drop_p: float = 0.0, seed: int = 0, seed_offset=None):
+def _check_maps_out(maps_out, lead, like: torch.Tensor) -> None:
+    if maps_out is not None and (maps_out.dim() != 3 or tuple(maps_out.shape[:2]) != tuple(lead) or maps_out.dtype != like.dtype
+                                 or maps_out.device != like.device or not maps_out.is_contiguous()):
+        raise ValueError(f"maps_out must be a contiguous [{lead[0]}, {lead[1]}, keys] {like.dtype} tensor on {like.device}")
+
+
+def cross_attention(q, kv, phantom, resid, graph: CrystalGraph, S: int, drop_p: float = 0.0, seed: int = 0, seed_offset=None,
+                    maps_out=None):
     """Energy -> atom cross attention (see _CrossAttention).  Dropout masks with ``seed``, plus the value of ``seed_offset``
-    (optional 1-element int64 CUDA tensor) read on the device when the kernels run: a captured step rewrites it per replay."""
+    (optional 1-element int64 CUDA tensor) read on the device when the kernels run: a captured step rewrites it per replay.
+    ``maps_out`` (optional, contiguous [S, T, Nmax] in kv's dtype, Nmax = the padding length on the device ``graph.nmax``)
+    receives the attention probabilities in the reference's padded layout: atom j of the crystal in column j, the
+    probability of one zero-padded key in each of the columns n_b .. Nmax - 1, with dropout the dropped-out values."""
     _check_seed_offset(seed_offset)
     H = kv.shape[1]
+    _check_maps_out(maps_out, (S, q.shape[-2]), kv)
     if (tc_active(kv) and H % 128 == 0 and S % graph.B == 0 and graph.nmax_host is not None
             and graph.nkeys_host <= 1016 and q.shape[-2] >= 64 and not L.switch("DOST_NO_XATTN_TC")
             and (q.dim() == 3 or S == graph.B)):
-        out = _CrossAttentionTC.apply(q, kv, phantom, resid, graph, _planes3(q), S, drop_p, seed, seed_offset)
+        out = _CrossAttentionTC.apply(q, kv, phantom, resid, graph, _planes3(q), S, drop_p, seed, seed_offset, maps_out)
         out._dost_attn_out = True        # (its backward takes the incoming gradient as operand planes, see _grad_planes)
         return out
-    return _CrossAttention.apply(q, kv, phantom, resid, graph, S, drop_p, seed, seed_offset)
+    return _CrossAttention.apply(q, kv, phantom, resid, graph, S, drop_p, seed, seed_offset, maps_out)
 
 
 # =====================================================================================================
@@ -1599,7 +1629,7 @@ class _SelfAttention(torch.autograd.Function):
     """out = resid + softmax_fp32(q k^T / sqrt(H)) k, per sequence; q, resid: [S,Lq,H], k (= v): [S,Lk,H]."""
 
     @staticmethod
-    def forward(ctx, q, k, resid, drop_p: float, seed: int, seed_offset=None):
+    def forward(ctx, q, k, resid, drop_p: float, seed: int, seed_offset=None, maps_out=None):
         S, Lq, H = q.shape
         Lk = k.shape[1]
         qpl, kpl = _planes3(q), _planes3(k)
@@ -1616,10 +1646,13 @@ class _SelfAttention(torch.autograd.Function):
             ctx.fused = fused_attention_ok(H, Lk, drop_p)
             if ctx.fused:
                 out = torch.empty(S, Lq, H, dtype=dtype, device=dev)
-                pdp = empty_planes(S * Lq, Lk, dev, _with_lo()) if any(ctx.needs_input_grad[:3]) else None
+                need = any(ctx.needs_input_grad[:3])
+                pdp = empty_planes(S * Lq, Lk, dev, _with_lo()) if (need or maps_out is not None) else None
                 _fused_attention_fwd(qp, kp, S * Lk, S, Lq, Lk, H, None, None, None, Lk, resid.view(S * Lq, H), Lq * H,
                                      out.view(S * Lq, H), pdp, drop_p, seed, seed_offset=seed_offset)
-                if pdp is not None:
+                if maps_out is not None:
+                    _maps_from_planes(pdp, maps_out, S * Lq, None)
+                if need:
                     ctx.save_for_backward(None, None, *_planes_save(qp), *_planes_save(kp), *_planes_save(pdp))
                 return out
             scores = torch.empty(S, Lq, Lp, dtype=dtype, device=dev)
@@ -1630,6 +1663,8 @@ class _SelfAttention(torch.autograd.Function):
             L.check(L.lib().dost_softmax_fwd_planes_dseed(L.p(scores), L.p(scores), L.p(pd), S * Lq, Lk, Lp, float(H) ** -0.5,
                                                           drop_p, seed, L.p(seed_offset), L.p(pdp.hi), L.p(pdp.lo), pdp.ld,
                                                           L.stream()), "softmax_fwd_planes")
+            if maps_out is not None:
+                _maps_from_planes(pdp, maps_out, S * Lq, None)
             out = torch.empty(S, Lq, H, dtype=dtype, device=dev)
             gemm_planes(M=Lq, N=H, K=Lk, a=[pdp], a_mode=L.KC, b=kp, b_mode=L.MC, out=out.view(S * Lq, H),
                         residual=resid.view(S * Lq, H), batch=S, a_bstride=Lq * pdp.ld, b_bstride=Lk * kp.ld, c_bstride=Lq * H,
@@ -1642,6 +1677,8 @@ class _SelfAttention(torch.autograd.Function):
         pd = torch.empty_like(scores) if drop_p > 0 else scores
         L.check(L.lib().dost_softmax_fwd_dseed(L.dt(q), L.p(scores), L.p(scores), L.p(pd), S * Lq, Lk, Lp, float(H) ** -0.5,
                                                drop_p, seed, L.p(seed_offset), L.stream()), "softmax_fwd")
+        if maps_out is not None:      # the softmax wrote P (and the dropped-out P) into row-padded score buffers
+            maps_out.copy_(pd[:, :, :Lk])
         out = torch.empty(S, Lq, H, dtype=dtype, device=dev)
         gemm_raw(M=Lq, N=H, K=Lk, a=[(pd.view(S * Lq, Lp), None)], a_mode=L.KC, b=k.view(S * Lk, H), b_mode=L.MC,
                  out=out, residual=resid, batch=S, a_bstride=Lq * Lp, b_bstride=Lk * H, c_bstride=Lq * H, ldc=H, lda=Lp)
@@ -1680,7 +1717,7 @@ class _SelfAttention(torch.autograd.Function):
         gemm_raw(M=Lk, N=H, K=Lq, a=[(pd.view(S * Lq, Lp), None)], a_mode=L.MC, b=d_out.view(S * Lq, H), b_mode=L.MC,
                  out=dk, accumulate=True, batch=S, a_bstride=Lq * Lp, b_bstride=Lq * H, c_bstride=Lk * H, ldc=H, lda=Lp,
                  prec=ctx.prec)
-        return dq, dk, d_out, None, None, None
+        return dq, dk, d_out, None, None, None, None
 
 
 def _self_attention_backward_planes(ctx, d_out):
@@ -1719,7 +1756,7 @@ def _self_attention_backward_planes(ctx, d_out):
                 a_bstride=Lq * dsp.ld, b_bstride=Lq * qp.ld, c_bstride=Lk * H)
     gemm_planes(M=Lk, N=H, K=Lq, a=[pdp], a_mode=L.MC, b=dop, b_mode=L.MC, out=dk.view(S * Lk, H), accumulate=True, batch=S,
                 a_bstride=Lq * pdp.ld, b_bstride=Lq * dop.ld, c_bstride=Lk * H)
-    return dq, dk, d_out, None, None, None
+    return dq, dk, d_out, None, None, None, None
 
 
 _SelfAttention._backward_planes = staticmethod(_self_attention_backward_planes)
@@ -1739,10 +1776,14 @@ def _planes3(t: torch.Tensor) -> Optional[Planes]:
     return None
 
 
-def self_attention(q, k, resid, drop_p: float = 0.0, seed: int = 0, seed_offset=None):
-    """Dense self attention (see _SelfAttention); ``seed_offset`` as in cross_attention."""
+def self_attention(q, k, resid, drop_p: float = 0.0, seed: int = 0, seed_offset=None, maps_out=None):
+    """Dense self attention (see _SelfAttention); ``seed_offset`` as in cross_attention.  ``maps_out`` (optional, contiguous
+    [S, Lq, Lk] in q's dtype) receives the attention probabilities that multiply k (with dropout the dropped-out ones)."""
     _check_seed_offset(seed_offset)
-    out = _SelfAttention.apply(q, k, resid, drop_p, seed, seed_offset)
+    _check_maps_out(maps_out, q.shape[:2], q)
+    if maps_out is not None and maps_out.shape[2] != k.shape[1]:
+        raise ValueError(f"maps_out must have {k.shape[1]} columns (one per key)")
+    out = _SelfAttention.apply(q, k, resid, drop_p, seed, seed_offset, maps_out)
     if tc_active(q) and q.shape[-1] % 8 == 0:
         out._dost_attn_out = True
     return out

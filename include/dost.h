@@ -301,6 +301,13 @@ int dost_xattn_bwd_dseed(int dtype, const void* d_out, const void* q, long long 
                          void* dkv, void* dphantom, int S, int B, int T, int H, long long N, double scale, double drop_p,
                          unsigned long long seed, const unsigned long long* seed_offset, void* workspace,
                          size_t workspace_bytes, dost_stream_t stream);
+/* Attention map of a dost_xattn_fwd call (the reference's attn_weights, multihead_attention.py:68-71, batch-first, keys
+ * zero-padded by to_dense_batch): out [S, T, cols] in dtype, recomputed from that call's lse.  Column j < n_b is atom j of the
+ * crystal, columns n_b .. *nmax - 1 each hold the probability of ONE phantom key, columns past *nmax are 0.  drop_p,
+ * mask_seed, seed_offset: those of the forward (mask / (1 - p) applied per key slot, the same bits). */
+int dost_xattn_probs(int dtype, const void* q, long long q_sstride, const void* kv, const void* phantom, const int32_t* ptr,
+                     const int32_t* nmax, const float* lse, void* out, int cols, int S, int B, int T, int H, double scale,
+                     double drop_p, unsigned long long mask_seed, const unsigned long long* seed_offset, dost_stream_t stream);
 
 /* Tensor-core formulation of the same attention (fp32, no dropout, one sequence per crystal): the contractions are ragged
  * batched dost_gemm_bf16 problems over an extended key plane [N + B, H] that holds one phantom-key row per crystal after its
@@ -391,6 +398,15 @@ int dost_attn_fused_fwd_dseed(const void* q_hi, const void* q_lo, long long ld_q
                               dost_stream_t stream);
 int dost_softmax_bwd_from_planes(const void* p_hi, const void* p_lo, long long ld_pp, const float* dP, long long ld_dp,
                                  long long rows, int cols, double scale, void* hi, void* lo, long long ldp, dost_stream_t stream);
+/* Attention maps from the probability planes [rows, ld_p] written by dost_attn_fused_fwd, dost_softmax_fwd_planes or
+ * dost_xattn_softmax_fwd: out [rows, cols] fp32 = hi + lo (hi alone when p_lo is NULL), the P the P k product consumed.
+ *   ptr == NULL: dense, plane column c -> column c < cols (cols <= ld_p)
+ *   ptr != NULL: ragged rows (row r attends to crystal (r / T) % B): the n_b atom columns, then the phantom column expanded
+ *                into the key slots n_b .. *nmax - 1 (total / (*nmax - n_b) each; with drop_p > 0 total / kept for the slots
+ *                whose mask bit, index r * *nmax + slot with mask_seed + *seed_offset, survived, 0 for the others), 0 past *nmax. */
+int dost_attn_maps_from_planes(const void* p_hi, const void* p_lo, long long ld_p, long long rows, int cols, int T, int B,
+                               const int32_t* ptr, const int32_t* nmax, float* out, double drop_p, unsigned long long mask_seed,
+                               const unsigned long long* seed_offset, dost_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * DOS loss.  mode 0 (eDOS, main_eDOS.py:111-123): y = max(y,0); per-crystal RMSE; mean over crystals;

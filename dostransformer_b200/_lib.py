@@ -129,6 +129,8 @@ _SIGNATURES = {
     "dost_phonon_edge_feat": (C.c_int, [C.c_int, C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p]),
     "dost_phonon_edge_encode": (C.c_int, [C.c_int, C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
                                           C.c_void_p, C.c_void_p]),
+    "dost_phonon_edge_encode_bwd": (C.c_int, [C.c_int, C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                              C.c_void_p]),
     "dost_xattn_fwd": (C.c_int, [C.c_int, C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                  C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                  C.c_double, C.c_double, C.c_ulonglong, C.c_void_p]),
@@ -191,6 +193,8 @@ _SIGNATURES = {
                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "dost_gaussian_expand": (C.c_int, [C.c_void_p, C.c_longlong, C.c_double, C.c_double, C.c_int, C.c_double, C.c_void_p,
                                        C.c_void_p]),
+    "dost_gaussian_expand_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_double, C.c_double, C.c_int, C.c_double,
+                                           C.c_void_p, C.c_void_p]),
 }
 
 

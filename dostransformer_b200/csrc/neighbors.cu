@@ -202,6 +202,28 @@ __global__ void gaussian_expand_kernel(const double* __restrict__ dist, long lon
   }
 }
 
+// Its distance gradient: d_dist[e] = sum_f d_out[e, f] phi_f (-2 (d_e - mu_f) / var^2), phi_f recomputed in fp64 with mu_f
+// formed as above (the fp32 cast of the forward differentiates as the identity, like torch's .float()).  One warp per
+// distance, lanes over the filters, a fixed butterfly for the sum (bitwise reproducible).
+__global__ void __launch_bounds__(256) gaussian_expand_bwd_kernel(const float* __restrict__ d_out, const double* __restrict__ dist,
+                                                                  long long n, double dmin, double step, int nfilt, double var2,
+                                                                  double* __restrict__ d_dist) {
+  const int lane = threadIdx.x & 31;
+  const long long e = blockIdx.x * 8LL + (threadIdx.x >> 5);
+  if (e >= n) return;
+  const double d = dist[e];
+  double acc = 0.0;
+  for (int f = lane; f < nfilt; f += 32) {
+    const double mu = __dadd_rn(dmin, __dmul_rn((double)f, step));
+    const double u = __dsub_rn(d, mu);
+    const double phi = exp(__ddiv_rn(-__dmul_rn(u, u), var2));
+    acc += (double)d_out[e * nfilt + f] * phi * (-2.0 * u / var2);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  if (lane == 0) d_dist[e] = acc;
+}
+
 }  // namespace
 }  // namespace dost
 
@@ -251,4 +273,13 @@ extern "C" int dost_gaussian_expand(const double* dist, long long n, double dmin
   const int blocks = (int)min64(ceil_div(total, 256), (long long)kNumSMs * 16);
   gaussian_expand_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(dist, n, dmin, step, nfilt, var * var, out);
   return check_launch("gaussian_expand");
+}
+
+extern "C" int dost_gaussian_expand_bwd(const float* d_out, const double* dist, long long n, double dmin, double step,
+                                        int nfilt, double var, double* d_dist, dost_stream_t stream) {
+  if (n == 0) return DOST_OK;
+  DOST_REQUIRE(d_out && dist && d_dist && n > 0 && nfilt > 0 && step > 0 && var > 0, "gaussian_expand_bwd: bad args");
+  gaussian_expand_bwd_kernel<<<(unsigned)((n + 7) / 8), 256, 0, (cudaStream_t)stream>>>(d_out, dist, n, dmin, step, nfilt,
+                                                                                         var * var, d_dist);
+  return check_launch("gaussian_expand_bwd");
 }

@@ -275,6 +275,63 @@ __global__ void __launch_bounds__(256) phonon_edge_encode_kernel(const T* __rest
   }
 }
 
+// Input gradient of the kernel above: d_vec[e] = J(e)^T g(e) with g_k = sum_c dv[e, c] W[c, k] (dv = gradient at the
+// pre-activation) and J the Jacobian of feat(v) = cut(|v|) [1, sqrt(3) v / max(|v|, 1e-12)], differentiated the way torch
+// autograd differentiates the reference's expression (oracle/dost_oracle.py phonon_edge_features): cut' = 0 where the
+// torch.where branches replace it (u > 0 or u < -1), else (pi/4) sin(pi u); the clamp passes the norm's gradient for
+// |v| >= 1e-12 (clamp_min's backward) and otherwise divides by the constant 1e-12 - the zero vector of a self-interaction
+// edge therefore gets sqrt(3) * 1e12 * g[1..3], as in the reference.  One warp per edge, lanes over the H columns (dv is
+// read once, coalesced); the four column sums are reduced by a fixed butterfly (bitwise reproducible).
+template <typename T>
+__global__ void __launch_bounds__(256) phonon_edge_encode_bwd_kernel(const T* __restrict__ vec, long long E,
+                                                                     const T* __restrict__ W, const T* __restrict__ dv, int H,
+                                                                     T* __restrict__ d_vec) {
+  const int lane = threadIdx.x & 31;
+  const long long e = blockIdx.x * 8LL + (threadIdx.x >> 5);
+  if (e >= E) return;
+  T g0 = T(0), g1 = T(0), g2 = T(0), g3 = T(0);
+  const T* row = dv + e * H;
+  for (int c = lane; c < H; c += 32) {
+    const T d = row[c];
+    g0 = fma(d, W[4 * c + 0], g0);
+    g1 = fma(d, W[4 * c + 1], g1);
+    g2 = fma(d, W[4 * c + 2], g2);
+    g3 = fma(d, W[4 * c + 3], g3);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    g0 += __shfl_xor_sync(0xffffffffu, g0, o);
+    g1 += __shfl_xor_sync(0xffffffffu, g1, o);
+    g2 += __shfl_xor_sync(0xffffffffu, g2, o);
+    g3 += __shfl_xor_sync(0xffffffffu, g3, o);
+  }
+  if (lane >= 3) return;
+  const T v[3] = {vec[3 * e], vec[3 * e + 1], vec[3 * e + 2]};
+  const T len = sqrt(v[0] * v[0] + v[1] * v[1] + v[2] * v[2]);
+  const T u = T(2) * (len / T(4) - T(1));
+  const T pi = T(3.14159265358979323846);
+  const T s3 = T(1.7320508075688772935);
+  T cut, dcut;                        // cut(|v|) and d cut / d|v|
+  if (u > T(0)) cut = T(0), dcut = T(0);
+  else if (u < T(-1)) cut = T(1), dcut = T(0);
+  else cut = (T(1) - cos(pi * u)) / T(2), dcut = (pi / T(4)) * sin(pi * u);
+  // lane l < 3 writes component l (selects, not indexed arrays: no local memory)
+  const T gl = lane == 0 ? g1 : (lane == 1 ? g2 : g3);
+  const T vl = lane == 0 ? v[0] : (lane == 1 ? v[1] : v[2]);
+  T r;
+  if (len >= T(1e-12)) {
+    const T inv = T(1) / len;
+    const T gn = (g1 * v[0] + g2 * v[1] + g3 * v[2]) * inv;
+    const T nl = vl * inv;
+    // d cut/dv = dcut n;  d(n_i)/dv = (I - n n^T) / |v|
+    r = dcut * (g0 + s3 * gn) * nl + s3 * cut * (gl - nl * gn) * inv;
+  } else {
+    // |v| < 2 here, so cut is the constant 1 and only the clamped direction contributes
+    r = s3 * cut * gl / T(1e-12);
+  }
+  d_vec[3 * e + lane] = r;
+}
+
 static inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 template <typename T>
@@ -395,4 +452,23 @@ extern "C" int dost_phonon_edge_encode(int dtype, const void* edge_vec, long lon
     return DOST_ERR_UNSUPPORTED;
   }
   return check_launch("phonon_edge_encode");
+}
+
+extern "C" int dost_phonon_edge_encode_bwd(int dtype, const void* edge_vec, long long E, const void* weight, const void* dv,
+                                           int H, void* d_edge_vec, dost_stream_t stream) {
+  if (E == 0) return DOST_OK;
+  DOST_REQUIRE(edge_vec && weight && dv && d_edge_vec && E > 0 && H > 0, "phonon_edge_encode_bwd: bad args");
+  cudaStream_t st = (cudaStream_t)stream;
+  const unsigned blocks = (unsigned)((E + 7) / 8);
+  if (dtype == DOST_F32)
+    phonon_edge_encode_bwd_kernel<float><<<blocks, 256, 0, st>>>((const float*)edge_vec, E, (const float*)weight,
+                                                                 (const float*)dv, H, (float*)d_edge_vec);
+  else if (dtype == DOST_F64)
+    phonon_edge_encode_bwd_kernel<double><<<blocks, 256, 0, st>>>((const double*)edge_vec, E, (const double*)weight,
+                                                                  (const double*)dv, H, (double*)d_edge_vec);
+  else {
+    set_error("phonon_edge_encode_bwd: unsupported dtype %d", dtype);
+    return DOST_ERR_UNSUPPORTED;
+  }
+  return check_launch("phonon_edge_encode_bwd");
 }

@@ -11,7 +11,8 @@ This module provides
 * ``loss_weight``         B_local / B_global, which makes SUM-reduced local gradients equal the single-process
                           gradient of the reference's mean-over-crystals loss.
 
-It is model-agnostic (works on CPU tensors with gloo, which is how the CPU tests exercise it).
+It is model-agnostic (works on CPU tensors with gloo, which is how the CPU tests exercise it).  It reduces parameter
+gradients only; gradients with respect to a rank's inputs (positions, lattices) stay local to that rank.
 """
 from __future__ import annotations
 

@@ -70,7 +70,8 @@ class _Entry:
 class GraphedStep:
     """``step = GraphedStep(model, mode="edos")``; ``loss = step(batch)`` runs forward + loss + backward (gradients in
     ``p.grad``, freshly written every call) as one graph replay.  ``train=False`` captures the forward only under
-    ``no_grad`` and returns ``(dos_global, x, dos_system)`` (static tensors).
+    ``no_grad`` and returns ``(dos_global, x, dos_system)`` (static tensors).  Only parameter gradients are carried:
+    gradients with respect to the batch's inputs (``edge_vec``, positions, lattices) need the eager step.
 
     loss_weight: scales the loss (data parallel: B_local / B_global).  world > 1: all-reduce after the replay.
     A new signature costs one eager warm-up step plus the capture (~3 eager steps); ``max_graphs`` bounds the cache

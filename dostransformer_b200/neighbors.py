@@ -7,6 +7,13 @@ self_interaction=True)`` + ``edge_vec = pos[dst] - pos[src] + shift @ lattice`` 
 (data/mat2graph.py:162-179,185,212-243).  These functions take a whole batch / dataset of crystals at once
 (``lattice`` [C,3,3], Cartesian ``pos`` [N,3], ``node_ptr`` [C+1]) and run the kernels of csrc/neighbors.cu; the edge order
 is the library's canonical one (centre atom, neighbour atom, shift), see that file.  fp64 like the reference's geometry.
+
+Gradients with respect to the structure: when ``pos`` or ``lattice`` requires grad, ``edge_vec``, ``edge_len``,
+``nbr_dist`` and ``edge_attr`` are differentiable in them.  The topology (which images are neighbours, which k are nearest)
+is held at the forward's values.  The identity edges (i, i, shift 0) of the phonon lists have ``edge_vec == 0`` for every
+geometry and contribute nothing to ``pos.grad`` / ``lattice.grad``.  The sums of the backward run in a fixed order
+(``dost_segment_reduce`` over CSR segments), so they are bitwise reproducible.  With neither input requiring grad the
+forward launches exactly the kernels it launches without this support.
 """
 from __future__ import annotations
 
@@ -15,6 +22,7 @@ from typing import Dict, Tuple
 import torch
 
 from . import _lib as L
+from . import ops
 
 
 def _prep(lattice: torch.Tensor, pos: torch.Tensor, node_ptr: torch.Tensor):
@@ -30,31 +38,81 @@ def _prep(lattice: torch.Tensor, pos: torch.Tensor, node_ptr: torch.Tensor):
     return lattice, pos, node_ptr, crystal_of
 
 
+class _NeighborList(torch.autograd.Function):
+    """The neighbour list as a function of (lattice, pos).  Forward: the count / fill kernels.  Backward, with the topology
+    fixed: g_e = d_vec_e + d_len_e v_e / |v_e| (0 on identity edges), d_pos = sum_{dst=i} g - sum_{src=i} g,
+    d_lattice[c] = sum_{e in c} shift_e^T g_e."""
+
+    @staticmethod
+    def forward(ctx, lattice, pos, node_ptr, crystal_of, cutoff, self_interaction, local_ids):
+        lib = L.lib()
+        N = pos.shape[0]
+        dev = pos.device
+        st = L.stream()
+        count = torch.zeros(N, dtype=torch.int64, device=dev)
+        L.check(lib.dost_neighbor_count(L.p(lattice), L.p(pos), L.p(node_ptr), L.p(crystal_of), N, float(cutoff),
+                                        int(self_interaction), L.p(count), st), "neighbor_count")
+        edge_ptr = torch.zeros(N + 1, dtype=torch.int64, device=dev)
+        torch.cumsum(count, 0, out=edge_ptr[1:])
+        E = int(edge_ptr[-1].item()) if N else 0
+        ei = torch.empty(2, E, dtype=torch.int64, device=dev)
+        shift = torch.empty(E, 3, dtype=torch.int64, device=dev)
+        vec = torch.empty(E, 3, dtype=torch.float64, device=dev)
+        length = torch.empty(E, dtype=torch.float64, device=dev)
+        if E:
+            L.check(lib.dost_neighbor_fill(L.p(lattice), L.p(pos), L.p(node_ptr), L.p(crystal_of), N, float(cutoff),
+                                           int(self_interaction), L.p(edge_ptr), int(local_ids), L.p(ei[0]), L.p(ei[1]),
+                                           L.p(shift), L.p(vec), L.p(length), st), "neighbor_fill")
+        ctx.mark_non_differentiable(ei, shift, edge_ptr)
+        ctx.set_materialize_grads(False)
+        if any(ctx.needs_input_grad[:2]):
+            ctx.save_for_backward(ei, shift, vec, length, edge_ptr, node_ptr, crystal_of)
+            ctx.local_ids = bool(local_ids)
+        return ei, shift, vec, length, edge_ptr
+
+    @staticmethod
+    def backward(ctx, _ei, _shift, d_vec, d_len, _ptr):
+        ei, shift, vec, length, edge_ptr, node_ptr, crystal_of = ctx.saved_tensors
+        E, N, C = vec.shape[0], edge_ptr.numel() - 1, node_ptr.numel() - 1
+        dev = vec.device
+        d_pos = torch.zeros(N, 3, dtype=torch.float64, device=dev)
+        d_lat = torch.zeros(C, 3, 3, dtype=torch.float64, device=dev)
+        if E == 0 or (d_vec is None and d_len is None):
+            return d_lat, d_pos, None, None, None, None, None
+        g = torch.zeros(E, 3, dtype=torch.float64, device=dev) if d_vec is None else d_vec.to(torch.float64)
+        if d_len is not None:
+            # |v|' = v / |v|; 0 at |v| = 0 like torch's norm (only identity edges have |v| = 0, and they are dropped below)
+            g = g + d_len.to(torch.float64)[:, None] * torch.where(length[:, None] > 0, vec / length[:, None], 0.0)
+        centre = torch.repeat_interleave(torch.arange(N, device=dev), edge_ptr[1:] - edge_ptr[:-1], output_size=E)
+        dst = ei[1] + node_ptr[crystal_of[centre]] if ctx.local_ids else ei[1]
+        # identity edges: edge_vec == 0 whatever the geometry; their (possibly ~1e12) gradient rows must not enter the sums
+        identity = (dst == centre) & (shift == 0).all(dim=1)
+        g = g.masked_fill(identity[:, None], 0.0).contiguous()
+        want_lat = ctx.needs_input_grad[0] and C > 0
+        # one pass over the edges grouped by centre (= src): per atom, sum g and (for the lattice) shift^T g; the lattice
+        # gradient is then the sum over each crystal's atoms - two short fixed-order sums instead of one serial chain
+        # over all of a crystal's edges
+        cols = torch.cat([g, (shift.to(torch.float64)[:, :, None] * g[:, None, :]).reshape(E, 9)], 1) if want_lat else g
+        per_atom = ops.segment_reduce_raw(cols, ops.to_i32(edge_ptr), None, N)
+        if ctx.needs_input_grad[1]:
+            by_dst, _ = ops.csr_build(ops.to_i32(dst), N)
+            ops.segment_reduce_raw(g, by_dst.rowptr, by_dst.perm, N, out=d_pos)
+            d_pos -= per_atom[:, :3]
+        if want_lat:
+            ops.segment_reduce_raw(per_atom[:, 3:], ops.to_i32(node_ptr), None, C, out=d_lat.view(C, 9))
+        return d_lat, d_pos, None, None, None, None, None
+
+
 def neighbor_list(lattice: torch.Tensor, pos: torch.Tensor, node_ptr: torch.Tensor, cutoff: float,
                   self_interaction: bool = True, local_ids: bool = False) -> Dict[str, torch.Tensor]:
     """All periodic images within ``cutoff`` of every atom.  Returns ``edge_index`` [2,E] (row 0 = centre, row 1 =
     neighbour; ids local to the crystal if ``local_ids`` else rows of ``pos``), ``edge_shift`` [E,3] int64, ``edge_vec`` [E,3],
     ``edge_len`` [E] and ``edge_ptr`` [N+1] (edges of atom i are edge_ptr[i]..edge_ptr[i+1]).  One device->host read
-    (the edge total) sizes the outputs; this is the offline stage of the reference."""
-    lib = L.lib()
+    (the edge total) sizes the outputs; this is the offline stage of the reference.  ``edge_vec`` and ``edge_len`` are
+    differentiable in ``lattice`` and ``pos`` (topology fixed, see the module docstring)."""
     lattice, pos, node_ptr, crystal_of = _prep(lattice, pos, node_ptr)
-    N = pos.shape[0]
-    dev = pos.device
-    st = L.stream()
-    count = torch.zeros(N, dtype=torch.int64, device=dev)
-    L.check(lib.dost_neighbor_count(L.p(lattice), L.p(pos), L.p(node_ptr), L.p(crystal_of), N, float(cutoff),
-                                    int(self_interaction), L.p(count), st), "neighbor_count")
-    edge_ptr = torch.zeros(N + 1, dtype=torch.int64, device=dev)
-    torch.cumsum(count, 0, out=edge_ptr[1:])
-    E = int(edge_ptr[-1].item()) if N else 0
-    ei = torch.empty(2, E, dtype=torch.int64, device=dev)
-    shift = torch.empty(E, 3, dtype=torch.int64, device=dev)
-    vec = torch.empty(E, 3, dtype=torch.float64, device=dev)
-    length = torch.empty(E, dtype=torch.float64, device=dev)
-    if E:
-        L.check(lib.dost_neighbor_fill(L.p(lattice), L.p(pos), L.p(node_ptr), L.p(crystal_of), N, float(cutoff),
-                                       int(self_interaction), L.p(edge_ptr), int(local_ids), L.p(ei[0]), L.p(ei[1]),
-                                       L.p(shift), L.p(vec), L.p(length), st), "neighbor_fill")
+    ei, shift, vec, length, edge_ptr = _NeighborList.apply(lattice, pos, node_ptr, crystal_of, float(cutoff),
+                                                          bool(self_interaction), bool(local_ids))
     return {"edge_index": ei, "edge_shift": shift, "edge_vec": vec, "edge_len": length, "edge_ptr": edge_ptr}
 
 
@@ -63,28 +121,76 @@ def phonon_edges(lattice, pos, node_ptr, r_max: float = 4.0) -> Dict[str, torch.
     return neighbor_list(lattice, pos, node_ptr, r_max, self_interaction=True, local_ids=False)
 
 
+class _KnnSelect(torch.autograd.Function):
+    """k nearest entries of every atom's list (dost_knn_select); dist is differentiable in edge_len: the gradient of a
+    slot goes to the list edge it picked (out_edge), padded slots (edge id -1) carry none."""
+
+    @staticmethod
+    def forward(ctx, edge_len, edge_ptr, edge_dst, k, pad_idx, pad_dist):
+        N = edge_ptr.numel() - 1
+        dev = edge_ptr.device
+        idx = torch.empty(N, k, dtype=torch.int64, device=dev)
+        dist = torch.empty(N, k, dtype=torch.float64, device=dev)
+        out_edge = torch.empty(N, k, dtype=torch.int64, device=dev) if ctx.needs_input_grad[0] else None
+        L.check(L.lib().dost_knn_select(L.p(edge_ptr), L.p(edge_dst), L.p(edge_len), N, k, pad_idx, float(pad_dist),
+                                        L.p(idx), L.p(dist), L.p(out_edge), L.stream()), "knn_select")
+        ctx.mark_non_differentiable(idx)
+        ctx.set_materialize_grads(False)
+        if out_edge is not None:
+            ctx.save_for_backward(out_edge)
+            ctx.E = edge_len.numel()
+        return idx, dist
+
+    @staticmethod
+    def backward(ctx, _idx, d_dist):
+        (out_edge,) = ctx.saved_tensors
+        E = ctx.E
+        if d_dist is None or E == 0 or out_edge.numel() == 0:
+            return torch.zeros(E, dtype=torch.float64, device=out_edge.device), None, None, None, None, None
+        # each list edge is picked at most once; padded slots are routed to an extra segment E that is dropped
+        key = torch.where(out_edge >= 0, out_edge, E).reshape(-1)
+        by_edge, _ = ops.csr_build(ops.to_i32(key), E + 1)
+        d_len = ops.segment_reduce_raw(d_dist.to(torch.float64).reshape(-1, 1).contiguous(), by_edge.rowptr, by_edge.perm,
+                                       E + 1)
+        return d_len[:E].reshape(E), None, None, None, None, None
+
+
 def knn_select(nl: Dict[str, torch.Tensor], k: int, pad_idx: int, pad_dist: float) -> Tuple[torch.Tensor, torch.Tensor]:
-    lib = L.lib()
     edge_ptr = nl["edge_ptr"]
-    N = edge_ptr.numel() - 1
-    dev = edge_ptr.device
-    idx = torch.empty(N, k, dtype=torch.int64, device=dev)
-    dist = torch.empty(N, k, dtype=torch.float64, device=dev)
     dst = nl["edge_index"][1].contiguous()
-    L.check(lib.dost_knn_select(L.p(edge_ptr), L.p(dst), L.p(nl["edge_len"]), N, k, pad_idx, float(pad_dist), L.p(idx),
-                                L.p(dist), None, L.stream()), "knn_select")
-    return idx, dist
+    return _KnnSelect.apply(nl["edge_len"], edge_ptr, dst, int(k), int(pad_idx), float(pad_dist))
+
+
+class _GaussianExpand(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, flat, dmin, step, nfilt):
+        out = torch.empty(flat.numel(), nfilt, dtype=torch.float32, device=flat.device)
+        L.check(L.lib().dost_gaussian_expand(L.p(flat), flat.numel(), dmin, step, nfilt, step, L.p(out), L.stream()),
+                "gaussian_expand")
+        if ctx.needs_input_grad[0]:
+            ctx.save_for_backward(flat)
+            ctx.args = (dmin, step, nfilt)
+        return out
+
+    @staticmethod
+    def backward(ctx, d_out):
+        (flat,) = ctx.saved_tensors
+        dmin, step, nfilt = ctx.args
+        d_out = d_out.to(torch.float32).contiguous()
+        d_dist = torch.empty(flat.numel(), dtype=torch.float64, device=flat.device)
+        L.check(L.lib().dost_gaussian_expand_bwd(L.p(d_out), L.p(flat), flat.numel(), dmin, step, nfilt, step, L.p(d_dist),
+                                                 L.stream()), "gaussian_expand_bwd")
+        return d_dist, None, None, None
 
 
 def gaussian_expand(dist: torch.Tensor, dmin: float = 0.0, dmax: float = 8.0, step: float = 0.2) -> torch.Tensor:
-    """GaussianDistance(dmin, dmax, step).expand + fp32 cast (mat2graph.py:162-179,235): [..., nfilt]."""
-    lib = L.lib()
+    """GaussianDistance(dmin, dmax, step).expand + fp32 cast (mat2graph.py:162-179,235): [..., nfilt].  Differentiable in
+    ``dist`` (dost_gaussian_expand_bwd; the fp32 cast counts as the identity, as torch's ``.float()`` does)."""
+    L.lib()
     import numpy as np
     nfilt = int(np.arange(dmin, dmax + step, step).shape[0])      # the reference's own filter count (41 for 0..8 by 0.2)
     flat = dist.to(torch.float64).contiguous().reshape(-1)
-    out = torch.empty(flat.numel(), nfilt, dtype=torch.float32, device=dist.device)
-    L.check(lib.dost_gaussian_expand(L.p(flat), flat.numel(), float(dmin), float(step), nfilt, float(step), L.p(out),
-                                     L.stream()), "gaussian_expand")
+    out = _GaussianExpand.apply(flat, float(dmin), float(step), nfilt)
     return out.reshape(tuple(dist.shape) + (nfilt,))
 
 

@@ -1837,26 +1837,28 @@ def eval_metrics(pred: torch.Tensor, target: torch.Tensor, clamp_pred: bool = Tr
 class _PhononEdgeEncode(torch.autograd.Function):
     """First Linear + PReLU of the phonon model's edge encoder with the edge features (smooth cutoff x l <= 1 spherical
     harmonics of edge_vec, DOSTransformer_phonon.py:74-77) computed inside the same kernel: the [E, 4] feature tensor never
-    exists in the forward.  The backward recomputes it once for the weight gradient."""
+    exists in the forward.  The backward recomputes it once for the weight gradient; the edge_vec gradient
+    (dost_phonon_edge_encode_bwd) is formed only when edge_vec requires grad."""
 
     @staticmethod
     def forward(ctx, edge_vec, weight, bias, slope):
         ev = edge_vec.contiguous()
         w = weight.contiguous()
         E, H = ev.shape[0], w.shape[0]
-        need = any(ctx.needs_input_grad[1:])
+        need = any(ctx.needs_input_grad)
         pre = torch.empty(E, H, dtype=ev.dtype, device=ev.device) if need else None
         out = torch.empty(E, H, dtype=ev.dtype, device=ev.device)
         L.check(L.lib().dost_phonon_edge_encode(L.dt(ev), L.p(ev), E, L.p(w), L.p(bias), L.p(slope), H, L.p(pre), L.p(out),
                                                 L.stream()), "phonon_edge_encode")
         if need:
-            ctx.save_for_backward(ev, slope, pre)
+            ctx.save_for_backward(ev, w, slope, pre)
         ctx.has_bias = bias is not None
         return out
 
     @staticmethod
     def backward(ctx, d_out):
-        ev, slope, pre = ctx.saved_tensors
+        ev, w, slope, pre = ctx.saved_tensors
+        needs = ctx.needs_input_grad
         E, H = pre.shape
         dev, dtype = pre.device, pre.dtype
         d_out = d_out.contiguous()
@@ -1867,12 +1869,19 @@ class _PhononEdgeEncode(torch.autograd.Function):
         ws = _ws(nb, dev)
         L.check(lib.dost_prelu_bwd(L.dt(d_out), L.p(d_out), L.p(pre), L.p(slope), L.p(dv), L.p(d_slope), d_out.numel(), L.p(ws), nb,
                                    L.stream()), "prelu_bwd")
-        feat = phonon_edge_features(ev)
-        d_w = torch.empty(H, 4, dtype=dtype, device=dev)
-        gemm_raw(M=H, N=4, K=E, a=[(dv, None)], a_mode=L.MC, b=feat, b_mode=L.MC, out=d_w,
-                 split_k=_pick_split(H, 4, E, dv.element_size()), prec=L.PREC_FMA)
-        d_b = colsum(dv) if ctx.has_bias else None
-        return None, d_w, d_b, d_slope
+        d_w = None
+        if needs[1]:
+            feat = phonon_edge_features(ev)
+            d_w = torch.empty(H, 4, dtype=dtype, device=dev)
+            gemm_raw(M=H, N=4, K=E, a=[(dv, None)], a_mode=L.MC, b=feat, b_mode=L.MC, out=d_w,
+                     split_k=_pick_split(H, 4, E, dv.element_size()), prec=L.PREC_FMA)
+        d_b = colsum(dv) if (ctx.has_bias and needs[2]) else None
+        d_ev = None
+        if needs[0]:
+            d_ev = torch.empty(E, 3, dtype=dtype, device=dev)
+            L.check(lib.dost_phonon_edge_encode_bwd(L.dt(ev), L.p(ev), E, L.p(w), L.p(dv), H, L.p(d_ev), L.stream()),
+                    "phonon_edge_encode_bwd")
+        return d_ev, d_w, d_b, (d_slope if needs[3] else None)
 
 
 def phonon_edge_encode(edge_vec: torch.Tensor, weight: torch.Tensor, bias, slope: torch.Tensor) -> torch.Tensor:

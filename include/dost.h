@@ -270,6 +270,11 @@ int dost_phonon_edge_feat(int dtype, const void* edge_vec, long long E, void* ou
  * tensor is never written.  pre may be NULL (inference). */
 int dost_phonon_edge_encode(int dtype, const void* edge_vec, long long E, const void* weight, const void* bias,
                             const void* prelu_slope, int H, void* pre, void* out, dost_stream_t stream);
+/* its edge_vec gradient: dv [E, H] is the gradient at the pre-activation; d_edge_vec [E, 3] = J^T (dv . weight) with J the
+ * Jacobian of the features as torch autograd forms it for the reference's expression (cutoff derivative 0 outside
+ * 2 < |v| < 4; |v| < 1e-12, e.g. a self-interaction edge: no norm gradient, the direction divided by the clamp 1e-12). */
+int dost_phonon_edge_encode_bwd(int dtype, const void* edge_vec, long long E, const void* weight, const void* dv, int H,
+                                void* d_edge_vec, dost_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Ragged energy->atom cross attention with analytic phantom keys: to_dense_batch zero padding +
@@ -490,6 +495,10 @@ int dost_knn_select(const int64_t* edge_ptr, const int64_t* edge_dst, const doub
  * fp64 then rounded to fp32 like torch.Tensor(numpy_array) does. */
 int dost_gaussian_expand(const double* dist, long long n, double dmin, double step, int nfilt, double var, float* out,
                          dost_stream_t stream);
+/* Its distance gradient: d_dist [n] fp64 = sum_f d_out[e, f] * phi_f * (-2 (d - mu_f) / var^2), phi_f recomputed in fp64
+ * (the fp32 cast counts as the identity); one fixed summation order. */
+int dost_gaussian_expand_bwd(const float* d_out, const double* dist, long long n, double dmin, double step, int nfilt,
+                             double var, double* d_dist, dost_stream_t stream);
 
 #ifdef __cplusplus
 }

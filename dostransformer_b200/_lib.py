@@ -195,6 +195,10 @@ _SIGNATURES = {
                                        C.c_void_p]),
     "dost_gaussian_expand_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_double, C.c_double, C.c_int, C.c_double,
                                            C.c_void_p, C.c_void_p]),
+    "dost_edge_geometry": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong,
+                                     C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "dost_edge_geometry_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_longlong, C.c_int, C.c_void_p, C.c_void_p]),
 }
 
 

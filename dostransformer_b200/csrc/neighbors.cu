@@ -224,6 +224,64 @@ __global__ void __launch_bounds__(256) gaussian_expand_bwd_kernel(const float* _
   if (lane == 0) d_dist[e] = acc;
 }
 
+// The geometry of a fixed list: v = (pos[dst] - pos[src]) + s and |v| through image_dist, the operations neighbor_kernel
+// performs, so at the geometry the list was built at the results are its bits.  dst < 0 marks a padded slot: len = pad, v = 0.
+__global__ void edge_geometry_kernel(const double* __restrict__ lattice, const double* __restrict__ pos,
+                                     const long long* __restrict__ crystal_of, const long long* __restrict__ src,
+                                     const long long* __restrict__ dst, const long long* __restrict__ shift, long long n,
+                                     double pad, double* __restrict__ edge_vec, double* __restrict__ edge_len) {
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
+    const long long j = dst[e];
+    double v[3] = {0.0, 0.0, 0.0}, d = pad;
+    if (j >= 0) {
+      const long long i = src[e];
+      double dp[3];
+#pragma unroll
+      for (int k = 0; k < 3; ++k) dp[k] = __dsub_rn(pos[3 * j + k], pos[3 * i + k]);
+      d = image_dist(lattice + 9 * crystal_of[i], dp, (int)shift[3 * e], (int)shift[3 * e + 1], (int)shift[3 * e + 2], v);
+    }
+    if (edge_vec) {
+      edge_vec[3 * e] = v[0];
+      edge_vec[3 * e + 1] = v[1];
+      edge_vec[3 * e + 2] = v[2];
+    }
+    if (edge_len) edge_len[e] = d;
+  }
+}
+
+// g_e = d_vec_e + d_len_e v_e / |v_e| (v / |v| := 0 at |v| = 0), 0 on identity edges (i, i, 0) and padded slots; with the
+// lattice columns g[e, 3 + 3a + b] = S_a g_b.  The operations of the torch expression in neighbors._edge_grad, one by one.
+__global__ void edge_geometry_bwd_kernel(const double* __restrict__ d_vec, const double* __restrict__ d_len,
+                                         const double* __restrict__ edge_vec, const double* __restrict__ edge_len,
+                                         const long long* __restrict__ src, const long long* __restrict__ dst,
+                                         const long long* __restrict__ shift, long long n, int with_lattice,
+                                         double* __restrict__ g) {
+  const int ld = with_lattice ? 12 : 3;
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
+    const long long j = dst[e];
+    const long long s[3] = {shift[3 * e], shift[3 * e + 1], shift[3 * e + 2]};
+    const bool drop = j < 0 || (j == src[e] && s[0] == 0 && s[1] == 0 && s[2] == 0);
+    double gv[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      double t = d_vec ? d_vec[3 * e + c] : 0.0;
+      if (d_len) {
+        const double l = edge_len[e];
+        const double u = l > 0.0 ? __ddiv_rn(edge_vec[3 * e + c], l) : 0.0;
+        t = __dadd_rn(t, __dmul_rn(d_len[e], u));
+      }
+      gv[c] = drop ? 0.0 : t;
+      g[e * ld + c] = gv[c];
+    }
+    if (with_lattice) {
+#pragma unroll
+      for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int b = 0; b < 3; ++b) g[e * ld + 3 + 3 * a + b] = __dmul_rn((double)s[a], gv[b]);
+    }
+  }
+}
+
 }  // namespace
 }  // namespace dost
 
@@ -282,4 +340,29 @@ extern "C" int dost_gaussian_expand_bwd(const float* d_out, const double* dist, 
   gaussian_expand_bwd_kernel<<<(unsigned)((n + 7) / 8), 256, 0, (cudaStream_t)stream>>>(d_out, dist, n, dmin, step, nfilt,
                                                                                          var * var, d_dist);
   return check_launch("gaussian_expand_bwd");
+}
+
+extern "C" int dost_edge_geometry(const double* lattice, const double* pos, const int64_t* crystal_of, const int64_t* src,
+                                  const int64_t* dst, const int64_t* shift, long long n, double pad, double* edge_vec,
+                                  double* edge_len, dost_stream_t stream) {
+  if (n == 0) return DOST_OK;
+  DOST_REQUIRE(lattice && pos && crystal_of && src && dst && shift && (edge_vec || edge_len) && n > 0,
+               "edge_geometry: bad args");
+  const int blocks = (int)min64(ceil_div(n, 256), (long long)kNumSMs * 16);
+  edge_geometry_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(
+      lattice, pos, (const long long*)crystal_of, (const long long*)src, (const long long*)dst, (const long long*)shift, n,
+      pad, edge_vec, edge_len);
+  return check_launch("edge_geometry");
+}
+
+extern "C" int dost_edge_geometry_bwd(const double* d_vec, const double* d_len, const double* edge_vec,
+                                      const double* edge_len, const int64_t* src, const int64_t* dst, const int64_t* shift,
+                                      long long n, int with_lattice, double* g, dost_stream_t stream) {
+  if (n == 0) return DOST_OK;
+  DOST_REQUIRE(src && dst && shift && g && n > 0 && (!d_len || (edge_vec && edge_len)), "edge_geometry_bwd: bad args");
+  const int blocks = (int)min64(ceil_div(n, 256), (long long)kNumSMs * 16);
+  edge_geometry_bwd_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(
+      d_vec, d_len, edge_vec, edge_len, (const long long*)src, (const long long*)dst, (const long long*)shift, n,
+      with_lattice, g);
+  return check_launch("edge_geometry_bwd");
 }

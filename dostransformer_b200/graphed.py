@@ -64,14 +64,37 @@ def allreduce_gradients(params, group=None, average: bool = False) -> None:
 
 
 class _Entry:
-    __slots__ = ("graph", "static", "out", "launches", "tensor_keys", "grads", "leaves")
+    __slots__ = ("graph", "static", "out", "launches", "tensor_keys", "grads", "leaves", "topo", "input_leaves",
+                 "input_grad")
+
+
+_TOPO = "topology."          # prefix of the topology's tensors among a structure input's fields
+
+
+def _structure_input(topo, lattice, pos, x, per_crystal) -> CrystalBatch:
+    """One flat batch of a structure step's tensors (the topology's, lattice, pos, the atom rows, the per-crystal fields):
+    they are copied into the static buffers and enter the signature like any batch's tensors."""
+    fields = {_TOPO + k: v for k, v in topo.tensors().items()}
+    fields.update(lattice=lattice, pos=pos, x=x, **per_crystal)
+    s = CrystalBatch(**fields)
+    s.topology_host = tuple(sorted((k, v) for k, v in topo.host().items()))
+    s.topology = topo
+    return s
 
 
 class GraphedStep:
     """``step = GraphedStep(model, mode="edos")``; ``loss = step(batch)`` runs forward + loss + backward (gradients in
     ``p.grad``, freshly written every call) as one graph replay.  ``train=False`` captures the forward only under
-    ``no_grad`` and returns ``(dos_global, x, dos_system)`` (static tensors).  Only parameter gradients are carried:
-    gradients with respect to the batch's inputs (``edge_vec``, positions, lattices) need the eager step.
+    ``no_grad`` and returns ``(dos_global, x, dos_system)`` (static tensors).
+
+    Structure gradients: ``GraphedStep(model, mode, structure=True)`` takes ``step(topology, lattice, pos, x,
+    **per_crystal)`` instead of a batch, with ``topology`` from ``neighbors.phonon_topology`` / ``edos_topology`` and ``x``
+    the atom rows its ``batch`` takes.  The graph contains ``topology.batch(lattice, pos, x, **per_crystal)``, so each
+    replay recomputes the edge geometry at the given positions; a training replay also leaves the gradients of the loss
+    with respect to ``pos`` and ``lattice`` in ``step.input_grad["pos"]`` / ``["lattice"]`` (static tensors the next replay
+    of that signature overwrites).  The topology's tensors are inputs like the others: a rebuilt topology with the same
+    shapes replays the same graph, another edge count captures a new one.  Without ``structure`` only parameter gradients
+    are carried.
 
     loss_weight: scales the loss (data parallel: B_local / B_global).  world > 1: all-reduce after the replay.
     A new signature costs one eager warm-up step plus the capture (~3 eager steps); ``max_graphs`` bounds the cache
@@ -79,8 +102,11 @@ class GraphedStep:
     """
 
     def __init__(self, model, mode: str = "edos", beta: float = 1.0, *, train: bool = True, loss_weight: float = 1.0,
-                 group=None, world: int = 1, max_graphs: int = 16, target_key: Optional[str] = None):
+                 group=None, world: int = 1, max_graphs: int = 16, target_key: Optional[str] = None,
+                 structure: bool = False):
         self.model, self.mode, self.beta, self.train = model, mode, float(beta), train
+        self.structure = bool(structure)
+        self.input_grad: Dict[str, torch.Tensor] = {}
         self.loss_weight = float(loss_weight)
         self.group, self.world = group, int(world)
         self.max_graphs = max_graphs
@@ -131,12 +157,27 @@ class GraphedStep:
         loss.backward()
         return loss.detach()       # (a loss with its grad_fn would keep the whole autograd graph of a capture alive)
 
+    def _input(self, e: _Entry):
+        """The model's batch: the static batch itself, or (structure) the topology's batch at the static positions, through
+        fresh leaves of lattice / pos (same storage) created on the current stream like the parameter leaves."""
+        if not self.structure:
+            return e.static
+        st = e.static
+        lat, pos = st.lattice, st.pos
+        if self.train:
+            lat, pos = lat.detach().requires_grad_(), pos.detach().requires_grad_()
+        e.input_leaves = {"pos": pos, "lattice": lat}
+        per_crystal = {k: getattr(st, k) for k in st.keys() if not k.startswith(_TOPO) and k not in ("lattice", "pos", "x")}
+        return e.topo.batch(lat, pos, st.x, **per_crystal)
+
     def _capture(self, g) -> _Entry:
         dev = g.x.device
         e = _Entry()
         e.tensor_keys = [k for k in g.keys() if torch.is_tensor(getattr(g, k))]
         e.static = CrystalBatch(**{k: (getattr(g, k).clone() if torch.is_tensor(getattr(g, k)) else getattr(g, k))
                                    for k in g.keys()})
+        e.topo = g.topology.with_tensors({k[len(_TOPO):]: getattr(e.static, k) for k in g.keys() if k.startswith(_TOPO)}) \
+            if self.structure else None
         # Warm-up (lazy one-time initialisation: kernel attributes, index caches, allocator pools) on the SAME side stream
         # the capture will use.  Autograd runs each parameter's AccumulateGrad node on the stream that was current when
         # the node was created; a node that survives from an earlier eager iteration on the default stream would pull the
@@ -153,7 +194,7 @@ class GraphedStep:
         with torch.cuda.stream(s), device_seed(self._seed_word):
             if self.train:
                 e.leaves = {n: p.detach().requires_grad_(p.requires_grad) for n, p in self.model.named_parameters()}
-            self._eager(e.static, leaves=e.leaves)
+            self._eager(self._input(e), leaves=e.leaves)
         torch.cuda.current_stream(dev).wait_stream(s)
         torch.cuda.synchronize(dev)
         L.poll_device_errors()
@@ -166,8 +207,9 @@ class GraphedStep:
         import os
         pool = None if os.environ.get("DOST_GRAPH_PRIVATE_POOLS") else self._pool
         with torch.cuda.graph(e.graph, pool=pool, stream=s, capture_error_mode="thread_local"), device_seed(self._seed_word):
-            e.out = self._eager(e.static, refresh=True, leaves=e.leaves)
+            e.out = self._eager(self._input(e), refresh=True, leaves=e.leaves)
         e.launches = L.launch_count() - l0
+        e.input_grad = {k: t.grad for k, t in e.input_leaves.items()} if self.structure and self.train else {}
         # the gradient buffers this graph writes (graph-pool memory, fixed addresses): re-attached on every replay, since
         # another signature's capture / replay leaves p.grad pointing at ITS buffers
         e.grads = [e.leaves[n].grad for n, _ in self.model.named_parameters()] if self.train else None
@@ -177,7 +219,11 @@ class GraphedStep:
         self.captures += 1
         return e
 
-    def __call__(self, g):
+    def __call__(self, g, *structure, **per_crystal):
+        if self.structure:
+            g = _structure_input(g, *structure, per_crystal)
+        else:
+            assert not structure and not per_crystal, "positional structure inputs need GraphedStep(..., structure=True)"
         if active_recorder() is not None:
             raise RuntimeError("GraphedStep cannot run inside attention_maps(): a replayed graph has no attention maps to "
                                "record; run the model eagerly to record them")
@@ -186,6 +232,8 @@ class GraphedStep:
         attn_drop = float(getattr(self.model, "attn_drop", 0.0))
         sig = batch_signature(g) + (("model_max_num_nodes", getattr(self.model, "max_num_nodes", None)),
                                     ("attn_drop", attn_drop), ("training", self.model.training))
+        if self.structure:
+            sig += (("topology", type(g.topology).__name__, g.topology_host),)
         if self.model.training and attn_drop > 0.0:
             # exactly the host draw of the eager step (nn_core._Seeds); a capture draws nothing.  No sync, no device read.
             if self._seed_word is None:
@@ -205,6 +253,7 @@ class GraphedStep:
         if e.grads is not None:
             for p, gr in zip(self._params, e.grads):
                 p.grad = gr
+        self.input_grad = e.input_grad
         self.replays += 1
         self.launches += e.launches
         if self.train and self.world > 1:

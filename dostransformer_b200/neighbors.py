@@ -14,6 +14,10 @@ is held at the forward's values.  The identity edges (i, i, shift 0) of the phon
 geometry and contribute nothing to ``pos.grad`` / ``lattice.grad``.  The sums of the backward run in a fixed order
 (``dost_segment_reduce`` over CSR segments), so they are bitwise reproducible.  With neither input requiring grad the
 forward launches exactly the kernels it launches without this support.
+
+Many steps on one topology: ``phonon_topology`` / ``edos_topology`` search once and keep the list; their ``batch(lattice,
+pos, ...)`` recomputes only the edge geometry (``dost_edge_geometry``), with no device->host read, so that a CUDA graph can
+capture it (``graphed.GraphedStep(..., structure=True)``); ``matches(lattice, pos)`` tells when to rebuild.
 """
 from __future__ import annotations
 
@@ -75,32 +79,55 @@ class _NeighborList(torch.autograd.Function):
         ei, shift, vec, length, edge_ptr, node_ptr, crystal_of = ctx.saved_tensors
         E, N, C = vec.shape[0], edge_ptr.numel() - 1, node_ptr.numel() - 1
         dev = vec.device
-        d_pos = torch.zeros(N, 3, dtype=torch.float64, device=dev)
-        d_lat = torch.zeros(C, 3, 3, dtype=torch.float64, device=dev)
         if E == 0 or (d_vec is None and d_len is None):
-            return d_lat, d_pos, None, None, None, None, None
-        g = torch.zeros(E, 3, dtype=torch.float64, device=dev) if d_vec is None else d_vec.to(torch.float64)
-        if d_len is not None:
-            # |v|' = v / |v|; 0 at |v| = 0 like torch's norm (only identity edges have |v| = 0, and they are dropped below)
-            g = g + d_len.to(torch.float64)[:, None] * torch.where(length[:, None] > 0, vec / length[:, None], 0.0)
+            return (torch.zeros(C, 3, 3, dtype=torch.float64, device=dev),
+                    torch.zeros(N, 3, dtype=torch.float64, device=dev), None, None, None, None, None)
         centre = torch.repeat_interleave(torch.arange(N, device=dev), edge_ptr[1:] - edge_ptr[:-1], output_size=E)
         dst = ei[1] + node_ptr[crystal_of[centre]] if ctx.local_ids else ei[1]
-        # identity edges: edge_vec == 0 whatever the geometry; their (possibly ~1e12) gradient rows must not enter the sums
-        identity = (dst == centre) & (shift == 0).all(dim=1)
-        g = g.masked_fill(identity[:, None], 0.0).contiguous()
         want_lat = ctx.needs_input_grad[0] and C > 0
-        # one pass over the edges grouped by centre (= src): per atom, sum g and (for the lattice) shift^T g; the lattice
-        # gradient is then the sum over each crystal's atoms - two short fixed-order sums instead of one serial chain
-        # over all of a crystal's edges
-        cols = torch.cat([g, (shift.to(torch.float64)[:, :, None] * g[:, None, :]).reshape(E, 9)], 1) if want_lat else g
-        per_atom = ops.segment_reduce_raw(cols, ops.to_i32(edge_ptr), None, N)
+        cols = _edge_grad(d_vec, d_len, vec, length, centre, dst, shift, want_lat)
+        rowptr = perm = None
         if ctx.needs_input_grad[1]:
             by_dst, _ = ops.csr_build(ops.to_i32(dst), N)
-            ops.segment_reduce_raw(g, by_dst.rowptr, by_dst.perm, N, out=d_pos)
-            d_pos -= per_atom[:, :3]
-        if want_lat:
-            ops.segment_reduce_raw(per_atom[:, 3:], ops.to_i32(node_ptr), None, C, out=d_lat.view(C, 9))
+            rowptr, perm = by_dst.rowptr, by_dst.perm
+        d_lat, d_pos = _structure_grad(cols, ops.to_i32(edge_ptr), rowptr, perm, ops.to_i32(node_ptr), N, C,
+                                       ctx.needs_input_grad[1], want_lat)
         return d_lat, d_pos, None, None, None, None, None
+
+
+def _edge_grad(d_vec, d_len, vec, length, src, dst, shift, want_lat):
+    """Per-edge structure gradient g_e = d_vec_e + d_len_e v_e / |v_e|, 0 on the identity edges; with ``want_lat`` [E,12]:
+    g, then the 9 columns shift_e^T g_e (column 3 + 3a + b = S_a g_b), else [E,3].  ``dost_edge_geometry_bwd`` performs
+    these operations one by one."""
+    E = vec.shape[0]
+    g = torch.zeros(E, 3, dtype=torch.float64, device=vec.device) if d_vec is None else d_vec.to(torch.float64)
+    if d_len is not None:
+        # |v|' = v / |v|; 0 at |v| = 0 like torch's norm (only identity edges have |v| = 0, and they are dropped below)
+        g = g + d_len.to(torch.float64)[:, None] * torch.where(length[:, None] > 0, vec / length[:, None], 0.0)
+    # identity edges: edge_vec == 0 whatever the geometry; their (possibly ~1e12) gradient rows must not enter the sums
+    identity = (dst == src) & (shift == 0).all(dim=1)
+    g = g.masked_fill(identity[:, None], 0.0).contiguous()
+    return torch.cat([g, (shift.to(torch.float64)[:, :, None] * g[:, None, :]).reshape(E, 9)], 1) if want_lat else g
+
+
+def _structure_grad(cols, edge_ptr32, dst_rowptr, dst_perm, node_ptr32, N, C, want_pos, want_lat):
+    """The per-edge gradients ``cols`` (``_edge_grad``'s layout; edges grouped by source atom along ``edge_ptr32``,
+    ``dst_rowptr`` / ``dst_perm`` the CSR of their destination atoms, its first N segments used) -> (d_lattice [C,3,3],
+    d_pos [N,3]): d_pos = sum_{dst=i} g - sum_{src=i} g, d_lattice[c] = sum_{e in c} shift_e^T g_e, every sum in a fixed
+    order.  ``_NeighborList`` and the topologies' backward both reduce here."""
+    dev = cols.device
+    d_pos = torch.zeros(N, 3, dtype=torch.float64, device=dev)
+    d_lat = torch.zeros(C, 3, 3, dtype=torch.float64, device=dev)
+    # one pass over the edges grouped by centre (= src): per atom, sum g and (for the lattice) shift^T g; the lattice
+    # gradient is then the sum over each crystal's atoms - two short fixed-order sums instead of one serial chain
+    # over all of a crystal's edges
+    per_atom = ops.segment_reduce_raw(cols, edge_ptr32, None, N)
+    if want_pos:
+        ops.segment_reduce_raw(cols[:, :3], dst_rowptr, dst_perm, N, out=d_pos)
+        d_pos -= per_atom[:, :3]
+    if want_lat:
+        ops.segment_reduce_raw(per_atom[:, 3:], node_ptr32, None, C, out=d_lat.view(C, 9))
+    return d_lat, d_pos
 
 
 def neighbor_list(lattice: torch.Tensor, pos: torch.Tensor, node_ptr: torch.Tensor, cutoff: float,
@@ -251,3 +278,166 @@ def phonon_graph_batch(lattice, pos, node_ptr, x: torch.Tensor, r_max: float = 4
     batch = torch.repeat_interleave(torch.arange(C, device=dev, dtype=torch.int64), counts, output_size=pos.shape[0])
     return CrystalBatch(x=x.to(dev), edge_index=nl["edge_index"], edge_vec=nl["edge_vec"], edge_shift=nl["edge_shift"],
                         batch=batch, **per_crystal)
+
+
+# ------------------------------------------------------------------------------------------------ reusable topologies
+class _EdgeGeometry(torch.autograd.Function):
+    """The edge vectors (``want_vec``) or lengths of a topology's fixed list as a function of (lattice, pos):
+    ``dost_edge_geometry`` forward, ``dost_edge_geometry_bwd`` + ``_structure_grad`` backward.  No host read either way."""
+
+    @staticmethod
+    def forward(ctx, lattice, pos, topo, want_vec):
+        E = topo.src.numel()
+        dev = pos.device
+        need = any(ctx.needs_input_grad[:2])
+        vec = torch.empty(E, 3, dtype=torch.float64, device=dev) if want_vec or need else None
+        length = None if want_vec else torch.empty(E, dtype=torch.float64, device=dev)
+        L.check(L.lib().dost_edge_geometry(L.p(lattice), L.p(pos), L.p(topo.crystal_of), L.p(topo.src), L.p(topo.dst),
+                                           L.p(topo.shift), E, float(topo.pad), L.p(vec), L.p(length), L.stream()),
+                "edge_geometry")
+        ctx.set_materialize_grads(False)
+        if need:
+            ctx.save_for_backward(vec, length)
+            ctx.topo = topo
+        return vec if want_vec else length
+
+    @staticmethod
+    def backward(ctx, d_out):
+        vec, length = ctx.saved_tensors
+        t = ctx.topo
+        E, N, C = t.src.numel(), t.crystal_of.numel(), t.node_ptr.numel() - 1
+        want_pos, want_lat = ctx.needs_input_grad[1], ctx.needs_input_grad[0] and C > 0
+        if E == 0 or d_out is None:
+            return (torch.zeros(C, 3, 3, dtype=torch.float64, device=vec.device),
+                    torch.zeros(N, 3, dtype=torch.float64, device=vec.device), None, None)
+        d_out = d_out.to(torch.float64).contiguous()
+        d_vec, d_len = (d_out, None) if length is None else (None, d_out)
+        cols = torch.empty(E, 12 if want_lat else 3, dtype=torch.float64, device=vec.device)
+        L.check(L.lib().dost_edge_geometry_bwd(L.p(d_vec), L.p(d_len), L.p(vec), L.p(length), L.p(t.src), L.p(t.dst),
+                                               L.p(t.shift), E, int(want_lat), L.p(cols), L.stream()), "edge_geometry_bwd")
+        d_lat, d_pos = _structure_grad(cols, t.src_ptr, t.dst_rowptr, t.dst_perm, t.node_ptr32, N, C, want_pos, want_lat)
+        return d_lat, d_pos, None, None
+
+
+class _Topology:
+    """A neighbour list held fixed while the geometry moves: integer device tensors (the ``TENSORS`` fields) plus host
+    values.  Entry e joins ``src[e]`` to ``dst[e]`` (rows of ``pos``; ``dst < 0``: a padded eDOS slot) through the image
+    ``shift[e]``; entries are grouped by source along ``src_ptr`` (int32 [N+1]); ``dst_rowptr`` / ``dst_perm`` group them
+    by destination (built once here instead of in every backward).  ``batch(lattice, pos, ...)`` is differentiable in
+    ``lattice`` / ``pos``, reads nothing back to the host and can be captured in a CUDA graph; the identity entries
+    (i, i, 0) and padded slots carry no gradient."""
+    TENSORS = ("src", "dst", "shift", "src_ptr", "dst_rowptr", "dst_perm", "node_ptr", "node_ptr32", "crystal_of",
+               "edge_index", "batch_of")
+
+    def __init__(self, **fields):
+        for k, v in fields.items():
+            setattr(self, k, v)
+
+    def tensors(self) -> Dict[str, torch.Tensor]:
+        return {k: getattr(self, k) for k in self.TENSORS}
+
+    def host(self) -> Dict[str, object]:
+        return {k: v for k, v in vars(self).items() if k not in self.TENSORS}
+
+    def with_tensors(self, tensors: Dict[str, torch.Tensor]):
+        """The same host values over other tensors of the same shapes (a CUDA graph's static buffers)."""
+        return type(self)(**self.host(), **tensors)
+
+    def _geometry(self, lattice, pos, want_vec):
+        assert lattice.shape == (self.node_ptr.numel() - 1, 3, 3) and pos.shape == (self.crystal_of.numel(), 3)
+        return _EdgeGeometry.apply(lattice.to(torch.float64).contiguous(), pos.to(torch.float64).contiguous(), self,
+                                   want_vec)
+
+    def _same(self, fresh) -> bool:
+        keys = ("src", "dst", "shift")
+        return all(getattr(self, k).shape == getattr(fresh, k).shape for k in keys) and \
+            all(torch.equal(getattr(self, k), getattr(fresh, k)) for k in keys)
+
+
+def _topology_common(src, dst, shift, src_ptr32, node_ptr, crystal_of, N, padded):
+    """The CSR of the entries by destination (``_NeighborList.backward``'s for a list without ``padded`` slots; padded
+    slots, dst < 0, go to a segment N past the atoms)."""
+    key = torch.where(dst >= 0, dst, N) if padded else dst
+    by_dst, _ = ops.csr_build(ops.to_i32(key), N + 1 if padded else N)
+    return dict(src=src, dst=dst, shift=shift, src_ptr=src_ptr32, dst_rowptr=by_dst.rowptr, dst_perm=by_dst.perm,
+                node_ptr=node_ptr, node_ptr32=ops.to_i32(node_ptr), crystal_of=crystal_of)
+
+
+class PhononTopology(_Topology):
+    """``phonon_topology``'s result: the entries are the edges of ``phonon_edges`` in their order."""
+
+    def batch(self, lattice, pos, x: torch.Tensor, **per_crystal):
+        """The phonon model's input batch at (lattice, pos): ``phonon_graph_batch``'s fields, ``edge_vec`` recomputed on
+        the fixed list (bitwise ``phonon_graph_batch``'s at the geometry the list was built at)."""
+        from .synthetic import CrystalBatch
+        vec = self._geometry(lattice, pos, True)
+        return CrystalBatch(x=x.to(pos.device), edge_index=self.edge_index, edge_vec=vec, edge_shift=self.shift,
+                            batch=self.batch_of, **per_crystal)
+
+    def matches(self, lattice, pos) -> bool:
+        """Rebuild the list at (lattice, pos) (one host read) and compare edges and their order with this one."""
+        return self._same(phonon_topology(lattice, pos, self.node_ptr, self.r_max))
+
+
+class EdosTopology(_Topology):
+    """``edos_topology``'s result: N*k slots, slot i*k + r = the r-th nearest neighbour of atom i (its list edge: dst and
+    shift), or a padded slot (dst = -1, distance radius + 1).  ``rows`` places the atoms among the prompt nodes."""
+    TENSORS = _Topology.TENSORS + ("rows",)
+
+    def batch(self, lattice, pos, atom_feats: torch.Tensor, **per_crystal):
+        """The eDOS model's input batch at (lattice, pos): ``edos_graph_batch``'s fields, the picked distances recomputed on
+        the fixed slots (bitwise ``edos_graph_batch``'s at the geometry the slots were picked at)."""
+        from .synthetic import CrystalBatch
+        dist = self._geometry(lattice, pos, False)
+        N, C = self.crystal_of.numel(), self.node_ptr.numel() - 1
+        feats = gaussian_expand(dist.view(N, self.k), 0.0, self.radius, 0.2)
+        x = torch.zeros(N + C, atom_feats.shape[1], dtype=atom_feats.dtype, device=pos.device)
+        x[self.rows] = atom_feats.to(pos.device)
+        return CrystalBatch(x=x, edge_index=self.edge_index, edge_attr=feats.reshape(N * self.k, -1), batch=self.batch_of,
+                            max_num_nodes=self.max_num_nodes, **per_crystal)
+
+    def matches(self, lattice, pos) -> bool:
+        """Rebuild at (lattice, pos) (one host read) and compare every slot's picked neighbour and shift with this one."""
+        return self._same(edos_topology(lattice, pos, self.node_ptr, self.radius, self.k))
+
+
+def phonon_topology(lattice, pos, node_ptr, r_max: float = 4.0) -> PhononTopology:
+    """The phonon list of ``phonon_edges`` at (lattice, pos), kept for reuse at other geometries (one host read, here)."""
+    with torch.no_grad():
+        lattice, pos, node_ptr, crystal_of = _prep(lattice.detach(), pos.detach(), node_ptr)
+        ei, shift, _, _, edge_ptr = _NeighborList.apply(lattice, pos, node_ptr, crystal_of, float(r_max), True, False)
+        N = pos.shape[0]
+        t = _topology_common(ei[0], ei[1], shift, ops.to_i32(edge_ptr), node_ptr, crystal_of, N, False)
+        return PhononTopology(**t, edge_index=ei, batch_of=crystal_of, r_max=float(r_max), pad=0.0)
+
+
+def edos_topology(lattice, pos, node_ptr, radius: float = 8.0, k: int = 12) -> EdosTopology:
+    """The k nearest images within ``radius`` of every atom at (lattice, pos) (``edos_edges``' picks), kept for reuse at
+    other geometries (one host read, here)."""
+    with torch.no_grad():
+        lattice, pos, node_ptr, crystal_of = _prep(lattice.detach(), pos.detach(), node_ptr)
+        ei, shift, _, length, edge_ptr = _NeighborList.apply(lattice, pos, node_ptr, crystal_of, float(radius), False, True)
+        N, C, dev = pos.shape[0], lattice.shape[0], pos.device
+        idx = torch.empty(N, k, dtype=torch.int64, device=dev)
+        dist = torch.empty(N, k, dtype=torch.float64, device=dev)
+        pick = torch.empty(N, k, dtype=torch.int64, device=dev)
+        L.check(L.lib().dost_knn_select(L.p(edge_ptr), L.p(ei[1].contiguous()), L.p(length), N, k, 0, float(radius) + 1.0,
+                                        L.p(idx), L.p(dist), L.p(pick), L.stream()), "knn_select")
+        first = node_ptr[crystal_of]                                               # first row of each atom's crystal
+        E = ei.shape[1]
+        sel = torch.where(pick >= 0, pick, E).reshape(-1)                         # padded slots -> an appended row
+        dst = torch.cat([ei[1], ei.new_full((1,), -1)])[sel].view(N, k)
+        dst = torch.where(dst >= 0, dst + first[:, None], -1).reshape(-1)
+        shift = torch.cat([shift, shift.new_zeros(1, 3)])[sel]
+        src = torch.arange(N, device=dev, dtype=torch.int64).repeat_interleave(k)
+        src_ptr = torch.arange(0, N * k + 1, k, device=dev, dtype=torch.int32)
+        t = _topology_common(src, dst, shift, src_ptr, node_ptr, crystal_of, N, True)
+        # the model's edge_index and node layout, as edos_edges / edos_graph_batch build them
+        nbr = (idx + first[:, None]).reshape(-1)
+        edge_index = torch.stack([src + crystal_of[src], nbr + crystal_of[nbr]])
+        counts = node_ptr[1:] - node_ptr[:-1]
+        batch_of = torch.repeat_interleave(torch.arange(C, device=dev, dtype=torch.int64), counts + 1, output_size=N + C)
+        rows = torch.arange(N, device=dev, dtype=torch.int64) + crystal_of
+        nmax = int(counts.max().item()) + 1 if C else 0
+        return EdosTopology(**t, edge_index=edge_index, batch_of=batch_of, rows=rows, radius=float(radius), k=int(k),
+                            pad=float(radius) + 1.0, max_num_nodes=nmax)

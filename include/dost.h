@@ -499,6 +499,19 @@ int dost_gaussian_expand(const double* dist, long long n, double dmin, double st
  * (the fp32 cast counts as the identity); one fixed summation order. */
 int dost_gaussian_expand_bwd(const float* d_out, const double* dist, long long n, double dmin, double step, int nfilt,
                              double var, double* d_dist, dost_stream_t stream);
+/* The geometry of a fixed list at new positions / lattices (the topology held, the edge vectors recomputed): per entry e,
+ * src[e], dst[e] rows of pos, shift [n,3] int64, the lattice of crystal_of[src[e]]; v = (pos[dst] - pos[src]) + s and
+ * d = |v| by the arithmetic contract above, so at the geometry of a dost_neighbor_fill list the results are its bits.
+ * dst[e] < 0 marks a padded slot: d = pad, v = 0.  Optional edge_vec [n,3], edge_len [n] (at least one). */
+int dost_edge_geometry(const double* lattice, const double* pos, const int64_t* crystal_of, const int64_t* src,
+                       const int64_t* dst, const int64_t* shift, long long n, double pad, double* edge_vec, double* edge_len,
+                       dost_stream_t stream);
+/* Its per-entry backward: g_e = d_vec_e + d_len_e * v_e / |v_e| (v / |v| taken as 0 at |v| = 0; either gradient may be
+ * NULL, edge_vec / edge_len are needed with d_len), each op rounded; 0 on identity entries (src == dst, shift 0) and
+ * padded slots.  g [n,3], or with with_lattice [n,12]: the 3 columns of g, then S_a * g_b at column 3 + 3a + b. */
+int dost_edge_geometry_bwd(const double* d_vec, const double* d_len, const double* edge_vec, const double* edge_len,
+                           const int64_t* src, const int64_t* dst, const int64_t* shift, long long n, int with_lattice,
+                           double* g, dost_stream_t stream);
 
 #ifdef __cplusplus
 }

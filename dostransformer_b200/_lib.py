@@ -199,6 +199,9 @@ _SIGNATURES = {
                                      C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]),
     "dost_edge_geometry_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                          C.c_longlong, C.c_int, C.c_void_p, C.c_void_p]),
+    "dost_knn_reselect": (C.c_int, [C.c_void_p] * 7 + [C.c_longlong, C.c_int, C.c_double, C.c_double] + [C.c_void_p] * 8),
+    "dost_topology_check": (C.c_int, [C.c_void_p] * 5 + [C.c_longlong, C.c_double, C.c_double] + [C.c_void_p] * 5
+                            + [C.c_longlong, C.c_void_p, C.c_void_p]),
 }
 
 

@@ -282,6 +282,163 @@ __global__ void edge_geometry_bwd_kernel(const double* __restrict__ d_vec, const
   }
 }
 
+// The re-pick of a skin topology: atom i's candidates (every image within cutoff + skin at the build geometry, canonical
+// order, rows cand_ptr[i]..cand_ptr[i+1]) get their distance at the current geometry through image_dist (written to
+// cand_len, and the vector to cand_vec when given), then the k nearest with d < cutoff are selected exactly as
+// knn_select_kernel selects from a list: smallest (d, candidate id) first.  Filtering the candidates at d < cutoff leaves
+// the list a fresh search at this geometry finds, in the same order and with the same bits, whenever the candidates
+// contain every pair within the cutoff (dost_topology_check tells when they may not).  One warp per atom.
+__global__ void __launch_bounds__(128) knn_reselect_kernel(
+    const double* __restrict__ lattice, const double* __restrict__ pos, const long long* __restrict__ node_ptr,
+    const long long* __restrict__ crystal_of, const int* __restrict__ cand_ptr, const long long* __restrict__ cand_dst,
+    const long long* __restrict__ cand_shift, long long N, int k, double cutoff, double pad_dist,
+    double* __restrict__ cand_len, double* __restrict__ cand_vec, long long* __restrict__ out_pick,
+    double* __restrict__ out_dist, long long* __restrict__ out_nbr, long long* __restrict__ out_shift,
+    long long* __restrict__ out_edge_index) {
+  const int lane = threadIdx.x & 31;
+  const long long i = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (i >= N) return;
+  const long long c = crystal_of[i];
+  const double* L = lattice + 9 * c;
+  const long long e0 = cand_ptr[i], e1 = cand_ptr[i + 1];
+  for (long long e = e0 + lane; e < e1; e += 32) {
+    const long long j = cand_dst[e];
+    double dp[3], v[3];
+#pragma unroll
+    for (int q = 0; q < 3; ++q) dp[q] = __dsub_rn(pos[3 * j + q], pos[3 * i + q]);
+    cand_len[e] = image_dist(L, dp, (int)cand_shift[3 * e], (int)cand_shift[3 * e + 1], (int)cand_shift[3 * e + 2], v);
+    if (cand_vec) {
+      cand_vec[3 * e] = v[0];
+      cand_vec[3 * e + 1] = v[1];
+      cand_vec[3 * e + 2] = v[2];
+    }
+  }
+  __syncwarp();             // the distances of the whole segment are visible to every lane
+  double last_d = -1.0;
+  long long last_e = -1;
+  bool done = false;
+  for (int r = 0; r < k; ++r) {
+    double bd = 0.0;
+    long long be = -1;
+    if (!done) {
+      for (long long e = e0 + lane; e < e1; e += 32) {
+        const double d = cand_len[e];
+        if (!(d < cutoff)) continue;
+        const bool after = d > last_d || (d == last_d && e > last_e);
+        if (after && (be < 0 || d < bd)) {
+          bd = d;
+          be = e;
+        }
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        const double od = __shfl_xor_sync(0xffffffffu, bd, o);
+        const long long oe = __shfl_xor_sync(0xffffffffu, be, o);
+        if (oe >= 0 && (be < 0 || od < bd || (od == bd && oe < be))) {
+          bd = od;
+          be = oe;
+        }
+      }
+    }
+    if (lane == 0) {
+      const long long s = i * k + r;
+      out_pick[s] = be;
+      out_dist[s] = be >= 0 ? bd : pad_dist;
+      const long long j = be >= 0 ? cand_dst[be] : -1;
+      if (out_nbr) out_nbr[s] = j;
+      if (out_shift)
+#pragma unroll
+        for (int q = 0; q < 3; ++q) out_shift[3 * s + q] = be >= 0 ? cand_shift[3 * be + q] : 0;
+      if (out_edge_index) {      // the model's node ids: one prompt node per preceding crystal; padded slots -> atom 0
+        out_edge_index[s] = i + c;
+        out_edge_index[N * k + s] = (j >= 0 ? j : node_ptr[c]) + c;
+      }
+    }
+    done = be < 0;          // list exhausted: the remaining slots are padded
+    last_d = bd;
+    last_e = be;
+  }
+}
+
+// Completeness of a skin list, and (phonon) whether a held edge set is still the list at the current geometry.  Sets
+// *flag = 1 (never clears it) when the result of the topology may differ from a fresh search.
+//
+// Per crystal, build cell L0 and positions p0, current cell L and positions p (unwrapped), fractional coordinates
+// f = p L^-1, f0 = p0 L0^-1 (rows are vectors throughout).  A pair (i, j, S) has v = (f_j - f_i + S) L = u L now and
+// v0 = (f0_j - f0_i + S) L0 = u0 L0 at the build.  With u - u0 = (f_j - f0_j) - (f_i - f0_i) and
+// delta = max_i |(f_i - f0_i) L|:  |u0 L| <= |v| + 2 delta.  With eps = ||L0^-1 (L - L0)||_F (>= the spectral norm):
+// u0 L = v0 + v0 L0^-1 (L - L0), so |u0 L| >= |v0| (1 - eps).  Hence, for eps < 1, every pair with |v| < r now had
+// |v0| < (r + 2 delta) / (1 - eps) at the build, and the candidates (every image with |v0| < r + skin) contain every pair
+// within r as long as (r + 2 delta) / (1 - eps) <= r + skin.  The flag is set when eps >= 1 or
+// (r + 2 delta) / (1 - eps) * (1 + kSkinSlack) >= r + skin: the relative slack covers the rounding of eps, delta and the
+// distances themselves (all fp64, errors ~1e-15 relative) with a wide margin; a NaN anywhere sets the flag.
+//
+// Phonon: cand_held[e] says whether candidate e is one of the held edges (d < cutoff at the build); the flag is also set
+// when its status at the current geometry (image_dist, d < cutoff) differs.  Warps 0..C-1 test one crystal each (lanes
+// over its atoms); every thread then walks the candidates grid-stride.
+constexpr double kSkinSlack = 1e-9;
+
+__global__ void __launch_bounds__(256) topology_check_kernel(
+    const double* __restrict__ lattice, const double* __restrict__ pos, const double* __restrict__ lattice0,
+    const double* __restrict__ pos0, const long long* __restrict__ node_ptr, long long C, double cutoff, double skin,
+    const long long* __restrict__ crystal_of, const long long* __restrict__ cand_src,
+    const long long* __restrict__ cand_dst, const long long* __restrict__ cand_shift,
+    const unsigned char* __restrict__ cand_held, long long n_cand, int* __restrict__ flag) {
+  const int lane = threadIdx.x & 31;
+  const long long w = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (w < C) {
+    Cell cur, ref;
+    make_cell(lattice + 9 * w, cur);
+    make_cell(lattice0 + 9 * w, ref);
+    double delta = 0.0;
+    for (long long a = node_ptr[w] + lane; a < node_ptr[w + 1]; a += 32) {
+      double df[3], m = 0.0;
+#pragma unroll
+      for (int q = 0; q < 3; ++q) {
+        const double f = pos[3 * a] * cur.Li[q] + pos[3 * a + 1] * cur.Li[3 + q] + pos[3 * a + 2] * cur.Li[6 + q];
+        const double f0 = pos0[3 * a] * ref.Li[q] + pos0[3 * a + 1] * ref.Li[3 + q] + pos0[3 * a + 2] * ref.Li[6 + q];
+        df[q] = f - f0;
+      }
+#pragma unroll
+      for (int q = 0; q < 3; ++q) {
+        const double x = df[0] * cur.L[q] + df[1] * cur.L[3 + q] + df[2] * cur.L[6 + q];
+        m += x * x;
+      }
+      m = sqrt(m);
+      delta = (m > delta || m != m) ? m : delta;           // a NaN propagates
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const double od = __shfl_xor_sync(0xffffffffu, delta, o);
+      delta = (od > delta || od != od) ? od : delta;
+    }
+    if (lane == 0) {
+      double eps2 = 0.0;       // ||L0^-1 (L - L0)||_F^2; L0^-1[a][m] = ref.Li[3a + m]
+#pragma unroll
+      for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int b = 0; b < 3; ++b) {
+          double x = 0.0;
+#pragma unroll
+          for (int m = 0; m < 3; ++m) x += ref.Li[3 * a + m] * (cur.L[3 * m + b] - ref.L[3 * m + b]);
+          eps2 += x * x;
+        }
+      const double eps = sqrt(eps2);
+      const bool complete = eps < 1.0 && (cutoff + 2.0 * delta) / (1.0 - eps) * (1.0 + kSkinSlack) < cutoff + skin;
+      if (!complete) *flag = 1;
+    }
+  }
+  for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < n_cand; e += (long long)gridDim.x * blockDim.x) {
+    const long long i = cand_src[e], j = cand_dst[e];
+    double dp[3], v[3];
+#pragma unroll
+    for (int q = 0; q < 3; ++q) dp[q] = __dsub_rn(pos[3 * j + q], pos[3 * i + q]);
+    const double d = image_dist(lattice + 9 * crystal_of[i], dp, (int)cand_shift[3 * e], (int)cand_shift[3 * e + 1],
+                                (int)cand_shift[3 * e + 2], v);
+    if ((d < cutoff) != (cand_held[e] != 0)) *flag = 1;
+  }
+}
+
 }  // namespace
 }  // namespace dost
 
@@ -365,4 +522,37 @@ extern "C" int dost_edge_geometry_bwd(const double* d_vec, const double* d_len, 
       d_vec, d_len, edge_vec, edge_len, (const long long*)src, (const long long*)dst, (const long long*)shift, n,
       with_lattice, g);
   return check_launch("edge_geometry_bwd");
+}
+
+extern "C" int dost_knn_reselect(const double* lattice, const double* pos, const int64_t* node_ptr,
+                                 const int64_t* crystal_of, const int32_t* cand_ptr, const int64_t* cand_dst,
+                                 const int64_t* cand_shift, long long N, int k, double cutoff, double pad_dist,
+                                 double* cand_len, double* cand_vec, int64_t* out_pick, double* out_dist, int64_t* out_nbr,
+                                 int64_t* out_shift, int64_t* out_edge_index, dost_stream_t stream) {
+  if (N == 0 || k == 0) return DOST_OK;
+  DOST_REQUIRE(lattice && pos && node_ptr && crystal_of && cand_ptr && cand_dst && cand_shift && cand_len && out_pick &&
+                   out_dist && N > 0 && k > 0 && cutoff > 0,
+               "knn_reselect: bad args");
+  knn_reselect_kernel<<<ceil_div(N, 4), 128, 0, (cudaStream_t)stream>>>(
+      lattice, pos, (const long long*)node_ptr, (const long long*)crystal_of, cand_ptr, (const long long*)cand_dst,
+      (const long long*)cand_shift, N, k, cutoff, pad_dist, cand_len, cand_vec, (long long*)out_pick, out_dist,
+      (long long*)out_nbr, (long long*)out_shift, (long long*)out_edge_index);
+  return check_launch("knn_reselect");
+}
+
+extern "C" int dost_topology_check(const double* lattice, const double* pos, const double* lattice0, const double* pos0,
+                                   const int64_t* node_ptr, long long C, double cutoff, double skin,
+                                   const int64_t* crystal_of, const int64_t* cand_src, const int64_t* cand_dst,
+                                   const int64_t* cand_shift, const uint8_t* cand_held, long long n_cand, int32_t* flag,
+                                   dost_stream_t stream) {
+  if (C == 0) return DOST_OK;
+  DOST_REQUIRE(lattice && pos && lattice0 && pos0 && node_ptr && flag && C > 0 && cutoff > 0 && skin >= 0 && n_cand >= 0 &&
+                   (n_cand == 0 || (crystal_of && cand_src && cand_dst && cand_shift && cand_held)),
+               "topology_check: bad args");
+  const long long per_crystal = ceil_div(C, 8), per_cand = min64(ceil_div(n_cand, 256), (long long)kNumSMs * 16);
+  const int blocks = (int)(per_crystal > per_cand ? per_crystal : per_cand);
+  topology_check_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(
+      lattice, pos, lattice0, pos0, (const long long*)node_ptr, C, cutoff, skin, (const long long*)crystal_of,
+      (const long long*)cand_src, (const long long*)cand_dst, (const long long*)cand_shift, cand_held, n_cand, flag);
+  return check_launch("topology_check");
 }

@@ -93,8 +93,9 @@ class GraphedStep:
     replay recomputes the edge geometry at the given positions; a training replay also leaves the gradients of the loss
     with respect to ``pos`` and ``lattice`` in ``step.input_grad["pos"]`` / ``["lattice"]`` (static tensors the next replay
     of that signature overwrites).  The topology's tensors are inputs like the others: a rebuilt topology with the same
-    shapes replays the same graph, another edge count captures a new one.  Without ``structure`` only parameter gradients
-    are carried.
+    shapes replays the same graph, another edge count captures a new one.  Skin topologies (``skin=``) work the same way:
+    each replay re-picks the eDOS neighbours of the given positions and runs the topology check, and the replay's flag is
+    ORed into the caller's ``topology.stale`` on the device.  Without ``structure`` only parameter gradients are carried.
 
     loss_weight: scales the loss (data parallel: B_local / B_global).  world > 1: all-reduce after the replay.
     A new signature costs one eager warm-up step plus the capture (~3 eager steps); ``max_graphs`` bounds the cache
@@ -250,6 +251,10 @@ class GraphedStep:
             if src.data_ptr() != dst.data_ptr():
                 dst.copy_(src, non_blocking=True)
         e.graph.replay()
+        stale = getattr(e.static, _TOPO + "stale", None) if self.structure else None
+        if stale is not None and getattr(g, _TOPO + "stale").data_ptr() != stale.data_ptr():
+            # a skin topology: the replay ORed into the static copy of the caller's flag; hand the result back (no host read)
+            getattr(g, _TOPO + "stale").copy_(stale, non_blocking=True)
         if e.grads is not None:
             for p, gr in zip(self._params, e.grads):
                 p.grad = gr

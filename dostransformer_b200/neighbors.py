@@ -17,7 +17,10 @@ forward launches exactly the kernels it launches without this support.
 
 Many steps on one topology: ``phonon_topology`` / ``edos_topology`` search once and keep the list; their ``batch(lattice,
 pos, ...)`` recomputes only the edge geometry (``dost_edge_geometry``), with no device->host read, so that a CUDA graph can
-capture it (``graphed.GraphedStep(..., structure=True)``); ``matches(lattice, pos)`` tells when to rebuild.
+capture it (``graphed.GraphedStep(..., structure=True)``); ``matches(lattice, pos)`` tells when to rebuild.  With
+``skin=s`` they keep every image within cutoff + s instead (a Verlet skin): the eDOS topology re-picks its k nearest on the
+device at every geometry, the phonon topology holds its edges, and both set the device flag ``stale`` when their batch may
+differ from a fresh build (``_Skin``).
 """
 from __future__ import annotations
 
@@ -312,11 +315,17 @@ class _EdgeGeometry(torch.autograd.Function):
                     torch.zeros(N, 3, dtype=torch.float64, device=vec.device), None, None)
         d_out = d_out.to(torch.float64).contiguous()
         d_vec, d_len = (d_out, None) if length is None else (None, d_out)
-        cols = torch.empty(E, 12 if want_lat else 3, dtype=torch.float64, device=vec.device)
-        L.check(L.lib().dost_edge_geometry_bwd(L.p(d_vec), L.p(d_len), L.p(vec), L.p(length), L.p(t.src), L.p(t.dst),
-                                               L.p(t.shift), E, int(want_lat), L.p(cols), L.stream()), "edge_geometry_bwd")
-        d_lat, d_pos = _structure_grad(cols, t.src_ptr, t.dst_rowptr, t.dst_perm, t.node_ptr32, N, C, want_pos, want_lat)
-        return d_lat, d_pos, None, None
+        return (*_topology_grad(t, d_vec, d_len, vec, length, want_pos, want_lat), None, None)
+
+
+def _topology_grad(t, d_vec, d_len, vec, length, want_pos, want_lat):
+    """(d_lattice, d_pos) of a topology's entries (``t.src`` / ``dst`` / ``shift`` and their CSR sums) from the per-entry
+    gradients: ``dost_edge_geometry_bwd``, then ``_structure_grad``."""
+    E, N, C = t.src.numel(), t.crystal_of.numel(), t.node_ptr.numel() - 1
+    cols = torch.empty(E, 12 if want_lat else 3, dtype=torch.float64, device=t.src.device)
+    L.check(L.lib().dost_edge_geometry_bwd(L.p(d_vec), L.p(d_len), L.p(vec), L.p(length), L.p(t.src), L.p(t.dst),
+                                           L.p(t.shift), E, int(want_lat), L.p(cols), L.stream()), "edge_geometry_bwd")
+    return _structure_grad(cols, t.src_ptr, t.dst_rowptr, t.dst_perm, t.node_ptr32, N, C, want_pos, want_lat)
 
 
 class _Topology:
@@ -401,19 +410,44 @@ class EdosTopology(_Topology):
         return self._same(edos_topology(lattice, pos, self.node_ptr, self.radius, self.k))
 
 
-def phonon_topology(lattice, pos, node_ptr, r_max: float = 4.0) -> PhononTopology:
-    """The phonon list of ``phonon_edges`` at (lattice, pos), kept for reuse at other geometries (one host read, here)."""
+def _skin_fields(lattice, pos, skin):
+    skin = float(skin)
+    if not skin >= 0.0:
+        raise ValueError(f"skin must be >= 0, got {skin}")
+    return dict(lattice0=lattice.clone(), pos0=pos.clone(), stale=torch.zeros(1, dtype=torch.int32, device=pos.device),
+                skin=skin)
+
+
+def phonon_topology(lattice, pos, node_ptr, r_max: float = 4.0, *, skin=None) -> PhononTopology:
+    """The phonon list of ``phonon_edges`` at (lattice, pos), kept for reuse at other geometries (one host read, here).
+    With ``skin`` (>= 0): a ``PhononSkinTopology`` that holds the same edges and also watches the candidates within
+    ``r_max + skin`` (see there)."""
     with torch.no_grad():
         lattice, pos, node_ptr, crystal_of = _prep(lattice.detach(), pos.detach(), node_ptr)
-        ei, shift, _, _, edge_ptr = _NeighborList.apply(lattice, pos, node_ptr, crystal_of, float(r_max), True, False)
         N = pos.shape[0]
-        t = _topology_common(ei[0], ei[1], shift, ops.to_i32(edge_ptr), node_ptr, crystal_of, N, False)
-        return PhononTopology(**t, edge_index=ei, batch_of=crystal_of, r_max=float(r_max), pad=0.0)
+        if skin is None:
+            ei, shift, _, _, edge_ptr = _NeighborList.apply(lattice, pos, node_ptr, crystal_of, float(r_max), True, False)
+            t = _topology_common(ei[0], ei[1], shift, ops.to_i32(edge_ptr), node_ptr, crystal_of, N, False)
+            return PhononTopology(**t, edge_index=ei, batch_of=crystal_of, r_max=float(r_max), pad=0.0)
+        sk = _skin_fields(lattice, pos, skin)
+        cei, cshift, _, clen, cptr = _NeighborList.apply(lattice, pos, node_ptr, crystal_of, float(r_max) + sk["skin"],
+                                                         True, False)
+        # the edges: the candidates within r_max (the fill's own distances, so the list phonon_edges finds, in its order)
+        held = clen < float(r_max)
+        before = torch.zeros(clen.numel() + 1, dtype=torch.int64, device=pos.device)
+        torch.cumsum(held, 0, out=before[1:])
+        ei, shift = cei[:, held], cshift[held]
+        t = _topology_common(ei[0], ei[1], shift, ops.to_i32(before[cptr]), node_ptr, crystal_of, N, False)
+        return PhononSkinTopology(**t, edge_index=ei, batch_of=crystal_of, r_max=float(r_max), pad=0.0, cand_src=cei[0],
+                                  cand_dst=cei[1], cand_shift=cshift, cand_held=held.to(torch.uint8), **sk)
 
 
-def edos_topology(lattice, pos, node_ptr, radius: float = 8.0, k: int = 12) -> EdosTopology:
+def edos_topology(lattice, pos, node_ptr, radius: float = 8.0, k: int = 12, *, skin=None) -> EdosTopology:
     """The k nearest images within ``radius`` of every atom at (lattice, pos) (``edos_edges``' picks), kept for reuse at
-    other geometries (one host read, here)."""
+    other geometries (one host read, here).  With ``skin`` (>= 0): an ``EdosSkinTopology`` that keeps every image within
+    ``radius + skin`` and re-picks the k nearest at each geometry (see there)."""
+    if skin is not None:
+        return _edos_skin_topology(lattice, pos, node_ptr, float(radius), int(k), skin)
     with torch.no_grad():
         lattice, pos, node_ptr, crystal_of = _prep(lattice.detach(), pos.detach(), node_ptr)
         ei, shift, _, length, edge_ptr = _NeighborList.apply(lattice, pos, node_ptr, crystal_of, float(radius), False, True)
@@ -441,3 +475,147 @@ def edos_topology(lattice, pos, node_ptr, radius: float = 8.0, k: int = 12) -> E
         nmax = int(counts.max().item()) + 1 if C else 0
         return EdosTopology(**t, edge_index=edge_index, batch_of=batch_of, rows=rows, radius=float(radius), k=int(k),
                             pad=float(radius) + 1.0, max_num_nodes=nmax)
+
+
+def _edos_skin_topology(lattice, pos, node_ptr, radius, k, skin) -> "EdosSkinTopology":
+    with torch.no_grad():
+        lattice, pos, node_ptr, crystal_of = _prep(lattice.detach(), pos.detach(), node_ptr)
+        sk = _skin_fields(lattice, pos, skin)
+        ei, shift, _, _, edge_ptr = _NeighborList.apply(lattice, pos, node_ptr, crystal_of, radius + sk["skin"], False,
+                                                        False)
+        N, C, dev = pos.shape[0], lattice.shape[0], pos.device
+        t = _topology_common(ei[0], ei[1], shift, ops.to_i32(edge_ptr), node_ptr, crystal_of, N, False)
+        counts = node_ptr[1:] - node_ptr[:-1]
+        batch_of = torch.repeat_interleave(torch.arange(C, device=dev, dtype=torch.int64), counts + 1, output_size=N + C)
+        rows = torch.arange(N, device=dev, dtype=torch.int64) + crystal_of
+        nmax = int(counts.max().item()) + 1 if C else 0
+        return EdosSkinTopology(**t, batch_of=batch_of, rows=rows, radius=radius, k=k, pad=radius + 1.0,
+                                max_num_nodes=nmax, **sk)
+
+
+# ------------------------------------------------------------------------------------------------ skin topologies
+class _Skin:
+    """What the skin topologies share: the build geometry ``lattice0`` / ``pos0``, ``skin`` and ``stale``, an int32 [1]
+    device word.  Every ``batch()`` runs ``dost_topology_check``, which sets ``stale`` when its result may differ from a
+    fresh build at that geometry; nothing clears it but ``clear()`` (or a new topology), so one 4-byte read whenever the
+    caller chooses covers every call since, eager calls and CUDA-graph replays alike.
+
+    Completeness test (per crystal, derivation in csrc/neighbors.cu): with eps = ||L0^-1 (L - L0)||_F and delta = the
+    largest move of an atom's fractional coordinates measured in the current cell, every pair within the cutoff r now
+    was within (r + 2 delta) / (1 - eps) at the build, so the candidates (within r + skin at the build) hold every
+    such pair while that bound stays below r + skin."""
+
+    def clear(self) -> None:
+        """Reset ``stale`` on the device (no host read)."""
+        self.stale.zero_()
+
+    def _check(self, lattice, pos, cutoff, cand=(None, None, None, None)):
+        src, dst, shift, held = cand
+        L.check(L.lib().dost_topology_check(L.p(lattice), L.p(pos), L.p(self.lattice0), L.p(self.pos0), L.p(self.node_ptr),
+                                            self.node_ptr.numel() - 1, float(cutoff), self.skin, L.p(self.crystal_of),
+                                            L.p(src), L.p(dst), L.p(shift), L.p(held), 0 if src is None else src.numel(),
+                                            L.p(self.stale), L.stream()), "topology_check")
+
+
+def _f64(t):
+    return t.to(torch.float64).contiguous()
+
+
+class PhononSkinTopology(_Skin, PhononTopology):
+    """``phonon_topology(..., skin=s)``: the edges of ``phonon_edges`` at the build geometry, held (the phonon model's edge
+    count is a shape, fixed inside a CUDA graph), plus the candidates (``cand_*``: every image within r_max + s at the
+    build, ``cand_held`` marking the edges).  ``batch`` is ``PhononTopology.batch`` and also sets ``stale`` when a
+    candidate crossed r_max (the held set is no longer the list) or the candidates may be incomplete.  While ``stale`` is
+    clear the batch is bitwise ``phonon_graph_batch`` at that geometry."""
+    TENSORS = PhononTopology.TENSORS + ("cand_src", "cand_dst", "cand_shift", "cand_held", "lattice0", "pos0", "stale")
+
+    def batch(self, lattice, pos, x: torch.Tensor, **per_crystal):
+        g = super().batch(lattice, pos, x, **per_crystal)
+        self._check(_f64(lattice), _f64(pos), self.r_max, (self.cand_src, self.cand_dst, self.cand_shift, self.cand_held))
+        return g
+
+
+class _Reselect(torch.autograd.Function):
+    """The skin re-pick as a function of (lattice, pos): ``dost_knn_reselect`` -> (nbr_dist [N,k], the model's
+    edge_index [2,N*k]).  Backward: a slot's distance gradient goes to the candidate it picked (each candidate is picked
+    at most once: plain stores; padded slots carry none), then ``_topology_grad`` over the candidates with their CSR by
+    destination built once.  No host read either way."""
+
+    @staticmethod
+    def forward(ctx, lattice, pos, topo):
+        N, k, E = topo.crystal_of.numel(), topo.k, topo.src.numel()
+        dev = pos.device
+        need = any(ctx.needs_input_grad[:2])
+        cand_len = torch.empty(E, dtype=torch.float64, device=dev)
+        cand_vec = torch.empty(E, 3, dtype=torch.float64, device=dev) if need else None
+        pick = torch.empty(N, k, dtype=torch.int64, device=dev)
+        dist = torch.empty(N, k, dtype=torch.float64, device=dev)
+        edge_index = torch.empty(2, N * k, dtype=torch.int64, device=dev)
+        L.check(L.lib().dost_knn_reselect(L.p(lattice), L.p(pos), L.p(topo.node_ptr), L.p(topo.crystal_of),
+                                          L.p(topo.src_ptr), L.p(topo.dst), L.p(topo.shift), N, k, topo.radius, topo.pad,
+                                          L.p(cand_len), L.p(cand_vec), L.p(pick), L.p(dist), None, None, L.p(edge_index),
+                                          L.stream()), "knn_reselect")
+        ctx.mark_non_differentiable(edge_index)
+        ctx.set_materialize_grads(False)
+        if need:
+            ctx.save_for_backward(cand_vec, cand_len, pick)
+            ctx.topo = topo
+        return dist, edge_index
+
+    @staticmethod
+    def backward(ctx, d_dist, _ei):
+        cand_vec, cand_len, pick = ctx.saved_tensors
+        t = ctx.topo
+        E, N, C = t.src.numel(), t.crystal_of.numel(), t.node_ptr.numel() - 1
+        if E == 0 or d_dist is None:
+            return (torch.zeros(C, 3, 3, dtype=torch.float64, device=pick.device),
+                    torch.zeros(N, 3, dtype=torch.float64, device=pick.device), None)
+        d_len = torch.zeros(E + 1, dtype=torch.float64, device=pick.device)
+        # padded slots all store into the extra row E, which is dropped
+        d_len.scatter_(0, torch.where(pick >= 0, pick, E).reshape(-1), d_dist.to(torch.float64).reshape(-1))
+        want_pos, want_lat = ctx.needs_input_grad[1], ctx.needs_input_grad[0] and C > 0
+        return (*_topology_grad(t, None, d_len[:E], cand_vec, cand_len, want_pos, want_lat), None)
+
+
+class EdosSkinTopology(_Skin, _Topology):
+    """``edos_topology(..., skin=s)``: the entries (``src`` / ``dst`` / ``shift``, grouped by source along ``src_ptr``) are
+    the candidates, every image within radius + s of every atom at the build geometry in canonical order.  ``batch``
+    re-picks the k nearest within ``radius`` on every call (``dost_knn_reselect``): shapes never change, only the slots'
+    contents, so one CUDA graph serves every geometry.  While ``stale`` is clear the batch is bitwise ``edos_graph_batch``
+    at that geometry; gradients reach ``pos`` / ``lattice`` through the picked candidates."""
+    TENSORS = ("src", "dst", "shift", "src_ptr", "dst_rowptr", "dst_perm", "node_ptr", "node_ptr32", "crystal_of",
+               "batch_of", "rows", "lattice0", "pos0", "stale")
+
+    def batch(self, lattice, pos, atom_feats: torch.Tensor, **per_crystal):
+        """The eDOS model's input batch at (lattice, pos): ``edos_graph_batch``'s fields, the k nearest re-picked."""
+        from .synthetic import CrystalBatch
+        N, C = self.crystal_of.numel(), self.node_ptr.numel() - 1
+        assert lattice.shape == (C, 3, 3) and pos.shape == (N, 3)
+        lattice, pos = _f64(lattice), _f64(pos)
+        dist, edge_index = _Reselect.apply(lattice, pos, self)
+        self._check(lattice, pos, self.radius)
+        feats = gaussian_expand(dist, 0.0, self.radius, 0.2)
+        x = torch.zeros(N + C, atom_feats.shape[1], dtype=atom_feats.dtype, device=pos.device)
+        x[self.rows] = atom_feats.to(pos.device)
+        return CrystalBatch(x=x, edge_index=edge_index, edge_attr=feats.reshape(N * self.k, -1), batch=self.batch_of,
+                            max_num_nodes=self.max_num_nodes, **per_crystal)
+
+    def slots(self, lattice, pos):
+        """The re-pick at (lattice, pos) without touching ``stale``: (pick [N,k] candidate ids, nbr_dist [N,k], nbr [N,k]
+        rows of ``pos``, shift [N,k,3]); padded slots are (-1, radius + 1, -1, 0)."""
+        N, k, E = self.crystal_of.numel(), self.k, self.src.numel()
+        dev = self.src.device
+        out = (torch.empty(N, k, dtype=torch.int64, device=dev), torch.empty(N, k, dtype=torch.float64, device=dev),
+               torch.empty(N, k, dtype=torch.int64, device=dev), torch.empty(N, k, 3, dtype=torch.int64, device=dev))
+        cand_len = torch.empty(E, dtype=torch.float64, device=dev)
+        lattice, pos = _f64(lattice), _f64(pos)
+        L.check(L.lib().dost_knn_reselect(L.p(lattice), L.p(pos), L.p(self.node_ptr), L.p(self.crystal_of),
+                                          L.p(self.src_ptr), L.p(self.dst), L.p(self.shift), N, k, self.radius, self.pad,
+                                          L.p(cand_len), None, *(L.p(t) for t in out), None, L.stream()), "knn_reselect")
+        return out
+
+    def matches(self, lattice, pos) -> bool:
+        """Rebuild at (lattice, pos) (one host read) and compare every slot's neighbour and shift with the re-pick there."""
+        fresh = edos_topology(lattice, pos, self.node_ptr, self.radius, self.k)
+        _, _, nbr, shift = self.slots(lattice, pos)
+        return torch.equal(fresh.dst, nbr.reshape(-1)) and torch.equal(fresh.shift, shift.reshape(-1, 3))

@@ -512,6 +512,28 @@ int dost_edge_geometry(const double* lattice, const double* pos, const int64_t* 
 int dost_edge_geometry_bwd(const double* d_vec, const double* d_len, const double* edge_vec, const double* edge_len,
                            const int64_t* src, const int64_t* dst, const int64_t* shift, long long n, int with_lattice,
                            double* g, dost_stream_t stream);
+/* Skin topologies.  The re-pick: atom i's candidates are rows cand_ptr[i]..cand_ptr[i+1] (int32 [N+1]) of cand_dst (rows of
+ * pos) / cand_shift [.,3], every image within cutoff + skin at the build geometry in canonical order.  Their distances at
+ * (lattice, pos) by the arithmetic contract go to cand_len (and the vectors to the optional cand_vec [.,3]); then, like
+ * dost_knn_select, the k nearest with d < cutoff (ties by candidate order): out_pick [N,k] = candidate id (-1 padded),
+ * out_dist [N,k] (pad_dist padded); optional out_nbr [N,k] = row of pos (-1 padded), out_shift [N,k,3] (0 padded),
+ * out_edge_index [2,N*k] = the eDOS model's node ids (row + crystal index: one prompt node per preceding crystal; padded
+ * slots point at the crystal's atom 0).  While the candidates contain every pair within cutoff, the picks, distances and
+ * edge_index are bitwise those of dost_neighbor_fill at cutoff followed by dost_knn_select. */
+int dost_knn_reselect(const double* lattice, const double* pos, const int64_t* node_ptr, const int64_t* crystal_of,
+                      const int32_t* cand_ptr, const int64_t* cand_dst, const int64_t* cand_shift, long long N, int k,
+                      double cutoff, double pad_dist, double* cand_len, double* cand_vec, int64_t* out_pick,
+                      double* out_dist, int64_t* out_nbr, int64_t* out_shift, int64_t* out_edge_index,
+                      dost_stream_t stream);
+/* Sets *flag = 1 (never clears it, never synchronises) when a skin topology's result may differ from a fresh search at
+ * (lattice, pos): per crystal, with eps = ||L0^-1 (L - L0)||_F and delta = max_i |(f_i - f0_i) L| (f = p L^-1, build cell
+ * lattice0 and positions pos0), when eps >= 1 or (cutoff + 2 delta) / (1 - eps) >= cutoff + skin (relative slack 1e-9):
+ * then a pair within cutoff may lie outside the candidates.  With n_cand > 0 (phonon), also when a candidate's status
+ * d < cutoff (by the contract; lattice of crystal_of[cand_src]) differs from cand_held (uint8 [n_cand]). */
+int dost_topology_check(const double* lattice, const double* pos, const double* lattice0, const double* pos0,
+                        const int64_t* node_ptr, long long C, double cutoff, double skin, const int64_t* crystal_of,
+                        const int64_t* cand_src, const int64_t* cand_dst, const int64_t* cand_shift,
+                        const uint8_t* cand_held, long long n_cand, int32_t* flag, dost_stream_t stream);
 
 #ifdef __cplusplus
 }

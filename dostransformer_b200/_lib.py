@@ -84,6 +84,8 @@ _SIGNATURES = {
     "dost_csr_workspace_bytes": (C.c_size_t, [C.c_longlong, C.c_longlong]),
     "dost_csr_build": (C.c_int, [C.c_void_p, C.c_longlong, C.c_longlong, C.c_void_p, C.c_void_p, C.c_void_p,
                                  C.c_void_p, C.c_size_t, C.c_void_p]),
+    "dost_csr_build_masked": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_longlong, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "dost_gemm_workspace_bytes": (C.c_size_t, [C.POINTER(Gemm)]),
     "dost_gemm": (C.c_int, [C.POINTER(Gemm), C.c_void_p, C.c_size_t, C.c_void_p]),
     "dost_gemm_bf16_workspace_bytes": (C.c_size_t, [C.POINTER(GemmBf16)]),
@@ -126,6 +128,8 @@ _SIGNATURES = {
                                       C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_longlong, C.c_void_p]),
     "dost_gather_rows": (C.c_int, [C.c_int, C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p, C.c_void_p,
                                    C.c_longlong, C.c_longlong, C.c_int, C.c_void_p, C.c_longlong, C.c_void_p]),
+    "dost_gather_rows_masked": (C.c_int, [C.c_int, C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          C.c_longlong, C.c_longlong, C.c_int, C.c_void_p, C.c_longlong, C.c_void_p]),
     "dost_phonon_edge_feat": (C.c_int, [C.c_int, C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p]),
     "dost_phonon_edge_encode": (C.c_int, [C.c_int, C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
                                           C.c_void_p, C.c_void_p]),
@@ -199,6 +203,7 @@ _SIGNATURES = {
                                      C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]),
     "dost_edge_geometry_bwd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                          C.c_longlong, C.c_int, C.c_void_p, C.c_void_p]),
+    "dost_edge_within": (C.c_int, [C.c_void_p, C.c_longlong, C.c_double, C.c_void_p, C.c_void_p]),
     "dost_knn_reselect": (C.c_int, [C.c_void_p] * 7 + [C.c_longlong, C.c_int, C.c_double, C.c_double] + [C.c_void_p] * 8),
     "dost_topology_check": (C.c_int, [C.c_void_p] * 5 + [C.c_longlong, C.c_double, C.c_double] + [C.c_void_p] * 5
                             + [C.c_longlong, C.c_void_p, C.c_void_p]),

@@ -249,6 +249,15 @@ __global__ void edge_geometry_kernel(const double* __restrict__ lattice, const d
   }
 }
 
+// Membership of a candidate list at the current geometry: mask[e] = (len[e] < cutoff), the comparison neighbor_kernel
+// applies to the same image_dist bits (written by edge_geometry_kernel), so the live entries are exactly the list a fresh
+// search at cutoff finds whenever the candidates contain it.  A NaN length is not within.
+__global__ void edge_within_kernel(const double* __restrict__ edge_len, long long n, double cutoff,
+                                   unsigned char* __restrict__ mask) {
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x)
+    mask[e] = edge_len[e] < cutoff ? 1 : 0;
+}
+
 // g_e = d_vec_e + d_len_e v_e / |v_e| (v / |v| := 0 at |v| = 0), 0 on identity edges (i, i, 0) and padded slots; with the
 // lattice columns g[e, 3 + 3a + b] = S_a g_b.  The operations of the torch expression in neighbors._edge_grad, one by one.
 __global__ void edge_geometry_bwd_kernel(const double* __restrict__ d_vec, const double* __restrict__ d_len,
@@ -522,6 +531,14 @@ extern "C" int dost_edge_geometry_bwd(const double* d_vec, const double* d_len, 
       d_vec, d_len, edge_vec, edge_len, (const long long*)src, (const long long*)dst, (const long long*)shift, n,
       with_lattice, g);
   return check_launch("edge_geometry_bwd");
+}
+
+extern "C" int dost_edge_within(const double* edge_len, long long n, double cutoff, uint8_t* mask, dost_stream_t stream) {
+  if (n == 0) return DOST_OK;
+  DOST_REQUIRE(edge_len && mask && n > 0 && cutoff > 0, "edge_within: bad args");
+  const int blocks = (int)min64(ceil_div(n, 256), (long long)kNumSMs * 16);
+  edge_within_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(edge_len, n, cutoff, mask);
+  return check_launch("edge_within");
 }
 
 extern "C" int dost_knn_reselect(const double* lattice, const double* pos, const int64_t* node_ptr,

@@ -177,12 +177,17 @@ __global__ void __launch_bounds__(kSegWarps * 32) segment_reduce_scalar_kernel(
 template <typename T, int NV>
 __global__ void __launch_bounds__(kSegWarps * 32) gather_rows_vec_kernel(
     const T* __restrict__ src, long long ld, const int* __restrict__ idx, const int* __restrict__ deg_rowptr,
-    const T* __restrict__ add, long long ld_add, long long R, int W, T* __restrict__ out, long long ldo) {
+    const T* __restrict__ add, long long ld_add, long long R, int W, T* __restrict__ out, long long ldo,
+    const unsigned char* __restrict__ mask) {
   constexpr int V = VecOf<T>::N;
   using Vec = typename VecOf<T>::type;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int nvec = W / V;
   for (long long r = blockIdx.x * (long long)kSegWarps + warp; r < R; r += (long long)gridDim.x * kSegWarps) {
+    if (mask && !__ldg(mask + r)) {      // a masked row: written as 0, idx[r] never read
+      for (int c = lane; c < W; c += 32) out[r * ldo + c] = T(0);
+      continue;
+    }
     const long long s = __ldg(idx + r);
     T sc = T(1);
     if (deg_rowptr) {
@@ -205,9 +210,14 @@ __global__ void __launch_bounds__(kSegWarps * 32) gather_rows_vec_kernel(
 template <typename T>
 __global__ void __launch_bounds__(kSegWarps * 32) gather_rows_scalar_kernel(
     const T* __restrict__ src, long long ld, const int* __restrict__ idx, const int* __restrict__ deg_rowptr,
-    const T* __restrict__ add, long long ld_add, long long R, int W, T* __restrict__ out, long long ldo) {
+    const T* __restrict__ add, long long ld_add, long long R, int W, T* __restrict__ out, long long ldo,
+    const unsigned char* __restrict__ mask) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   for (long long r = blockIdx.x * (long long)kSegWarps + warp; r < R; r += (long long)gridDim.x * kSegWarps) {
+    if (mask && !__ldg(mask + r)) {
+      for (int c = lane; c < W; c += 32) out[r * ldo + c] = T(0);
+      continue;
+    }
     const long long s = __ldg(idx + r);
     T sc = T(1);
     if (deg_rowptr) {
@@ -371,7 +381,8 @@ static int run_segment_reduce(const void* src, long long ld, const int* rowptr, 
 
 template <typename T>
 static int run_gather_rows(const void* src, long long ld, const int* idx, const int* deg_rowptr, const void* add,
-                           long long ld_add, long long R, int W, void* out, long long ldo, cudaStream_t st) {
+                           long long ld_add, long long R, int W, void* out, long long ldo, const uint8_t* mask,
+                           cudaStream_t st) {
   constexpr int V = VecOf<T>::N;
   int blocks = (int)min64((R + kSegWarps - 1) / kSegWarps, 32LL * kNumSMs);
   bool vec = (W % V == 0) && (ld % V == 0) && (ldo % V == 0) && al16(src) && al16(out) && W <= 32 * V * 8;
@@ -380,7 +391,7 @@ static int run_gather_rows(const void* src, long long ld, const int* idx, const 
     const int nv = (W / V + 31) / 32;
 #define DOST_GR(NV)                                                                                              \
   gather_rows_vec_kernel<T, NV><<<blocks, kSegWarps * 32, 0, st>>>((const T*)src, ld, idx, deg_rowptr, (const T*)add, \
-                                                                   ld_add, R, W, (T*)out, ldo)
+                                                                   ld_add, R, W, (T*)out, ldo, mask)
     if (nv <= 1) DOST_GR(1);
     else if (nv <= 2) DOST_GR(2);
     else if (nv <= 4) DOST_GR(4);
@@ -388,7 +399,7 @@ static int run_gather_rows(const void* src, long long ld, const int* idx, const 
 #undef DOST_GR
   } else {
     gather_rows_scalar_kernel<T><<<blocks, kSegWarps * 32, 0, st>>>((const T*)src, ld, idx, deg_rowptr, (const T*)add,
-                                                                    ld_add, R, W, (T*)out, ldo);
+                                                                    ld_add, R, W, (T*)out, ldo, mask);
   }
   return check_launch("gather_rows");
 }
@@ -415,9 +426,21 @@ extern "C" int dost_gather_rows(int dtype, const void* src, long long ld, const 
   if (R == 0) return DOST_OK;
   DOST_REQUIRE(src && idx && out && R > 0 && W > 0, "gather_rows: bad args");
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == DOST_F32) return run_gather_rows<float>(src, ld, idx, deg_rowptr, add, ld_add, R, W, out, ldo, st);
-  if (dtype == DOST_F64) return run_gather_rows<double>(src, ld, idx, deg_rowptr, add, ld_add, R, W, out, ldo, st);
+  if (dtype == DOST_F32) return run_gather_rows<float>(src, ld, idx, deg_rowptr, add, ld_add, R, W, out, ldo, nullptr, st);
+  if (dtype == DOST_F64) return run_gather_rows<double>(src, ld, idx, deg_rowptr, add, ld_add, R, W, out, ldo, nullptr, st);
   set_error("gather_rows: unsupported dtype %d", dtype);
+  return DOST_ERR_UNSUPPORTED;
+}
+
+extern "C" int dost_gather_rows_masked(int dtype, const void* src, long long ld, const int32_t* idx,
+                                       const int32_t* deg_rowptr, const uint8_t* mask, const void* add, long long ld_add,
+                                       long long R, int W, void* out, long long ldo, dost_stream_t stream) {
+  if (R == 0) return DOST_OK;
+  DOST_REQUIRE(src && idx && mask && out && R > 0 && W > 0, "gather_rows_masked: bad args");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == DOST_F32) return run_gather_rows<float>(src, ld, idx, deg_rowptr, add, ld_add, R, W, out, ldo, mask, st);
+  if (dtype == DOST_F64) return run_gather_rows<double>(src, ld, idx, deg_rowptr, add, ld_add, R, W, out, ldo, mask, st);
+  set_error("gather_rows_masked: unsupported dtype %d", dtype);
   return DOST_ERR_UNSUPPORTED;
 }
 

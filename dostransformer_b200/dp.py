@@ -106,6 +106,8 @@ def take_crystals(g: CrystalBatch, ids: Sequence[int]) -> CrystalBatch:
 
 def shard_batch(g: CrystalBatch, world: int, T: int, hidden: int = 256):
     """Returns (list of per-rank sub-batches, global Nmax, per-rank loss weights)."""
+    if "edge_mask" in g:
+        raise NotImplementedError("shard_batch does not carry edge_mask: shard an unmasked batch")
     B = g.system.numel()
     n = torch.bincount(g.batch, minlength=B)
     ne = torch.bincount(g.batch[g.edge_index[0]], minlength=B)

@@ -52,6 +52,9 @@ class DOSTransformer(nn.Module):
     def _forward(self, g):
         K.require_cuda(self.fc.weight, "the model")
         K.require_cuda(g.x, "the batch")
+        if "edge_mask" in g:
+            raise NotImplementedError("the eDOS model takes no edge_mask: its skin topology re-picks the bonds on the "
+                                      "device instead (neighbors.edos_topology(..., skin=s))")
         graph = ops.build_graph(g.edge_index, g.batch, g.system, nmax_override=self.max_num_nodes,
                                 need_backward=torch.is_grad_enabled(),
                                 nmax_hint=getattr(g, "max_num_nodes", None),

@@ -3,6 +3,10 @@
 Differences from the eDOS model, as in the reference: edge features are computed from ``edge_vec`` inside the
 forward (l<=1 spherical harmonics times a smooth cutoff), messages are aggregated with scatter_mean, there are no
 global features, T = 51.  Runs in the dtype of its parameters (float64 under main_phDOS.py:15-16).
+
+An optional batch field ``edge_mask`` (bool / uint8 [E] on the device) keeps only the edges with mask != 0: outputs and
+gradients are those of the batch without the other edges (``edge_vec.grad`` is 0 on their rows).  A masked edge's
+``edge_vec`` must be finite; ``neighbors.phonon_topology(..., skin=s, masked=True)`` builds such batches.
 """
 from __future__ import annotations
 
@@ -67,7 +71,8 @@ class DOSTransformer_phonon(nn.Module):
         graph = ops.build_graph(g["edge_index"], g.batch, g.system, nmax_override=self.max_num_nodes,
                                 need_backward=torch.is_grad_enabled(),
                                 nmax_hint=getattr(g, "max_num_nodes", None),
-                                phantoms=not (self.per_crystal_eval and not self.training))
+                                phantoms=not (self.per_crystal_eval and not self.training),
+                                edge_mask=g["edge_mask"] if "edge_mask" in g else None)
         seeds = K._Seeds(self.attn_drop, self.training)
         dtype = self.fc.weight.dtype
         enc = self.GN_encoder

@@ -20,7 +20,8 @@ pos, ...)`` recomputes only the edge geometry (``dost_edge_geometry``), with no 
 capture it (``graphed.GraphedStep(..., structure=True)``); ``matches(lattice, pos)`` tells when to rebuild.  With
 ``skin=s`` they keep every image within cutoff + s instead (a Verlet skin): the eDOS topology re-picks its k nearest on the
 device at every geometry, the phonon topology holds its edges, and both set the device flag ``stale`` when their batch may
-differ from a fresh build (``_Skin``).
+differ from a fresh build (``_Skin``).  ``phonon_topology(..., skin=s, masked=True)`` follows the phonon edge set instead:
+its batches carry every candidate and an ``edge_mask`` of those within r_max at each geometry.
 """
 from __future__ import annotations
 
@@ -286,21 +287,22 @@ def phonon_graph_batch(lattice, pos, node_ptr, x: torch.Tensor, r_max: float = 4
 # ------------------------------------------------------------------------------------------------ reusable topologies
 class _EdgeGeometry(torch.autograd.Function):
     """The edge vectors (``want_vec``) or lengths of a topology's fixed list as a function of (lattice, pos):
-    ``dost_edge_geometry`` forward, ``dost_edge_geometry_bwd`` + ``_structure_grad`` backward.  No host read either way."""
+    ``dost_edge_geometry`` forward, ``dost_edge_geometry_bwd`` + ``_structure_grad`` backward.  No host read either way.
+    With ``want_vec``, ``len_out`` (optional, fp64 [E]) also receives the lengths, outside autograd."""
 
     @staticmethod
-    def forward(ctx, lattice, pos, topo, want_vec):
+    def forward(ctx, lattice, pos, topo, want_vec, len_out=None):
         E = topo.src.numel()
         dev = pos.device
         need = any(ctx.needs_input_grad[:2])
         vec = torch.empty(E, 3, dtype=torch.float64, device=dev) if want_vec or need else None
-        length = None if want_vec else torch.empty(E, dtype=torch.float64, device=dev)
+        length = len_out if want_vec else torch.empty(E, dtype=torch.float64, device=dev)
         L.check(L.lib().dost_edge_geometry(L.p(lattice), L.p(pos), L.p(topo.crystal_of), L.p(topo.src), L.p(topo.dst),
                                            L.p(topo.shift), E, float(topo.pad), L.p(vec), L.p(length), L.stream()),
                 "edge_geometry")
         ctx.set_materialize_grads(False)
         if need:
-            ctx.save_for_backward(vec, length)
+            ctx.save_for_backward(vec, None if want_vec else length)
             ctx.topo = topo
         return vec if want_vec else length
 
@@ -312,10 +314,10 @@ class _EdgeGeometry(torch.autograd.Function):
         want_pos, want_lat = ctx.needs_input_grad[1], ctx.needs_input_grad[0] and C > 0
         if E == 0 or d_out is None:
             return (torch.zeros(C, 3, 3, dtype=torch.float64, device=vec.device),
-                    torch.zeros(N, 3, dtype=torch.float64, device=vec.device), None, None)
+                    torch.zeros(N, 3, dtype=torch.float64, device=vec.device), None, None, None)
         d_out = d_out.to(torch.float64).contiguous()
         d_vec, d_len = (d_out, None) if length is None else (None, d_out)
-        return (*_topology_grad(t, d_vec, d_len, vec, length, want_pos, want_lat), None, None)
+        return (*_topology_grad(t, d_vec, d_len, vec, length, want_pos, want_lat), None, None, None)
 
 
 def _topology_grad(t, d_vec, d_len, vec, length, want_pos, want_lat):
@@ -352,10 +354,10 @@ class _Topology:
         """The same host values over other tensors of the same shapes (a CUDA graph's static buffers)."""
         return type(self)(**self.host(), **tensors)
 
-    def _geometry(self, lattice, pos, want_vec):
+    def _geometry(self, lattice, pos, want_vec, len_out=None):
         assert lattice.shape == (self.node_ptr.numel() - 1, 3, 3) and pos.shape == (self.crystal_of.numel(), 3)
         return _EdgeGeometry.apply(lattice.to(torch.float64).contiguous(), pos.to(torch.float64).contiguous(), self,
-                                   want_vec)
+                                   want_vec, len_out)
 
     def _same(self, fresh) -> bool:
         keys = ("src", "dst", "shift")
@@ -418,10 +420,15 @@ def _skin_fields(lattice, pos, skin):
                 skin=skin)
 
 
-def phonon_topology(lattice, pos, node_ptr, r_max: float = 4.0, *, skin=None) -> PhononTopology:
+def phonon_topology(lattice, pos, node_ptr, r_max: float = 4.0, *, skin=None, masked: bool = False) -> PhononTopology:
     """The phonon list of ``phonon_edges`` at (lattice, pos), kept for reuse at other geometries (one host read, here).
     With ``skin`` (>= 0): a ``PhononSkinTopology`` that holds the same edges and also watches the candidates within
-    ``r_max + skin`` (see there)."""
+    ``r_max + skin`` (see there).  With ``skin`` and ``masked=True``: a ``PhononMaskedTopology`` whose batches carry every
+    candidate and an ``edge_mask`` of those within ``r_max`` at the batch's geometry (see there)."""
+    if masked:
+        if skin is None:
+            raise ValueError("phonon_topology(masked=True) needs skin=: the candidates are the images within r_max + skin")
+        return _phonon_masked_topology(lattice, pos, node_ptr, float(r_max), skin)
     with torch.no_grad():
         lattice, pos, node_ptr, crystal_of = _prep(lattice.detach(), pos.detach(), node_ptr)
         N = pos.shape[0]
@@ -533,6 +540,58 @@ class PhononSkinTopology(_Skin, PhononTopology):
         g = super().batch(lattice, pos, x, **per_crystal)
         self._check(_f64(lattice), _f64(pos), self.r_max, (self.cand_src, self.cand_dst, self.cand_shift, self.cand_held))
         return g
+
+
+def _phonon_masked_topology(lattice, pos, node_ptr, r_max, skin) -> "PhononMaskedTopology":
+    with torch.no_grad():
+        lattice, pos, node_ptr, crystal_of = _prep(lattice.detach(), pos.detach(), node_ptr)
+        sk = _skin_fields(lattice, pos, skin)
+        ei, shift, _, _, edge_ptr = _NeighborList.apply(lattice, pos, node_ptr, crystal_of, r_max + sk["skin"], True, False)
+        t = _topology_common(ei[0], ei[1], shift, ops.to_i32(edge_ptr), node_ptr, crystal_of, pos.shape[0], False)
+        return PhononMaskedTopology(**t, edge_index=ei, batch_of=crystal_of, r_max=r_max, pad=0.0, **sk)
+
+
+class PhononMaskedTopology(_Skin, _Topology):
+    """``phonon_topology(..., skin=s, masked=True)``: the entries (``src`` / ``dst`` / ``shift``, their CSR by destination
+    built once) are the candidates, every image within r_max + s at the build geometry in canonical order, identity
+    edges included.  ``batch`` carries all of them and the model's ``edge_mask``: the candidates within r_max at the
+    batch's geometry (``dost_edge_within`` on the lengths ``dost_edge_geometry`` writes, the fill's own comparison).  A
+    bond that crosses r_max is followed, not flagged: shapes never change, so one CUDA graph serves every geometry, and
+    while ``stale`` is clear the model's results are those on ``phonon_graph_batch`` at that geometry.  ``stale`` is set
+    by the completeness test only.  The masked candidates lie within r_max + s of the build geometry, so their edge
+    vectors stay finite, which the zero gradient of a masked edge relies on."""
+    TENSORS = _Topology.TENSORS + ("lattice0", "pos0", "stale")
+
+    def batch(self, lattice, pos, x: torch.Tensor, **per_crystal):
+        """The phonon model's input batch at (lattice, pos) over every candidate, with ``edge_mask`` (uint8 [E])."""
+        from .synthetic import CrystalBatch
+        lattice, pos = _f64(lattice), _f64(pos)
+        length = torch.empty(self.src.numel(), dtype=torch.float64, device=pos.device)
+        vec = self._geometry(lattice, pos, True, length)
+        mask = self.within(length)
+        self._check(lattice, pos, self.r_max)
+        return CrystalBatch(x=x.to(pos.device), edge_index=self.edge_index, edge_vec=vec, edge_shift=self.shift,
+                            edge_mask=mask, batch=self.batch_of, **per_crystal)
+
+    def within(self, length: torch.Tensor) -> torch.Tensor:
+        """uint8 [E]: candidate e is within r_max at the lengths ``length`` (``dost_edge_within``)."""
+        mask = torch.empty(length.numel(), dtype=torch.uint8, device=length.device)
+        L.check(L.lib().dost_edge_within(L.p(length), length.numel(), self.r_max, L.p(mask), L.stream()), "edge_within")
+        return mask
+
+    def live(self, lattice, pos):
+        """The candidates within r_max at (lattice, pos), without touching ``stale``: (edge_index [2,E'], shift [E',3])."""
+        with torch.no_grad():
+            length = self._geometry(_f64(lattice), _f64(pos), False)
+            keep = self.within(length).bool()
+        return self.edge_index[:, keep], self.shift[keep]
+
+    def matches(self, lattice, pos) -> bool:
+        """Rebuild the list at (lattice, pos) (one host read) and compare its edges and their order with the live
+        candidates there."""
+        fresh = phonon_topology(lattice, pos, self.node_ptr, self.r_max)
+        ei, shift = self.live(lattice, pos)
+        return ei.shape == fresh.edge_index.shape and torch.equal(ei, fresh.edge_index) and torch.equal(shift, fresh.shift)
 
 
 class _Reselect(torch.autograd.Function):

@@ -86,6 +86,9 @@ class CSR:
     perm: Optional[torch.Tensor]  # int32 [n] or None (identity)
     key: torch.Tensor         # int32 [n]  (the index the segments were built from)
     size: int
+    # uint8 [n] or None: a masked CSR's segments hold the entries with mask != 0 only (perm lists the others after
+    # rowptr[size]); the adjoint of its reduction writes 0 to the masked rows
+    mask: Optional[torch.Tensor] = None
 
 
 def to_i32(t: torch.Tensor) -> torch.Tensor:
@@ -98,7 +101,9 @@ def to_i32(t: torch.Tensor) -> torch.Tensor:
     return out
 
 
-def csr_build(key32: torch.Tensor, size: int, want_max: bool = False) -> Tuple[CSR, Optional[torch.Tensor]]:
+def csr_build(key32: torch.Tensor, size: int, want_max: bool = False,
+              mask: Optional[torch.Tensor] = None) -> Tuple[CSR, Optional[torch.Tensor]]:
+    """Stable CSR of the entries by key; with ``mask`` (uint8 [n]) of the entries with mask != 0 only."""
     n = key32.numel()
     dev = key32.device
     rowptr = torch.empty(size + 1, dtype=torch.int32, device=dev)
@@ -107,8 +112,21 @@ def csr_build(key32: torch.Tensor, size: int, want_max: bool = False) -> Tuple[C
     lib = L.lib()
     nb = lib.dost_csr_workspace_bytes(n, size)
     ws = _ws(nb, dev)
-    L.check(lib.dost_csr_build(L.p(key32), n, size, L.p(rowptr), L.p(perm), L.p(mx), L.p(ws), nb, L.stream()), "csr_build")
-    return CSR(rowptr, perm[:n], key32, size), mx
+    if mask is None:
+        L.check(lib.dost_csr_build(L.p(key32), n, size, L.p(rowptr), L.p(perm), L.p(mx), L.p(ws), nb, L.stream()),
+                "csr_build")
+    else:
+        L.check(lib.dost_csr_build_masked(L.p(key32), L.p(mask), n, size, L.p(rowptr), L.p(perm), L.p(mx), L.p(ws), nb,
+                                          L.stream()), "csr_build_masked")
+    return CSR(rowptr, perm[:n], key32, size, mask), mx
+
+
+def edge_mask_u8(edge_mask: torch.Tensor, E: int) -> torch.Tensor:
+    """A batch's ``edge_mask`` (bool or uint8 [E], on the device) as the uint8 mask of the masked kernels."""
+    if edge_mask.shape != (E,) or edge_mask.dtype not in (torch.bool, torch.uint8):
+        raise ValueError(f"edge_mask must be a bool or uint8 tensor of shape [{E}], got {edge_mask.dtype} "
+                         f"{tuple(edge_mask.shape)}")
+    return edge_mask.contiguous().view(torch.uint8)
 
 
 @dataclass
@@ -172,8 +190,13 @@ class CrystalGraph:
 
 
 def build_graph(edge_index: torch.Tensor, batch: torch.Tensor, system: torch.Tensor, *, nmax_override: Optional[int] = None,
-                need_backward: bool = True, nmax_hint: Optional[int] = None, phantoms: bool = True) -> CrystalGraph:
-    """edge_index int64 [2,E] (row = centre atom, col = neighbour), batch int64 [N] sorted, system int64 [B]."""
+                need_backward: bool = True, nmax_hint: Optional[int] = None, phantoms: bool = True,
+                edge_mask: Optional[torch.Tensor] = None) -> CrystalGraph:
+    """edge_index int64 [2,E] (row = centre atom, col = neighbour), batch int64 [N] sorted, system int64 [B].
+
+    ``edge_mask`` (bool / uint8 [E]): only the edges with mask != 0 enter ``by_dst`` / ``by_src``, in the order of the
+    batch without the others; ``row`` / ``col`` keep every edge, so the gathers x[row], x[col] of a masked edge stay in
+    bounds and compute a row that no reduction reads (``CSR.mask``)."""
     assert edge_index.is_cuda, "dostransformer_b200 has no CPU path: move the batch to a CUDA device"
     L.lib()
     L.poll_device_errors()        # invalid input skipped by the kernels of an earlier step (no synchronisation)
@@ -181,10 +204,11 @@ def build_graph(edge_index: torch.Tensor, batch: torch.Tensor, system: torch.Ten
     ei = to_i32(edge_index)
     row, col = ei[0], ei[1]
     b32, s32 = to_i32(batch), to_i32(system)
-    by_dst, _ = csr_build(col, N)
+    mask = None if edge_mask is None else edge_mask_u8(edge_mask, E)
+    by_dst, _ = csr_build(col, N, mask=mask)
     by_src = by_sys = None
     if need_backward:
-        by_src, _ = csr_build(row, N)
+        by_src, _ = csr_build(row, N, mask=mask)
         by_sys, _ = csr_build(s32, 7)
     crystals, nmax = csr_build(b32, B, want_max=True)
     crystals.perm = None
@@ -831,12 +855,18 @@ def segment_reduce_raw(src: torch.Tensor, rowptr: torch.Tensor, perm: Optional[t
 
 
 def gather_rows_raw(src: torch.Tensor, idx: torch.Tensor, *, deg_rowptr: Optional[torch.Tensor] = None,
-                    add: Optional[torch.Tensor] = None) -> torch.Tensor:
+                    add: Optional[torch.Tensor] = None, mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """out[r] = src[idx[r]] (scaled by 1 / degree with ``deg_rowptr``) (+ add[r]); rows with ``mask[r] == 0`` are 0."""
     R, W = idx.numel(), src.shape[1]
     out = torch.empty(R, W, dtype=src.dtype, device=src.device)
-    L.check(L.lib().dost_gather_rows(L.dt(src), L.p(src), _ld(src), L.p(idx), L.p(deg_rowptr), L.p(add),
-                                     _ld(add) if add is not None else 0, R, W, L.p(out), _ld(out), L.stream()),
-            "gather_rows")
+    if mask is None:
+        L.check(L.lib().dost_gather_rows(L.dt(src), L.p(src), _ld(src), L.p(idx), L.p(deg_rowptr), L.p(add),
+                                         _ld(add) if add is not None else 0, R, W, L.p(out), _ld(out), L.stream()),
+                "gather_rows")
+    else:
+        L.check(L.lib().dost_gather_rows_masked(L.dt(src), L.p(src), _ld(src), L.p(idx), L.p(deg_rowptr), L.p(mask),
+                                                L.p(add), _ld(add) if add is not None else 0, R, W, L.p(out), _ld(out),
+                                                L.stream()), "gather_rows_masked")
     return out
 
 
@@ -1350,7 +1380,9 @@ class _SegmentReduce(torch.autograd.Function):
     @staticmethod
     def backward(ctx, d_out):
         csr: CSR = ctx.csr
-        d_src = gather_rows_raw(d_out.contiguous(), csr.key, deg_rowptr=csr.rowptr if ctx.mean else None)
+        # a masked CSR: the masked rows' gradient is written as exact zeros (their forward rows are finite, so the zeros
+        # stay zeros through the edge MLP and encoder backward and reach edge_vec.grad as 0)
+        d_src = gather_rows_raw(d_out.contiguous(), csr.key, deg_rowptr=csr.rowptr if ctx.mean else None, mask=csr.mask)
         return d_src, None, None
 
 

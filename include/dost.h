@@ -73,6 +73,12 @@ size_t dost_csr_workspace_bytes(long long n, long long size);
 int dost_csr_build(const int32_t* key, long long n, long long size, int32_t* rowptr, int32_t* perm,
                    int32_t* maxcount, void* workspace, size_t workspace_bytes, dost_stream_t stream);
 
+/* The same sort over the entries with mask[i] != 0 only (mask uint8 [n]): rowptr[size+1] counts them, perm[0..rowptr[size])
+ * lists them in (key, index) order and perm[rowptr[size]..n) the masked entries in index order.  With every mask byte set
+ * the result is bitwise dost_csr_build's.  Keys of masked entries are not read for the sort. */
+int dost_csr_build_masked(const int32_t* key, const uint8_t* mask, long long n, long long size, int32_t* rowptr,
+                          int32_t* perm, int32_t* maxcount, void* workspace, size_t workspace_bytes, dost_stream_t stream);
+
 /* *value = max(*value, floor_value) on the device (one int): the data-parallel padding length Nmax = max(this rank's
  * measured maximum, the sharder's global value) without a device->host read (to_dense_batch's max(), SURVEY 8e). */
 int dost_imax_scalar(int32_t* value, int32_t floor_value, dost_stream_t stream);
@@ -262,6 +268,12 @@ int dost_segment_reduce(int dtype, const void* src, long long ld, const int32_t*
 int dost_gather_rows(int dtype, const void* src, long long ld, const int32_t* idx, const int32_t* deg_rowptr,
                      const void* add, long long ld_add, long long R, int W, void* out, long long ldo,
                      dost_stream_t stream);
+
+/* dost_gather_rows over a row mask (uint8 [R]): rows with mask[r] == 0 are written as 0 (add ignored there) and their
+ * idx[r] is never read; the other rows are dost_gather_rows's, deg_rowptr scaling included. */
+int dost_gather_rows_masked(int dtype, const void* src, long long ld, const int32_t* idx, const int32_t* deg_rowptr,
+                            const uint8_t* mask, const void* add, long long ld_add, long long R, int W, void* out,
+                            long long ldo, dost_stream_t stream);
 
 /* Phonon edge features: smooth_cutoff(|v|/4) * [1, sqrt(3) v/|v|] (DOSTransformer_phonon.py:75-77). */
 int dost_phonon_edge_feat(int dtype, const void* edge_vec, long long E, void* out, dost_stream_t stream);
@@ -512,6 +524,9 @@ int dost_edge_geometry(const double* lattice, const double* pos, const int64_t* 
 int dost_edge_geometry_bwd(const double* d_vec, const double* d_len, const double* edge_vec, const double* edge_len,
                            const int64_t* src, const int64_t* dst, const int64_t* shift, long long n, int with_lattice,
                            double* g, dost_stream_t stream);
+/* Membership at the current geometry: mask[e] = (edge_len[e] < cutoff) as uint8, the comparison dost_neighbor_fill applies,
+ * so on the distances dost_edge_geometry writes for a candidate list the live entries are the list a fresh search finds. */
+int dost_edge_within(const double* edge_len, long long n, double cutoff, uint8_t* mask, dost_stream_t stream);
 /* Skin topologies.  The re-pick: atom i's candidates are rows cand_ptr[i]..cand_ptr[i+1] (int32 [N+1]) of cand_dst (rows of
  * pos) / cand_shift [.,3], every image within cutoff + skin at the build geometry in canonical order.  Their distances at
  * (lattice, pos) by the arithmetic contract go to cand_len (and the vectors to the optional cand_vec [.,3]); then, like
